@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SPGG lattice step (BASELINE.json metric: site-updates/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A bench "step" is one chunk of ``--inner`` lattice iterations (default 100) of the whole
 L x L lattice through ``spgg_step`` (statistics on).  N=1 runs BASELINE config 4
@@ -222,7 +222,15 @@ def main():
                     help="c4: the headline L=4096 lattice (default); sweep: BASELINE config 3, the "
                          "r x kappa x M grid as 60 batched L=200 replicas; c1 / c2: the single small "
                          "lattices of configs 0-2 (none of these is a driver bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                         "(see dump_outputs); c4 workload on one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.workload != "c4" or args.only_variants
+                              or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs covers the native c4 workload on one GPU")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -296,7 +304,11 @@ def main():
     ms = e0.elapsed_time(e1)
     eng.sync()
     launches = eng.status().kernel_launches - l0
+    if eng.status().iteration != K * inner:
+        raise SystemExit(f"the timed steps ran {eng.status().iteration} iterations, not {K} x {inner}")
     value = n_sites * inner * K / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, inner)
 
     # ---------------- end to end through the public API with host buffers
     torch.cuda.synchronize()
@@ -399,6 +411,32 @@ def main():
         "extras": extras,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_SITES = 1 << 18    # sites sampled for the state dump
+DUMP_ROWS = 4096        # statistics rows of the dump: the last ones of the step
+
+
+def dump_outputs(out_dir, eng, inner):
+    """What the timed path computed in its last step, as a caller of spgg_step receives it:
+    ``stats`` the statistics rows of that step's last min(inner, DUMP_ROWS) iterations, and ``S``,
+    ``R``, ``Q`` the state it left (float64 R and Q in the reference's layout, S as float32 0 = C /
+    1 = D) at a fixed seeded sample of DUMP_SITES sites, whose flat indices are ``sites`` (the whole
+    state of the L=4096 lattice is 700 MB).  At most 15 MB for any arguments.  The inputs are fixed
+    by the arguments, so two builds can be compared file by file; the float statistics sums may
+    differ in the last bits between runs."""
+    os.makedirs(out_dir, exist_ok=True)
+    S, R, Q = eng.get_state()
+    n = S.size
+    sites = np.sort(np.random.RandomState(0).choice(n, min(DUMP_SITES, n), replace=False))
+    rows = min(inner, DUMP_ROWS)
+    out = {"stats": eng.stats(first=1 + inner - rows, n=rows),
+           "sites": sites.astype(np.float64),
+           "S": S.reshape(-1)[sites].astype(np.float32),
+           "R": R.reshape(-1)[sites],
+           "Q": Q.reshape(n, -1)[sites]}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 BYTES_PER_SITE = {"fp32": 34.25, "fp32_rfloat": 40.25, "fp64": 80.25}   # BASELINE.md section 3

@@ -1,64 +1,66 @@
-"""Container-only pin: the unmodified reference (``/root/reference``, executed through
-``oracle/ref_harness.py`` with h5py/matplotlib stubs) against the oracle restatements and
-against the committed golden fixtures.  Skipped where the reference is absent (GPU box)."""
+"""The unmodified reference against the oracle restatements, the drop-in and the committed
+golden fixtures.  Tests that execute the reference (the copy ``oracle/ref_harness.py`` finds, run
+with h5py/matplotlib stubs) are skipped where no copy is present; the others compare with what
+the fixtures recorded from it."""
 import json
 import os
 
 import numpy as np
 import pytest
 
-from helpers import RUNNER_FIXED, full_params, load_golden
+from helpers import full_params, load_golden
 
 from oracle import ref_harness
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_harness.reference_available(),
-                                 reason="/root/reference not present")]
+needs_ref = pytest.mark.skipif(not ref_harness.reference_available(),
+                               reason="/root/reference not present")
+QLEARNING_GOLDEN = ["c1_rep_m1", "c2_act_m2", "rep_m2_r36", "act_m1_k0", "ctor_defaults", "odd_L_fracR"]
 
 
-@pytest.mark.parametrize("state,second,r,kappa,wP", [
-    ("reputation", False, 3.0, 1.0, 0.95),
-    ("action", True, 4.0, 1.0, 1.0),
-    ("reputation", True, 3.6, 0.5, 1.0),
-])
-def test_reference_run_equals_oracles(state, second, r, kappa, wP):
+@pytest.mark.parametrize("name", ["c1_rep_m1", "c2_act_m2", "rep_m2_r36"])
+def test_reference_run_equals_oracles(golden_dir, name):
+    """Both oracles against a run the reference recorded: reputation state M=1 r=3 kappa=1,
+    action state M=2 r=4 kappa=1, reputation state M=2 r=3.6 kappa=0.5.  S, R, Q bit for bit, and
+    every series the run wrote that the NumPy oracle assembles."""
     from oracle import c_oracle, spgg_numpy
-    L, n, seed = 14, 30, 321
-    params = dict(RUNNER_FIXED, L=L, iterations=n, r=r, influence_factor=kappa,
-                  use_second_order=second, reward_weight_payoff=wP, rep_gain_C=1.0,
-                  state_representation=state)
-    ref = ref_harness.run_reference(seed, **params)
-    assert ref["n_steps"] == n
-    draws = lambda t, L_: (ref["u"][t - 1], ref["b"][t - 1])
+    z, params = load_golden(golden_dir, name)
     p = full_params(params)
-    out = spgg_numpy.simulate(p, ref["s0"], ref["r0"], ref["q0"], draws)
-    assert np.array_equal(out["Sn_final"], ref["s_final"])
-    assert np.array_equal(out["R_final"], ref["r_final"])
-    assert np.array_equal(out["q_final"], ref["q_final"])
-    for key in ("coop_rate_history", "switch_C_to_D", "neighbor_influence_percent",
-                "best_neighbor_second_order_percent", "group_comp_d2_history",
-                "cooperators_q_s1_c_history", "avg_q_s0_d_history", "reputation_reward_ratio"):
-        assert np.array_equal(out[key], ref["datasets"][key], equal_nan=True), key
-    sim = c_oracle.Sim(p, ref["s0"], ref["r0"], ref["q0"], "fp64")
+    L, n = p["L"], int(z["u"].shape[0])
+    assert n == params["iterations"]
+    draws = lambda t, L_: (z["u"][t - 1], z["b"][t - 1])
+    r0 = np.zeros((L, L))                       # spgg.py:129
+    out = spgg_numpy.simulate(p, z["s0"].astype(np.int64), r0, z["q0"], draws)
+    assert np.array_equal(out["Sn_final"], z["s_final"])
+    assert np.array_equal(out["R_final"], z["r_final"])
+    assert np.array_equal(out["q_final"], z["q_final"])
+    series = [k[3:] for k in z.files if k.startswith("ds_") and k[3:] in out]
+    assert {"coop_rate_history", "switch_C_to_D", "neighbor_influence_percent",
+            "best_neighbor_second_order_percent", "reputation_reward_ratio"} <= set(series)
+    for key in series:
+        assert np.array_equal(out[key], z["ds_" + key], equal_nan=True), key
+    sim = c_oracle.Sim(p, z["s0"], r0, z["q0"], "fp64")
     sim.run(n, draws)
-    assert np.array_equal(sim.S, ref["s_final"])
-    assert np.array_equal(sim.R, ref["r_final"])
-    assert np.array_equal(sim.Q, ref["q_final"])
+    assert np.array_equal(sim.S, z["s_final"])
+    assert np.array_equal(sim.R, z["r_final"])
+    assert np.array_equal(sim.Q, z["q_final"])
 
 
-def test_reconstructed_legacy_stream_is_what_the_reference_consumes():
+def test_reconstructed_legacy_stream_is_what_the_reference_consumes(golden_dir):
+    """The ctor draws and per-step draws the reference recorded in each Q-learning fixture, for
+    the fixture's pinned seed."""
     from oracle import spgg_numpy
-    L, n, seed = 10, 6, 99
-    params = dict(RUNNER_FIXED, L=L, iterations=n, r=3.0, influence_factor=1.0,
-                  use_second_order=False, reward_weight_payoff=0.95, rep_gain_C=1.0)
-    ref = ref_harness.run_reference(seed, **params)
-    Q0, S0, draws = spgg_numpy.legacy_draws(seed, L)
-    assert np.array_equal(Q0, ref["q0"]) and np.array_equal(S0, ref["s0"])
-    for t in range(1, n + 1):
-        u, b = draws(t, L)
-        assert np.array_equal(u, ref["u"][t - 1]) and np.array_equal(b, ref["b"][t - 1])
+    for name in QLEARNING_GOLDEN:
+        z, params = load_golden(golden_dir, name)
+        L, n = params["L"], int(z["u"].shape[0])
+        Q0, S0, draws = spgg_numpy.legacy_draws(int(z["seed"]), L)
+        assert np.array_equal(Q0, z["q0"]) and np.array_equal(S0, z["s0"]), name
+        for t in range(1, n + 1):
+            u, b = draws(t, L)
+            assert np.array_equal(u, z["u"][t - 1]) and np.array_equal(b, z["b"][t - 1]), (name, t)
 
 
+@pytest.mark.reference
+@needs_ref
 def test_committed_golden_fixture_is_reproducible(golden_dir):
     """Re-run the reference for one fixture and compare with what is committed."""
     z, params = load_golden(golden_dir, "c1_rep_m1")
@@ -70,6 +72,8 @@ def test_committed_golden_fixture_is_reproducible(golden_dir):
     assert sorted(shapes) == sorted(ref["datasets"])
 
 
+@pytest.mark.reference
+@needs_ref
 def test_dropin_class_has_the_reference_signature_and_exports():
     import inspect
     import spgg_b200
@@ -96,6 +100,8 @@ def test_dropin_class_has_the_reference_signature_and_exports():
         assert k in b.params, k
 
 
+@pytest.mark.reference
+@needs_ref
 def test_runner_folder_name_equals_reference():
     import importlib
     from spgg_b200 import runner
@@ -106,13 +112,13 @@ def test_runner_folder_name_equals_reference():
         assert runner.get_folder_name(*args) == ref_runner.get_folder_name(*args)
 
 
-def test_double_q_ctor_draw_order_equals_reference():
-    """spgg.py:121-127: uniform q_table (discarded), then table 1, table 2, then randint S."""
+def test_double_q_ctor_draw_order_equals_reference(golden_dir):
+    """spgg.py:121-127: uniform q_table (discarded), then table 1, table 2, then randint S - the
+    tables and strategies the reference's ctor drew in the Double Q-learning fixtures."""
     import spgg_b200
-    ref_model = ref_harness.import_reference()
-    with ref_harness.pinned_seed(9):
-        a = ref_model.SPGG(L=10, iterations=3, algorithm="double_qlearning")
-    b = spgg_b200.SPGG(L=10, iterations=3, algorithm="double_qlearning", seed=9)
-    assert np.array_equal(a.algorithm.q_table_1, b.algorithm.q_table_1)
-    assert np.array_equal(a.algorithm.q_table_2, b.algorithm.q_table_2)
-    assert np.array_equal(a.q_table, b.q_table) and np.array_equal(a._Sn, b._Sn)
+    for name in ("doubleq_rep_m1", "doubleq_act_m2"):
+        z, params = load_golden(golden_dir, name)
+        b = spgg_b200.SPGG(**params, seed=int(z["seed"]))
+        assert np.array_equal(b.algorithm.q_table_1, z["q1_0"]), name
+        assert np.array_equal(b.algorithm.q_table_2, z["q2_0"]), name
+        assert np.array_equal(b.q_table, z["q0"]) and np.array_equal(b._Sn, z["s0"]), name
