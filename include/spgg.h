@@ -177,7 +177,7 @@ int spgg_set_replay_pairs(spgg_t *h, int n_steps, int n_pairs, const double *u, 
  * (asynchronous on `cuda_stream`, a cudaStream_t or NULL).  One launch for the
  * whole call when the lattices fit in shared memory (one thread-block cluster
  * per replica, csrc/spgg_resident.cuh); otherwise per iteration either the exact
- * pair k_gmax (lattice-global max |reward difference|, spgg.py:488) + k_step, or -
+ * pair k_gmax_* (lattice-global max |reward difference|, spgg.py:488) + k_step*, or -
  * TMA fast path - ONE launch that assumes the maximum of the previous iteration,
  * computes the true one as a by-product of the update and compares.  A wrong guess
  * is caught on the device (every later launch of the call returns untouched) and the
@@ -212,7 +212,7 @@ int spgg_halo_unpack(spgg_t *h, const void *dev_from_up, const void *dev_from_do
 int spgg_phase_kernel(spgg_t *h, int do_update, int do_select, void *cuda_stream);
 int spgg_phase_gmax(spgg_t *h, void *cuda_stream);
 /* One whole iteration inside begin/end: what spgg_step does per iteration (a single
- * speculative launch when the handle can guess the maximum, else k_gmax + k_step). */
+ * speculative launch when the handle can guess the maximum, else k_gmax_* + k_step*). */
 int spgg_phase_iteration(spgg_t *h, int do_select, void *cuda_stream);
 void *spgg_gmax_device_ptr(spgg_t *h);
 /* Strips and the one-launch iteration: the maximum and the uniform-lattice test

@@ -57,8 +57,7 @@ struct spgg_handle {
   RepConst *d_rc = nullptr;
   double *d_valtab = nullptr;  // fp64 mode: {reward, ratio} per reward code and replica (k_build_valtab)
   bool lean = false;           // Q-learning on the general path: update launches run k_step_lean
-  bool lean_gmax = false;      // general path: k_gmax_lean instead of k_gmax
-  int gmax_ctas_gen = 1;       // CTAs per replica of the general path's k_gmax launch
+  int gmax_ctas_gen = 1;       // CTAs per replica of the general path's k_gmax_lean launch
   void *d_Qb[2] = {nullptr, nullptr};  // [1] only with spec: Q is then read from [qcur] and written to [qcur^1]
   int qcur = 0;
   void *Qcur() const { return d_Qb[qcur]; }
@@ -194,9 +193,6 @@ static void build_repconst(const spgg_params_t &p, RepConst *rc) {
 
 // ---------------------------------------------------------------- dispatch
 // the general and the lean kernels are instantiated in their own translation units (spgg_dispatch.h)
-static gmax_fn_t pick_gmax(int mode, int M, bool lean) {
-  return lean ? pick_gmax_lean(mode, M) : pick_gmax_general(mode, M);
-}
 static size_t step_smem(int mode, int TR) {
   switch (mode) {
     case MODE_F32_I8: return SmemLayout<ModeF32I8>(TR).total;
@@ -495,7 +491,6 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   int occ = 1;
   h->lean = !h->fast && p0.algorithm == 0 && getenv("SPGG_NO_LEAN") == nullptr;
   if (h->lean) h->smem_step = step_smem(h->mode, LEAN_TR_MAX);   // k_step_lean addresses the 16-row layout
-  h->lean_gmax = getenv("SPGG_NO_LEAN") == nullptr;
   for (int replay = 0; replay < 2; ++replay) {
     step_fn_t f = pick_step(h->mode, h->M, h->action, replay);
     CUDA_TRY(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_step));
@@ -523,7 +518,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
     h->gmax_ctas = (int)std::max<long long>(1, std::min<long long>((n_tiles_g + GWARPS - 1) / GWARPS,
                        ((long long)prop.multiProcessorCount * std::max(1, gocc)) / n_replicas));
   }
-  CUDA_TRY(cudaFuncSetAttribute(pick_gmax(h->mode, h->M, h->lean_gmax), cudaFuncAttributeMaxDynamicSharedMemorySize,
+  CUDA_TRY(cudaFuncSetAttribute(pick_gmax_lean(h->mode, h->M), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)h->smem_gmax));
   if (occ < 1) { delete h; return fail(SPGG_E_CUDA, "kernel does not fit on an SM (smem %zu)", h->smem_step); }
   const long long n_tiles = (long long)g.n_tx * g.n_ty;
@@ -531,7 +526,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   g.ctas_per_rep = (int)std::min<long long>(n_tiles, per_rep);
   {
     int gocc = 1;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&gocc, pick_gmax(h->mode, h->M, h->lean_gmax), h->threads, h->smem_gmax));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&gocc, pick_gmax_lean(h->mode, h->M), h->threads, h->smem_gmax));
     h->gmax_ctas_gen = (int)std::min<long long>(n_tiles, std::max<long long>(1, ((long long)prop.multiProcessorCount * std::max(1, gocc)) / n_replicas));
   }
   // the fast kernel's packed 16-bit counters bound the sites one thread may visit per launch
@@ -1060,7 +1055,7 @@ extern "C" int spgg_phase_kernel(spgg_t *h, int do_update, int do_select, void *
 }
 
 // finish the next iteration (and choose the action of the one after it when do_select): one speculative
-// launch when the handle can guess the global maximum, else the exact pair k_gmax + k_step
+// launch when the handle can guess the global maximum, else the exact pair (maximum kernel, then update kernel)
 extern "C" int spgg_phase_iteration(spgg_t *h, int do_select, void *stream_) {
   if (!h || !h->pending) return fail(SPGG_E_STATE, "spgg_phase_iteration outside begin/end");
   if (h->pend_rel >= h->pend_n) return fail(SPGG_E_STATE, "the chunk announced to spgg_begin_steps is complete");
@@ -1088,7 +1083,7 @@ extern "C" int spgg_phase_gmax(spgg_t *h, void *stream_) {
     CUDA_TRY(launch_pdl(pick_gfast(h->M), h->gmax_ctas * h->n_rep, GWARPS * 32, gfast_smem(h->M), st,
                         h->fmaps[h->cur].ld_code, a));
   } else {
-    gmax_fn_t f = pick_gmax(h->mode, h->M, h->lean_gmax);
+    gmax_fn_t f = pick_gmax_lean(h->mode, h->M);
     a.g.ctas_per_rep = h->gmax_ctas_gen;   // a light kernel: its own persistent grid (more CTAs per SM than k_step)
     const int grid = h->gmax_ctas_gen * h->n_rep;
     if ((long long)h->g.n_tx * h->g.n_ty * h->n_rep <= 160) CUDA_TRY(launch_pdl(f, grid, h->threads, h->smem_gmax, st, a));
@@ -1242,9 +1237,9 @@ extern "C" int spgg_describe(spgg_t *h, char *buf, int n) {
     len = snprintf(tmp, sizeof(tmp), "fast: TMA-staged %dx%d tiles, %d persistent CTAs per replica, %s (%s)",
                    FTR, TC, h->g.ctas_per_rep,
                    (h->spec && h->spec_on) ? "one launch per iteration (speculative global maximum, verified)"
-                                           : "two launches per iteration (k_gmax + k_step)", arith);
+                                           : "two launches per iteration (k_gmax_fast + k_step_fast)", arith);
   else
-    len = snprintf(tmp, sizeof(tmp), "general: %dx%d tiles, %d CTAs per replica, two launches per iteration (k_gmax + %s) (%s)", h->g.TR, TC,
+    len = snprintf(tmp, sizeof(tmp), "general: %dx%d tiles, %d CTAs per replica, two launches per iteration (k_gmax_lean + %s) (%s)", h->g.TR, TC,
                    h->g.ctas_per_rep, h->lean ? "k_step_lean" : "k_step", arith);
   if (buf && n > 0) {
     strncpy(buf, tmp, (size_t)n - 1);

@@ -1,7 +1,7 @@
 // Kernel pickers shared by the translation units of libspgg_b200.  The library is compiled as three units in
 // parallel (__graft_entry__.build): spgg_capi.cu (C ABI, host logic, fast / resident / helper kernels),
-// spgg_inst_general.cu (every instantiation of k_step / k_gmax) and spgg_inst_lean.cu (k_step_lean /
-// k_gmax_lean / k_build_valtab).  A kernel is compiled in the unit that instantiates it; the others launch it
+// spgg_inst_general.cu (every instantiation of k_step) and spgg_inst_lean.cu (k_step_lean / k_gmax_lean /
+// k_build_valtab).  A kernel is compiled in the unit that instantiates it; the others launch it
 // through the function pointer returned here.
 #pragma once
 #include "spgg_kernels.cuh"
@@ -15,7 +15,6 @@ typedef void (*gmax_fn_t)(GArgs);
 
 // spgg_inst_general.cu
 step_fn_t pick_step(int mode, int M, int action, int replay);
-gmax_fn_t pick_gmax_general(int mode, int M);
 // spgg_inst_lean.cu
 step_fn_t pick_lean(int mode, int M, int action, int replay);
 gmax_fn_t pick_gmax_lean(int mode, int M);

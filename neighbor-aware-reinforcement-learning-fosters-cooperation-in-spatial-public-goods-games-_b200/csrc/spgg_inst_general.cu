@@ -19,12 +19,5 @@ step_fn_t pick_step(int mode, int M, int action, int replay) {
     default: return pick_step1<ModeF64>(M, action, replay);
   }
 }
-gmax_fn_t pick_gmax_general(int mode, int M) {
-  switch (mode) {
-    case MODE_F32_I8: return M == 2 ? k_gmax<ModeF32I8, 2> : k_gmax<ModeF32I8, 1>;
-    case MODE_F32_F: return M == 2 ? k_gmax<ModeF32F, 2> : k_gmax<ModeF32F, 1>;
-    default: return M == 2 ? k_gmax<ModeF64, 2> : k_gmax<ModeF64, 1>;
-  }
-}
 
 }  // namespace spgg

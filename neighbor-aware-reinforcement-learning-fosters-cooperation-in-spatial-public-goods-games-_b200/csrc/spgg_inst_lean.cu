@@ -21,7 +21,7 @@ step_fn_t pick_lean(int mode, int M, int action, int replay) {
     default: return pick_lean1<ModeF64>(M, action, replay);
   }
 }
-// k_gmax_lean: same value as k_gmax, every neighbour pair once
+// the global maximum of the general path
 gmax_fn_t pick_gmax_lean(int mode, int M) {
   switch (mode) {
     case MODE_F32_I8: return M == 2 ? k_gmax_lean<ModeF32I8, 2> : k_gmax_lean<ModeF32I8, 1>;

@@ -4,7 +4,7 @@
 // rule src/model/algorithms.py:96-133) is split along its data dependencies
 // (DESIGN.md "step decomposition"):
 //
-//   k_gmax<t>   light: reads the per-site reward codes of iteration t, produces the
+//   k_gmax*<t>  light: reads the per-site reward codes of iteration t, produces the
 //               lattice-global max |reward difference|           (spgg.py:486-488)
 //   k_step<t>   heavy, fused: finishes iteration t (TD update algorithms.py:122-131,
 //               neighbour-aware update spgg.py:478-509, statistics spgg.py:512-592)
@@ -120,7 +120,7 @@ struct KArgs {
   // With spec != 0 the launch does not wait for a k_gmax pass: it uses the previous iteration's value
   // (gcarry[rep]) and the last CTA compares; on a mismatch it records rel in *bad_at, every later launch of
   // the chunk returns at once, and the host re-runs from there with the (now known) exact value.
-  int spec;                // 0 exact (gmax[rep][rel] was computed by k_gmax), 1 guess = gcarry[rep], 2 test hook: a wrong guess
+  int spec;                // 0 exact (gmax[rep][rel] was computed by k_gmax_*), 1 guess = gcarry[rep], 2 test hook: a wrong guess
   float *gcarry;           // [n_rep] exact maximum of the last finished iteration (written by every update launch)
   int *bad_at;             // handle-wide: INT_MAX, or the first rel whose speculation failed
   // Row strips (one lattice over several GPUs): the maximum and the uniform-lattice test of spgg.py:405 are
@@ -498,7 +498,7 @@ __device__ __forceinline__ void store_bits_word(uint32_t *S, const Geom &g, int 
   }
 }
 
-// =================================================================== k_gmax
+// =================================================================== global maximum (k_gmax_lean, spgg_lean.cuh)
 struct GArgs {
   Geom g;
   const RepConst *rc;
@@ -508,93 +508,6 @@ struct GArgs {
   const int *stop_at;
   int j, rel, cap;
 };
-
-template <class Md, int M>
-__global__ void __launch_bounds__(MAX_THREADS) k_gmax(GArgs a) {
-  typedef typename Md::Code Code;
-  typedef typename Md::Val Val;
-  constexpr int NK = (M == 2) ? 12 : 4;
-  const Geom &g = a.g;
-  const int rep = blockIdx.x / g.ctas_per_rep, cta = blockIdx.x % g.ctas_per_rep;
-  // launched with programmatic stream serialization only when a launch is short (spgg_capi.cu)
-  pdl_launch_dependents();
-  pdl_wait();  // the code plane and the stop flags come from the k_step before this kernel
-  const int stop = a.stop_at[rep];
-  if (stop >= 0 && a.j > stop) return;
-
-  extern __shared__ __align__(16) unsigned char smem[];
-  Val *sm_val = reinterpret_cast<Val *>(smem);
-  float *sm_tab = reinterpret_cast<float *>(smem + align_up(sizeof(Val) * (g.TR + 2 * HR) * SMW, 16));
-  __shared__ RepConst s_rc;
-  for (int i = threadIdx.x; i < (int)(sizeof(RepConst) / 4); i += blockDim.x)
-    reinterpret_cast<uint32_t *>(&s_rc)[i] = reinterpret_cast<const uint32_t *>(a.rc + rep)[i];
-  __syncthreads();
-  if (!Md::kFp64)
-    for (int i = threadIdx.x; i < 128; i += blockDim.x) sm_tab[i] = s_rc.rewtab[i];
-
-  const Code *code_in = reinterpret_cast<const Code *>(a.code_in) + (long long)rep * g.plane_stride;
-  const double *vtab = a.valtab ? a.valtab + ((size_t)rep << (VALTAB_BITS + 1)) : nullptr;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  Val lmax = Val(0);
-
-  const int n_tiles = g.n_tx * g.n_ty;
-  for (int tile = cta; tile < n_tiles; tile += g.ctas_per_rep) {
-    const int r0 = (tile / g.n_tx) * g.TR, c0 = (tile % g.n_tx) * TC;
-    __syncthreads();
-    {
-      constexpr int NC = TC + 2 * M;
-      const int nr = g.TR + 2 * M;
-      for (int e = threadIdx.x; e < nr * NC; e += blockDim.x) {
-        const int rr = e / NC - M, cc = e % NC - M;
-        const int prow = r0 + rr + GH;
-        Val v = Val(0);
-        if (prow >= 0 && prow < g.rows + 2 * GH) {
-          const int col = wrap_col(c0 + cc, g.L);
-          v = val_of_code<Md>(code_in[(long long)prow * g.pitchB + CPAD + col], s_rc, sm_tab, vtab);
-        }
-        sm_val[(rr + HR) * SMW + cc + HP] = v;
-      }
-    }
-    __syncthreads();
-    for (int rr = warp; rr < g.TR; rr += nw) {
-      if (r0 + rr >= g.rows) break;
-#pragma unroll
-      for (int k4 = 0; k4 < 4; ++k4) {
-        const int cc = k4 * 32 + lane;
-        if (c0 + cc >= g.L) continue;
-        const int sr = rr + HR, sc = cc + HP;
-        const Val vx = sm_val[sr * SMW + sc];
-#pragma unroll
-        for (int k = 0; k < NK; ++k) {
-          const Val vk = sm_val[(sr - c_off[k][0]) * SMW + (sc - c_off[k][1])];
-          Val d;
-          if constexpr (Md::kFp64) d = fabs(__dsub_rn(vk, vx));
-          else d = fabsf(__fsub_rn(vk, vx));
-          lmax = d > lmax ? d : lmax;
-        }
-      }
-    }
-  }
-  // block max -> one atomic per CTA (non-negative IEEE values order like unsigned ints)
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const Val other = __shfl_down_sync(0xffffffffu, lmax, o);
-    lmax = other > lmax ? other : lmax;
-  }
-  __shared__ Val s_wmax[MAX_THREADS / 32];
-  if (lane == 0) s_wmax[warp] = lmax;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    Val m = s_wmax[0];
-    for (int w = 1; w < nw; ++w) m = s_wmax[w] > m ? s_wmax[w] : m;
-    Val *dst = reinterpret_cast<Val *>(a.gmax) + (long long)rep * a.cap + a.rel;
-    if constexpr (Md::kFp64)
-      atomicMax(reinterpret_cast<unsigned long long *>(dst), (unsigned long long)__double_as_longlong(m));
-    else
-      atomicMax(reinterpret_cast<unsigned int *>(dst), __float_as_uint(m));
-  }
-}
-
 
 // Stages the halo'd planes of a tile with every global load of a thread in flight at once (the general
 // kernel's element loops expose one memory round trip per element: ncu, profiles/r02_fp64_lean.md).
@@ -789,6 +702,98 @@ __device__ __forceinline__ void step_epilogue(const KArgs &a, int rep, int cta, 
   }
 }
 
+// ------------------------------------------------------------------ site code of k_step and k_step_lean
+// k_step_lean (spgg_lean.cuh) must give k_step's results bit for bit: the pieces they share live here once.
+// The statistics, the epsilon-greedy choice and the stores stay in the kernels: as helpers they reorder
+// k_step_lean's machine code.  So does the group-count loop in k_step, where it adds spills (SARSA at fp32).
+
+// the replica's constants into shared memory, then NTAB of its fp32 tables (reward, ratio statistic) into sm_tab
+template <int NTAB>
+__device__ __forceinline__ void load_rep_const(RepConst &s_rc, const RepConst *src, float *sm_tab) {
+  for (int i = threadIdx.x; i < (int)(sizeof(RepConst) / 4); i += blockDim.x)
+    reinterpret_cast<uint32_t *>(&s_rc)[i] = reinterpret_cast<const uint32_t *>(src)[i];
+  __syncthreads();
+  if constexpr (NTAB > 0) {
+    for (int i = threadIdx.x; i < 128; i += blockDim.x) {
+      sm_tab[i] = s_rc.rewtab[i];
+      if constexpr (NTAB > 1) sm_tab[128 + i] = s_rc.ratiotab[i];
+    }
+  }
+}
+
+// denominator of lambda from the launch's global maximum (spgg.py:489): fp64 divides by den, fp32 multiplies by inv_den
+template <class Md>
+__device__ __forceinline__ void lambda_den(const KArgs &a, int rep, const RepConst &rc, typename Md::Val &den,
+                                           typename Md::Val &inv_den) {
+  const typename Md::Val gm = reinterpret_cast<const typename Md::Val *>(a.gmax)[(long long)rep * a.cap + a.rel];
+  if constexpr (Md::kFp64) den = __dadd_rn(gm, rc.leps);
+  else inv_den = __fdiv_rn(1.0f, __fadd_rn(gm, rc.leps_f));
+}
+
+// Philox words of the four sites a lane owns in the 128-site row segment at column c0 (c0 + 32*k4 + lane):
+// counter = (column / 4, global row, ctr2, ctr3), one call serves 4 consecutive sites.  This lane computes the
+// words of columns c0+4*lane..+3; its own sites fetch theirs from lane 8*k4 + lane/4, word lane%4.
+__device__ __forceinline__ void philox_row(int c0, int row, uint32_t ctr2, uint32_t ctr3, const RepConst &rc, int lane,
+                                           uint32_t w4[4]) {
+  uint32_t wc[4];
+  philox4x32_10((uint32_t)((c0 >> 2) + lane), (uint32_t)row, ctr2, ctr3, rc.seed_lo, rc.seed_hi, wc);
+#pragma unroll
+  for (int k4 = 0; k4 < 4; ++k4) {
+    const int src = 8 * k4 + (lane >> 2);
+    const uint32_t x0 = __shfl_sync(0xffffffffu, wc[0], src), x1 = __shfl_sync(0xffffffffu, wc[1], src);
+    const uint32_t x2 = __shfl_sync(0xffffffffu, wc[2], src), x3 = __shfl_sync(0xffffffffu, wc[3], src);
+    w4[k4] = sel4<uint32_t>(lane & 3, x0, x1, x2, x3);
+  }
+}
+
+// neighbour-aware term inputs (spgg.py:486-494): the largest neighbour reward difference d (first arg-max wins),
+// that neighbour's shared-memory index and its offset number k
+template <class Val>
+struct BestNeighbour {
+  Val d;
+  int idx, k;
+};
+template <class Md, int M>
+__device__ __forceinline__ BestNeighbour<typename Md::Val> best_neighbour(const typename Md::Val *sm_val, int sr, int sc,
+                                                                          typename Md::Val vx) {
+  typedef typename Md::Val Val;
+  constexpr int NK = (M == 2) ? 12 : 4;
+  Val best = Val(0);
+  int bidx = sr * SMW + sc, kstar = 0;
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    const int nidx = (sr - c_off[k][0]) * SMW + (sc - c_off[k][1]);
+    const Val vk = sm_val[nidx];
+    Val d;
+    if constexpr (Md::kFp64) d = __dsub_rn(vk, vx);
+    else d = __fsub_rn(vk, vx);
+    if (k == 0 || d > best) { best = d; bidx = nidx; kstar = k; }
+  }
+  return {best, bidx, kstar};
+}
+
+// fp32 TD update of Q[s][act] (algorithms.py:122-131) plus the neighbour-aware term (spgg.py:478-509); returns the
+// new entry and adds the site's NI statistic (spgg.py:512) to tni.  next(x0, x1, after) is the value of the next
+// state's row (x0, x1) before (after = false) and after (true) the TD write; na, nb is that row before it.
+template <class NextF>
+__device__ __forceinline__ float td_update_f32(const RepConst &rc, float vx, float qe, float na, float nb, int s,
+                                               int s_new, int act, float best, bool same, float inv_den, NextF next,
+                                               float &tni) {
+  const float mx = next(na, nb, false);
+  const float td = __fsub_rn(__fmaf_rn(rc.gamma_f, mx, vx), qe);
+  const float qtd = __fmaf_rn(rc.alpha_f, td, qe);
+  const float lam = __fmul_rn(__fmul_rn(rc.kappa_f, fmaxf(0.0f, best)), inv_den);
+  const float nu = same ? lam : -lam;
+  const float na2 = (s_new == s && act == 0) ? qtd : na;
+  const float nb2 = (s_new == s && act == 1) ? qtd : nb;
+  const float td2 = __fsub_rn(__fmaf_rn(rc.gamma_f, next(na2, nb2, true), vx), qtd);
+  const float qfin = __fadd_rn(qtd, nu);
+  const float an = fabsf(nu);
+  tni = __fmaf_rn(__fdividef(an, __fadd_rn(__fadd_rn(fabsf(__fmul_rn(rc.alpha_f, td2)), an), 1e-8f)), 100.0f, tni);
+  return qfin;
+}
+
+
 // The general kernel is latency-bound (one site per thread and row, dependent shared-memory stencils):
 // what it needs is resident warps, not registers.  Measured at L=4000 (fp32, int8 R), us per iteration:
 // 1 CTA/SM (190 registers) 1604, 2 CTAs/SM 891, 3 CTAs/SM (80 registers, a few hundred bytes of spills) 718.
@@ -801,11 +806,10 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
   typedef typename Md::R RT;
   typedef typename Md::Code Code;
   typedef typename Md::Val Val;
-  constexpr int NK = (M == 2) ? 12 : 4;
   constexpr bool kI8 = (sizeof(RT) == 1);
   const Geom &g = a.g;
   const int rep = blockIdx.x / g.ctas_per_rep, cta = blockIdx.x % g.ctas_per_rep;
-  pdl_launch_dependents();  // see k_gmax
+  pdl_launch_dependents();  // launched with programmatic stream serialization only when a launch is short (spgg_capi.cu)
   pdl_wait();  // the planes, the stop flags and gmax come from the kernels before this one
   const int stop = a.stop_at[rep];
   if (stop >= 0 && a.j > stop) return;
@@ -824,14 +828,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
   double *sm_red = reinterpret_cast<double *>(smem + lay.off_red);
   __shared__ RepConst s_rc;
   __shared__ int s_is_last;
-
-  for (int i = threadIdx.x; i < (int)(sizeof(RepConst) / 4); i += blockDim.x)
-    reinterpret_cast<uint32_t *>(&s_rc)[i] = reinterpret_cast<const uint32_t *>(a.rc + rep)[i];
-  __syncthreads();
-  for (int i = threadIdx.x; i < 128; i += blockDim.x) {
-    sm_tab[i] = s_rc.rewtab[i];
-    sm_ratio[i] = s_rc.ratiotab[i];
-  }
+  load_rep_const<2>(s_rc, a.rc + rep, sm_tab);
   const RepConst &rc = s_rc;
 
   const double *vtab = a.valtab ? a.valtab + ((size_t)rep << (VALTAB_BITS + 1)) : nullptr;
@@ -853,11 +850,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
 
   // scalars of this launch
   Val inv_den = Val(0), den = Val(1);
-  if (upd) {
-    const Val gm = reinterpret_cast<const Val *>(a.gmax)[(long long)rep * a.cap + a.rel];
-    if constexpr (Md::kFp64) den = __dadd_rn(gm, rc.leps);  // spgg.py:489 denominator
-    else inv_den = __fdiv_rn(1.0f, __fadd_rn(gm, rc.leps_f));
-  }
+  if (upd) lambda_den<Md>(a, rep, rc, den, inv_den);
   const long long tab_idx = (long long)(a.rel + 1) * g.n_rep + rep;
   // SARSA / Expected SARSA evaluate the policy of the iteration being finished (epsilon_j)
   const double eps_u = (upd && a.algo != 0) ? a.eps_tab[(long long)a.rel * g.n_rep + rep] : 0.0;
@@ -915,37 +908,12 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
       if (i >= g.rows) break;
       const int sr = rr + HR;
       uint32_t w4[4] = {0, 0, 0, 0};
-      if (sel && !REPLAY) {
-        // counter = (column / 4, global row, iteration, 0): one call serves 4 consecutive sites.
-        // This lane computes the words of columns c0+4*lane..+3; its own sites (columns
-        // c0 + 32*k4 + lane) fetch theirs from lane 8*k4 + lane/4, word lane%4.
-        uint32_t wc[4];
-        philox4x32_10((uint32_t)((c0 >> 2) + lane), (uint32_t)(g.row0 + i),
-                      (uint32_t)(a.j + 1), 0u, rc.seed_lo, rc.seed_hi, wc);
-#pragma unroll
-        for (int k4 = 0; k4 < 4; ++k4) {
-          const int src = 8 * k4 + (lane >> 2);
-          const uint32_t x0 = __shfl_sync(0xffffffffu, wc[0], src), x1 = __shfl_sync(0xffffffffu, wc[1], src);
-          const uint32_t x2 = __shfl_sync(0xffffffffu, wc[2], src), x3 = __shfl_sync(0xffffffffu, wc[3], src);
-          w4[k4] = sel4<uint32_t>(lane & 3, x0, x1, x2, x3);
-        }
-      }
+      if (sel && !REPLAY) philox_row(c0, g.row0 + i, (uint32_t)(a.j + 1), 0u, rc, lane, w4);
       uint32_t wS1[4] = {0, 0, 0, 0}, wS2[4] = {0, 0, 0, 0};
       if (upd && (a.algo == 1 || a.algo == 3) && a.u2 == nullptr) {
         // SARSA's two further draws of iteration j: Philox streams 1 and 2 (counter word 3)
-#pragma unroll
-        for (int st = 1; st <= 2; ++st) {
-          uint32_t wc[4];
-          philox4x32_10((uint32_t)((c0 >> 2) + lane), (uint32_t)(g.row0 + i), (uint32_t)a.j, (uint32_t)st,
-                        rc.seed_lo, rc.seed_hi, wc);
-#pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) {
-            const int src = 8 * k4 + (lane >> 2);
-            const uint32_t x0 = __shfl_sync(0xffffffffu, wc[0], src), x1 = __shfl_sync(0xffffffffu, wc[1], src);
-            const uint32_t x2 = __shfl_sync(0xffffffffu, wc[2], src), x3 = __shfl_sync(0xffffffffu, wc[3], src);
-            (st == 1 ? wS1 : wS2)[k4] = sel4<uint32_t>(lane & 3, x0, x1, x2, x3);
-          }
-        }
+        philox_row(c0, g.row0 + i, (uint32_t)a.j, 1u, rc, lane, wS1);
+        philox_row(c0, g.row0 + i, (uint32_t)a.j, 2u, rc, lane, wS2);
       }
 #pragma unroll
       for (int k4 = 0; k4 < 4; ++k4) {
@@ -985,19 +953,9 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
             const int s = code & 1u, coop = (code >> 1) & 1u, wasC = (code >> 2) & 1u;
             const int act = coop ^ 1;
             const Val vx = sm_val[sidx];
-            // neighbour-aware term inputs: spgg.py:486-494 (first arg-max wins)
-            Val best = Val(0);
-            int bidx = sidx, kstar = 0;
-#pragma unroll
-            for (int k = 0; k < NK; ++k) {
-              const int nidx = (sr - c_off[k][0]) * SMW + (sc - c_off[k][1]);
-              const Val vk = sm_val[nidx];
-              Val d;
-              if constexpr (Md::kFp64) d = __dsub_rn(vk, vx);
-              else d = __fsub_rn(vk, vx);
-              if (k == 0 || d > best) { best = d; bidx = nidx; kstar = k; }
-            }
-            const bool same = (((sm_code[bidx] >> 1) & 1u) == (unsigned)coop);
+            const auto bn = best_neighbour<Md, M>(sm_val, sr, sc, vx);
+            const Val best = bn.d;
+            const bool same = (((sm_code[bn.idx] >> 1) & 1u) == (unsigned)coop);
             const int e = 2 * s + act;
             const QT qe = sel4<QT>(e, q0_, q1_, q2_, q3_);
             const QT na = s_new ? q2_ : q0_, nb = s_new ? q3_ : q1_;  // pre-update row of s'
@@ -1089,24 +1047,14 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
                 sumRatio += __dmul_rn(
                     __ddiv_rn(fabs(__dmul_rn(rc.wR, 0.5)), __dadd_rn(fabs(vx), 1e-9)), 100.0);
             } else {
-              auto next_value = [&](float x0, float x1, bool ex, int rn) -> float {
+              auto next_value = [&](float x0, float x1, bool after) -> float {
                 if (a.algo == 0) return fmaxf(x0, x1);
                 const int greedy = (x1 > x0) ? 1 : 0;
-                if (a.algo == 1) return (ex ? rn : greedy) ? x1 : x0;
+                if (a.algo == 1) return ((after ? ex2 : ex1) ? (after ? rn2 : rn1) : greedy) ? x1 : x0;
                 const float e = (float)eps_u, po = __fmul_rn(e, 0.5f), pg = __fadd_rn(__fsub_rn(1.0f, e), po);
                 return __fmaf_rn(greedy ? pg : po, x1, __fmul_rn(greedy ? po : pg, x0));
               };
-              const float mx = next_value(na, nb, ex1, rn1);
-              const float td = __fsub_rn(__fmaf_rn(rc.gamma_f, mx, vx), qe);
-              qtd = __fmaf_rn(rc.alpha_f, td, qe);
-              const float lam = __fmul_rn(__fmul_rn(rc.kappa_f, fmaxf(0.0f, best)), inv_den);
-              const float nu = same ? lam : -lam;
-              const float na2 = (s_new == s && act == 0) ? qtd : na;
-              const float nb2 = (s_new == s && act == 1) ? qtd : nb;
-              const float td2 = __fsub_rn(__fmaf_rn(rc.gamma_f, next_value(na2, nb2, ex2, rn2), vx), qtd);
-              qfin = __fadd_rn(qtd, nu);
-              const float an = fabsf(nu);
-              tni = __fmaf_rn(__fdividef(an, __fadd_rn(__fadd_rn(fabsf(__fmul_rn(rc.alpha_f, td2)), an), 1e-8f)), 100.0f, tni);
+              qfin = td_update_f32(rc, vx, qe, na, nb, s, s_new, act, best, same, inv_den, next_value, tni);
               pk_sn += (unsigned long long)(code >> 3) << (16 * (wasC * 2 + coop));
               if (rc.has_ratio && coop) tratio += sm_ratio[code >> 1];
             }
@@ -1117,7 +1065,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs 
               q3_ = (e == 3) ? qfin : q3_;
             }
             pk_n += 1u << (8 * (wasC * 2 + coop));
-            if (best > Val(0)) { n_best += 1u; n_best2 += (kstar >= 4); }
+            if (best > Val(0)) { n_best += 1u; n_best2 += (bn.k >= 4); }
             pk_grp += 1ull << (10 * (5 - (int)sm_N[sidx]));                              // spgg.py:586-592
             if constexpr (Md::kFp64) {
               sumQ[0] += q0_; sumQ[1] += q1_; sumQ[2] += q2_; sumQ[3] += q3_;

@@ -1,12 +1,14 @@
-// Lean update kernel of the general path: the Q-learning iteration of k_step (spgg_kernels.cuh) for the
-// lattices the TMA fast path does not take - reference precision (fp64 Q and R, spgg.py:121,129), fp32
-// reputations, lattice sides that are not multiples of 32 - with the same thread <-> site mapping, the same
-// arithmetic in the same order and therefore the same results bit for bit, statistics included
-// (tests/test_gpu_lean.py compares the two with SPGG_NO_LEAN=1).
+// Kernels of the general path, for the lattices the TMA fast path does not take - reference precision (fp64 Q
+// and R, spgg.py:121,129), fp32 reputations, lattice sides that are not multiples of 32:
+//   k_gmax_lean  the global maximum of every iteration, whatever the TD rule;
+//   k_step_lean  the Q-learning iteration of k_step (spgg_kernels.cuh) with the same thread <-> site mapping, the
+//                same arithmetic in the same order and therefore the same results bit for bit, statistics included
+//                (tests/test_gpu_lean.py compares the two with SPGG_NO_LEAN=1).  The site code both kernels share
+//                (constants, lambda denominator, Philox words, arg-max neighbour, fp32 update) is written once in spgg_kernels.cuh.
 //
 // k_step carries every TD rule, the replay of up to three draw streams and the select-only / update-only
 // launches behind runtime switches; ncu counted 570 instructions per site for its select-only launch alone
-// (profiles/r02_fp64_lean.md).  What this kernel does differently:
+// (profiles/r02_fp64_lean.md).  What k_step_lean does differently:
 //   * Q-learning and "update" are compile-time facts (the host launches it for algo 0, do_update = 1);
 //   * the reward of an fp64 code is a table lookup (KArgs::valtab, built once per handle by k_build_valtab
 //     with payoff_f64 / reward_f64 themselves) instead of an fp64 division per staged site;
@@ -49,10 +51,10 @@ __global__ void k_build_valtab(const RepConst *rc_all, double *tab) {
 template <bool B>
 struct BoolC { static constexpr bool value = B; };
 
-// Lattice-global max |reward difference| over neighbour pairs (spgg.py:486-488), lean version of k_gmax:
-// tiles staged row by row with the rewards looked up while they land, and every unordered pair taken once
-// (|x - y| == |y - x| exactly): from each site towards (i+1,j), (i,j+1) and, second order, (i+2,j), (i,j+2),
-// (i+1,j+1), (i+1,j-1).  The maximum of a set does not depend on the order: same value as k_gmax.
+// Lattice-global max |reward difference| over neighbour pairs (spgg.py:486-488): tiles staged row by row with
+// the rewards looked up while they land, and every unordered pair taken once (|x - y| == |y - x| exactly): from
+// each site towards (i+1,j), (i,j+1) and, second order, (i+2,j), (i,j+2), (i+1,j+1), (i+1,j-1).  The maximum of
+// a set does not depend on the order.  One atomic per CTA (non-negative IEEE values order like unsigned ints).
 template <class Md, int M>
 __global__ void __launch_bounds__(MAX_THREADS) k_gmax_lean(GArgs a) {
   typedef typename Md::Code Code;
@@ -68,11 +70,7 @@ __global__ void __launch_bounds__(MAX_THREADS) k_gmax_lean(GArgs a) {
   Val *sm_val = reinterpret_cast<Val *>(smem);
   float *sm_tab = reinterpret_cast<float *>(smem + align_up(sizeof(Val) * (g.TR + 2 * HR) * SMW, 16));
   __shared__ RepConst s_rc;
-  for (int i = threadIdx.x; i < (int)(sizeof(RepConst) / 4); i += blockDim.x)
-    reinterpret_cast<uint32_t *>(&s_rc)[i] = reinterpret_cast<const uint32_t *>(a.rc + rep)[i];
-  __syncthreads();
-  if (!Md::kFp64)
-    for (int i = threadIdx.x; i < 128; i += blockDim.x) sm_tab[i] = s_rc.rewtab[i];
+  load_rep_const<Md::kFp64 ? 0 : 1>(s_rc, a.rc + rep, sm_tab);
 
   const Code *code_in = reinterpret_cast<const Code *>(a.code_in) + (long long)rep * g.plane_stride;
   const double *vtab = a.valtab ? a.valtab + ((size_t)rep << (VALTAB_BITS + 1)) : nullptr;
@@ -137,7 +135,6 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
   typedef typename Md::R RT;
   typedef typename Md::Code Code;
   typedef typename Md::Val Val;
-  constexpr int NK = (M == 2) ? 12 : 4;
   constexpr bool kI8 = (sizeof(RT) == 1);
   const Geom &g = a.g;
   const int rep = blockIdx.x / g.ctas_per_rep, cta = blockIdx.x % g.ctas_per_rep;
@@ -163,13 +160,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
   __shared__ RepConst s_rc;
   __shared__ int s_is_last;
 
-  for (int i = threadIdx.x; i < (int)(sizeof(RepConst) / 4); i += blockDim.x)
-    reinterpret_cast<uint32_t *>(&s_rc)[i] = reinterpret_cast<const uint32_t *>(a.rc + rep)[i];
-  __syncthreads();
-  for (int i = threadIdx.x; i < 128; i += blockDim.x) {
-    sm_tab[i] = s_rc.rewtab[i];
-    sm_ratio[i] = s_rc.ratiotab[i];
-  }
+  load_rep_const<2>(s_rc, a.rc + rep, sm_tab);
   const RepConst &rc = s_rc;
   const double *vtab = a.valtab ? a.valtab + ((size_t)rep << (VALTAB_BITS + 1)) : nullptr;
 
@@ -182,11 +173,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
   uint32_t *S_out = a.S_out + (long long)rep * g.bits_stride;
 
   Val inv_den = Val(0), den = Val(1);
-  {
-    const Val gm = reinterpret_cast<const Val *>(a.gmax)[(long long)rep * a.cap + a.rel];
-    if constexpr (Md::kFp64) den = __dadd_rn(gm, rc.leps);  // spgg.py:489 denominator
-    else inv_den = __fdiv_rn(1.0f, __fadd_rn(gm, rc.leps_f));
-  }
+  lambda_den<Md>(a, rep, rc, den, inv_den);
   const long long tab_idx = (long long)(a.rel + 1) * g.n_rep + rep;
   const uint32_t thr = sel ? a.thr_tab[tab_idx] : 0u;
   const double eps = (sel && REPLAY) ? a.eps_tab[tab_idx] : 0.0;
@@ -224,15 +211,6 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
         }
       }
     }
-#ifdef SPGG_LEAN_L1PF   // measured: 648 us per iteration with the L1 prefetches, 614 without (fp64, L=4096) - off
-    // ... and this warp's first row of this tile on its way into L1 while the tile is staged
-    auto prefetch_row_l1 = [&](int rr) {
-      constexpr int kLines = TC * 4 * (int)sizeof(QT) / 128;       // 128-byte lines of a 128-site row segment
-      if (lane < kLines && r0 + rr < g.rows && c0 + lane * (TC / kLines) < g.L)
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(Qp + ((long long)(r0 + rr) * g.L + c0) * 4 + lane * (128 / (int)sizeof(QT))));
-    };
-    prefetch_row_l1(warp);
-#endif
     // ---- stage the halo'd tiles: reward codes (+ their rewards), reputations, cooperator flags
     stage_tile<Md, M, true>(g, r0, c0, code_in, R_in, S_in, rc, sm_tab, vtab, sm_val, sm_code, sm_R, sm_C);
     __syncthreads();
@@ -264,23 +242,8 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
       constexpr bool INTERIOR = decltype(interiorc)::value;
       const int i = r0 + rr;
       const int sr = rr + HR;
-#ifdef SPGG_LEAN_L1PF
-      if (rr + nw < g.TR) prefetch_row_l1(rr + nw);    // the warp's next row
-#endif
       uint32_t w4[4] = {0, 0, 0, 0};
-      if (sel && !REPLAY) {
-        // counter = (column / 4, global row, iteration, 0), as in k_step
-        uint32_t wc[4];
-        philox4x32_10((uint32_t)((c0 >> 2) + lane), (uint32_t)(g.row0 + i), (uint32_t)(a.j + 1), 0u,
-                      rc.seed_lo, rc.seed_hi, wc);
-#pragma unroll
-        for (int k4 = 0; k4 < 4; ++k4) {
-          const int src = 8 * k4 + (lane >> 2);
-          const uint32_t x0 = __shfl_sync(0xffffffffu, wc[0], src), x1 = __shfl_sync(0xffffffffu, wc[1], src);
-          const uint32_t x2 = __shfl_sync(0xffffffffu, wc[2], src), x3 = __shfl_sync(0xffffffffu, wc[3], src);
-          w4[k4] = sel4<uint32_t>(lane & 3, x0, x1, x2, x3);
-        }
-      }
+      if (sel && !REPLAY) philox_row(c0, g.row0 + i, (uint32_t)(a.j + 1), 0u, rc, lane, w4);
       // ---- everything that comes from global memory for a batch of sites, before the first is processed
 // (measured at L=4096 in fp64: batches of 4 sites 648 us per iteration, pairs 630)
 #ifndef SPGG_LEAN_BATCH
@@ -289,9 +252,9 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
 #pragma unroll
       for (int kb = 0; kb < 4; kb += SPGG_LEAN_BATCH) {
       QT q[4][4];
-      double ru[4] = {0, 0, 0, 0};
-      uint8_t rb[4] = {0, 0, 0, 0};
-      double rat[4] = {0, 0, 0, 0};   // fp64: ratio statistic of the site's code (second table column)
+      [[maybe_unused]] double ru[4] = {0, 0, 0, 0};    // replayed draws
+      [[maybe_unused]] uint8_t rb[4] = {0, 0, 0, 0};
+      [[maybe_unused]] double rat[4] = {0, 0, 0, 0};   // fp64: ratio statistic of the site's code (second table column)
       const long long site_row = (long long)i * g.L + c0 + lane;
 #pragma unroll
       for (int k4 = kb; k4 < kb + SPGG_LEAN_BATCH; ++k4) {
@@ -339,17 +302,9 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
           const int act = coop ^ 1;
           const Val vx = sm_val[sidx];
           // neighbour-aware term inputs: spgg.py:486-494 (first arg-max wins)
-          Val best = Val(0);
-          int bidx = sidx, kstar = 0;
-#pragma unroll
-          for (int k = 0; k < NK; ++k) {
-            const int nidx = (sr - c_off[k][0]) * SMW + (sc - c_off[k][1]);
-            const Val vk = sm_val[nidx];
-            Val d;
-            if constexpr (Md::kFp64) d = __dsub_rn(vk, vx);
-            else d = __fsub_rn(vk, vx);
-            if (k == 0 || d > best) { best = d; bidx = nidx; kstar = k; }
-          }
+          const auto bn = best_neighbour<Md, M>(sm_val, sr, sc, vx);
+          const Val best = bn.d;
+          const int bidx = bn.idx, kstar = bn.k;
           const bool same = (((sm_code[bidx] >> 1) & 1u) == (unsigned)coop);
           const int e = 2 * s + act;
           const QT qe = sel4<QT>(e, q0_, q1_, q2_, q3_);
@@ -380,17 +335,8 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
             pk_sn += (unsigned long long)sigma_n_of_code(code) << (16 * (wasC * 2 + coop));
             if (coop) sumRatio += rat[k4];
           } else {
-            const float mx = fmaxf(na, nb);
-            const float td = __fsub_rn(__fmaf_rn(rc.gamma_f, mx, vx), qe);
-            const float qtd = __fmaf_rn(rc.alpha_f, td, qe);
-            const float lam = __fmul_rn(__fmul_rn(rc.kappa_f, fmaxf(0.0f, best)), inv_den);
-            const float nu = same ? lam : -lam;
-            const float na2 = (s_new == s && act == 0) ? qtd : na;
-            const float nb2 = (s_new == s && act == 1) ? qtd : nb;
-            const float td2 = __fsub_rn(__fmaf_rn(rc.gamma_f, fmaxf(na2, nb2), vx), qtd);
-            qfin = __fadd_rn(qtd, nu);
-            const float an = fabsf(nu);
-            tni = __fmaf_rn(__fdividef(an, __fadd_rn(__fadd_rn(fabsf(__fmul_rn(rc.alpha_f, td2)), an), 1e-8f)), 100.0f, tni);
+            auto next_value = [](float x0, float x1, bool) { return fmaxf(x0, x1); };
+            qfin = td_update_f32(rc, vx, qe, na, nb, s, s_new, act, best, same, inv_den, next_value, tni);
             pk_sn += (unsigned long long)(code >> 3) << (16 * (wasC * 2 + coop));
             if (rc.has_ratio && coop) tratio += sm_ratio[code >> 1];
           }

@@ -2,7 +2,8 @@
 iteration as k_step - reference spgg.py:368-592 with algorithms.py:96-133 - with the TD rule compiled
 in, the fp64 rewards looked up instead of divided and the Q entries of a row loaded ahead.  Same
 thread <-> site mapping, same arithmetic, same summation order: strategies, reputations, Q-tables AND
-every statistics column must be bit-identical to k_step (SPGG_NO_LEAN=1)."""
+every statistics column must be bit-identical to k_step (SPGG_NO_LEAN=1).  Both arms run the same
+global-maximum kernel, k_gmax_lean, which the oracle tests pin directly (column 33 of the replays)."""
 import numpy as np
 import pytest
 
