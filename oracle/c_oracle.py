@@ -19,11 +19,14 @@ NSTAT = 40
 ST = dict(NC_OLD=0, N_CD=1, N_DC=2, NC_NEW=3, SUM_P=4, SUM_P_C=5, SUM_P_D=6, SUM_WP_P=7,
           SUM_REW_C=8, SUM_REW_D=9, SUM_RATIO=10, GROUP0=11, SUM_R=17, SUM_Q=18,
           SUM_Q_C=22, SUM_Q_D=26, SUM_NI=30, N_BEST_POS=31, N_BEST_2ND=32, GMAX=33)
+# TD rule codes (include/spgg.h: SPGG_ALGO_*) and the draw pairs each consumes per iteration
+ALGOS = {"qlearning": 0, "sarsa": 1, "expected_sarsa": 2, "double_qlearning": 3}
+PAIRS = {0: 1, 1: 3, 2: 1, 3: 2}
 
 
 class OracleParams(C.Structure):
     _fields_ = [("L", C.c_int32), ("M", C.c_int32), ("state_mode", C.c_int32),
-                ("reserved", C.c_int32),
+                ("algorithm", C.c_int32),
                 ("r", C.c_double), ("c", C.c_double), ("cost", C.c_double),
                 ("alpha", C.c_double), ("gamma", C.c_double), ("kappa", C.c_double),
                 ("lambda_eps", C.c_double), ("rep_gain_C", C.c_double),
@@ -32,9 +35,9 @@ class OracleParams(C.Structure):
 
 
 def build(force: bool = False) -> str:
-    src = os.path.join(_HERE, "spgg_oracle.c")
-    if force or not os.path.exists(_LIB_PATH) or (
-            os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(_LIB_PATH)):
+    srcs = [os.path.join(_HERE, f) for f in ("spgg_oracle.c", "spgg_oracle.h")]
+    if force or not os.path.exists(_LIB_PATH) or any(
+            os.path.exists(s) and os.path.getmtime(s) > os.path.getmtime(_LIB_PATH) for s in srcs):
         subprocess.check_call(["make", "-C", _HERE, "-s", "libspgg_oracle.so"])
     return _LIB_PATH
 
@@ -55,6 +58,8 @@ def lib():
                            C.c_double, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32,
                            C.c_uint32, dp]
         _lib.oracle_philox4x32_10.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        _lib.oracle_site_word.restype = C.c_uint32
+        _lib.oracle_site_word.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, C.c_int]
         _lib.oracle_thr24.restype = C.c_uint32
         _lib.oracle_thr24.argtypes = [C.c_double]
         _lib.oracle_reward_table.argtypes = [C.POINTER(OracleParams), C.c_void_p]
@@ -67,7 +72,8 @@ def params_from_dict(p: dict) -> OracleParams:
     return OracleParams(
         L=int(p["L"]), M=2 if p.get("use_second_order", True) else 1,
         state_mode=1 if p.get("state_representation", "reputation") == "action" else 0,
-        reserved=0, r=float(p["r"]), c=float(p.get("c", 1)), cost=float(p.get("cost", 0.5)),
+        algorithm=ALGOS[str(p.get("algorithm", "qlearning")).lower()],
+        r=float(p["r"]), c=float(p.get("c", 1)), cost=float(p.get("cost", 0.5)),
         alpha=float(p.get("alpha", 0.1)), gamma=float(p.get("gamma", 0.9)),
         kappa=float(p.get("influence_factor", 1.0)),
         lambda_eps=float(p.get("lambda_epsilon", 0.01)),
@@ -84,6 +90,11 @@ def philox(ctr, key):
     return out
 
 
+def site_word(seed: int, step: int, stream: int, i: int, j: int) -> int:
+    """The Philox word the step functions draw for site (i, j) (spgg_oracle.h)."""
+    return int(lib().oracle_site_word(int(seed), int(step), int(stream), int(i), int(j)))
+
+
 def thr24(eps: float) -> int:
     return int(lib().oracle_thr24(float(eps)))
 
@@ -98,17 +109,23 @@ def reward_table(p: dict) -> np.ndarray:
 class Sim:
     """Stateful driver: holds S (uint8), R, Q and steps them with either
     arithmetic.  ``precision`` = 'fp64' (reference order) or 'fp32'
-    (throughput-mode arithmetic)."""
+    (throughput-mode arithmetic).  ``p['algorithm']`` picks the TD rule; Double
+    Q-learning holds both tables, ``Q`` of shape (L, L, 2, 2, 2) laid out
+    [site][table][s][a] like ``Engine.get_state``."""
 
     def __init__(self, p: dict, S0, R0, Q0, precision="fp64", seed=0):
         self.p = dict(p)
         self.op = params_from_dict(p)
         self.L = int(p["L"])
         self.precision = precision
+        self.pairs = PAIRS[self.op.algorithm]
         ft = np.float64 if precision == "fp64" else np.float32
         self.S = np.ascontiguousarray(np.asarray(S0) != 0, dtype=np.uint8)
-        self.R = np.ascontiguousarray(R0, dtype=ft)
-        self.Q = np.ascontiguousarray(np.asarray(Q0).reshape(self.L, self.L, 2, 2), dtype=ft)
+        self.R = np.array(R0, dtype=ft, order="C")          # copies: the caller's arrays stay as they are
+        qshape = (self.L, self.L, 2, 2, 2) if self.op.algorithm == 3 else (self.L, self.L, 2, 2)
+        if np.asarray(Q0).size != np.prod(qshape):
+            raise ValueError(f"Q0 must hold {qshape} values for this TD rule")
+        self.Q = np.array(np.asarray(Q0).reshape(qshape), dtype=ft, order="C")
         self.eps = float(p.get("epsilon", 0.5))
         self.decay = float(p.get("epsilon_decay", 0.995))
         self.eps_min = float(p.get("epsilon_min", 0.01))
@@ -116,13 +133,24 @@ class Sim:
         self.t = 0
         self.fn = lib().oracle_step_f64 if precision == "fp64" else lib().oracle_step_f32
 
+    @property
+    def q_combined(self):
+        """The table the policy acts on: Q itself, or the mean of Double Q's two tables."""
+        if self.Q.ndim == 5:
+            return (self.Q[:, :, 0] + self.Q[:, :, 1]) / self.Q.dtype.type(2)
+        return self.Q
+
     def step(self, u=None, b=None):
-        """One iteration; returns the stat row (NSTAT doubles)."""
+        """One iteration; returns the stat row (NSTAT doubles).  Replayed draws: ``u``, ``b`` of
+        shape (L, L), or (pairs, L, L) with the pairs the TD rule consumes (SARSA 3, Double Q 2:
+        u of pair 1 chooses the table, spgg_oracle.h)."""
         self.t += 1
         st = np.zeros(NSTAT)
         if u is not None:
             u = np.ascontiguousarray(u, np.float64)
             b = np.ascontiguousarray(b, np.uint8)
+            if u.size != self.pairs * self.L * self.L or b.size != u.size:
+                raise ValueError(f"this TD rule consumes {self.pairs} draw pair(s) per iteration")
             up, bp = u.ctypes.data, b.ctypes.data
         else:
             up = bp = None
@@ -134,7 +162,7 @@ class Sim:
         return st
 
     def run(self, n, draws=None):
-        """``draws(t, L) -> (u, b)`` or None for Philox.  Stops like spgg.py:405
+        """``draws(t, L) -> (u, b)`` (shapes as ``step``) or None for Philox.  Stops like spgg.py:405
         when the lattice is uniform.  Returns the stat rows of completed steps."""
         rows = []
         for _ in range(n):

@@ -4,6 +4,8 @@
  * (reference paths relative to /root/reference):
  *   src/model/spgg.py:368-592   (SPGG.run loop body)
  *   src/model/algorithms.py:96-133 (QLearning.select_action / update_q_table)
+ *   src/model/algorithms.py:136-341 (SARSA, Expected SARSA, Double Q-learning), applied as
+ *   spgg.py:431-473,498-505, in the operation order of oracle/spgg_numpy.py
  * It is the checker for the CUDA path; the product never links or loads it.
  * Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs do.
  *
@@ -17,7 +19,8 @@
  * kernel (fp32 Q, exact-count reward table, explicit fmaf, Philox draws); it
  * has no bit-level counterpart in the reference and is pinned statistically
  * (cooperation-rate curves inside the reference's seed-to-seed band) and
- * against oracle_step_f64 on dyadic parameter sets where both are exact.
+ * against oracle_step_f64 on dyadic parameter sets where both are exact.  For every TD rule
+ * it follows k_step (csrc/spgg_kernels.cuh: td_update_f32 and the Double-Q branch).
  *
  * Build with -ffp-contract=off (see oracle/Makefile): the reference is NumPy,
  * every operation is individually rounded.
@@ -83,15 +86,69 @@ uint32_t oracle_thr24(double eps) {
   return (uint32_t)t;
 }
 
-/* draw word of site (i,j) at iteration `step`: counter = (j>>2, row, step, 0), word index
- * j&3 - one Philox call serves four consecutive sites of a row. */
-static inline uint32_t site_word(uint64_t seed, uint32_t step, int i, int j) {
-  uint32_t ctr[4] = {(uint32_t)(j >> 2), (uint32_t)i, step, 0u};
+/* draw word of site (i,j) at iteration `step` from stream `stream`: counter = (j>>2, row, step,
+ * stream), word index j&3 - one Philox call serves four consecutive sites of a row.  Stream 0 is
+ * the action, streams 1 and 2 the further draws of SARSA and Double Q-learning. */
+static inline uint32_t site_word(uint64_t seed, uint32_t step, uint32_t stream, int i, int j) {
+  uint32_t ctr[4] = {(uint32_t)(j >> 2), (uint32_t)i, step, stream};
   uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
   uint32_t w[4];
   oracle_philox4x32_10(ctr, key, w);
   return w[j & 3];
 }
+
+uint32_t oracle_site_word(uint64_t seed, uint32_t step, uint32_t stream, int i, int j) {
+  return site_word(seed, step, stream, i, j);
+}
+
+/* the update's further draws of site (i,j): SARSA's next actions for the TD target (ex1, rn1)
+ * and for the NI statistic (ex2, rn2), spgg.py:433,452; Double Q's table choice upd1,
+ * algorithms.py:302.  Replayed: pairs 1 and 2 of u, b (n_sites apart).  Philox: streams 1, 2. */
+typedef struct {
+  int ex1, rn1, ex2, rn2, upd1;
+} td_draws_t;
+
+static td_draws_t td_draws(int algo, double eps, const double *u, const uint8_t *b, size_t n_sites,
+                           uint64_t seed, uint32_t step, uint32_t thr24, int i, int j, size_t x) {
+  td_draws_t d = {0, 0, 0, 0, 0};
+  if (algo == OALGO_SARSA) {
+    if (u) {
+      d.ex1 = (u[n_sites + x] < eps); d.rn1 = b[n_sites + x];
+      d.ex2 = (u[2 * n_sites + x] < eps); d.rn2 = b[2 * n_sites + x];
+    } else {
+      const uint32_t w1 = site_word(seed, step, 1u, i, j), w2 = site_word(seed, step, 2u, i, j);
+      d.ex1 = ((w1 >> 8) < thr24); d.rn1 = (int)(w1 & 1u);
+      d.ex2 = ((w2 >> 8) < thr24); d.rn2 = (int)(w2 & 1u);
+    }
+  } else if (algo == OALGO_DOUBLE_QLEARNING) {
+    if (u) d.upd1 = (u[n_sites + x] < 0.5);
+    else d.upd1 = ((site_word(seed, step, 1u, i, j) >> 8) < (1u << 23));
+  }
+  return d;
+}
+
+/* value of the next state's row (x0, x1) in the TD target: max (algorithms.py:125), Q[s',a']
+ * with a' eps-greedy (:142-150,169) or the eps-greedy expectation (:212-224), in the order of
+ * oracle/spgg_numpy.py */
+static double next_f64(int algo, double x0, double x1, double eps, int ex, int rn) {
+  if (algo == OALGO_QLEARNING) return fmax(x0, x1);
+  const int greedy = (x1 > x0) ? 1 : 0;
+  if (algo == OALGO_SARSA) return (ex ? rn : greedy) ? x1 : x0;
+  const double po = eps / 2.0, pg = (1.0 - eps) + po;
+  return (greedy ? po : pg) * x0 + (greedy ? pg : po) * x1;
+}
+
+/* the same in the kernel's fp32 arithmetic (k_step: next_value; epsilon rounded to float once) */
+static float next_f32(int algo, float x0, float x1, float e, int ex, int rn) {
+  if (algo == OALGO_QLEARNING) return fmaxf(x0, x1);
+  const int greedy = (x1 > x0) ? 1 : 0;
+  if (algo == OALGO_SARSA) return (ex ? rn : greedy) ? x1 : x0;
+  const float po = e * 0.5f, pg = (1.0f - e) + po;
+  return fmaf(greedy ? pg : po, x1, (greedy ? po : pg) * x0);
+}
+
+/* k_step's q_max: the first argument on a tie */
+static inline float qmaxf(float x, float y) { return x > y ? x : (y > x ? y : x); }
 
 /* ------------------------------------------------------------ shared bits */
 static void count_groups(int L, const uint8_t *S, uint8_t *N) {
@@ -123,6 +180,7 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q, 
   const double lo = p->r - 5.0;                            /* spgg.py:149 */
   const double span = 4.0 * p->r - lo;                     /* spgg.py:148,377 */
   const double wP = p->wP, wR = 1.0 - p->wP;               /* spgg.py:108 */
+  const int algo = p->algorithm, dq = (algo == OALGO_DOUBLE_QLEARNING), nq = dq ? 8 : 4;
 
   uint8_t *N = (uint8_t *)malloc(n_sites);
   uint8_t *a = (uint8_t *)malloc(n_sites);
@@ -170,12 +228,16 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q, 
         explore = (u[x] < eps);
         rnd = b[x];
       } else {
-        const uint32_t w = site_word(seed, step, i, j);
+        const uint32_t w = site_word(seed, step, 0u, i, j);
         explore = ((w >> 8) < thr24);
         rnd = (int)(w & 1u);
       }
-      const double *q = Q + 4 * x + 2 * s;
-      const int greedy = (q[1] > q[0]) ? 1 : 0; /* np.argmax: first max */
+      const double *q = Q + nq * x + 2 * s;
+      int greedy;
+      if (dq) /* the policy acts on the mean of the two tables (algorithms.py:263,283-290) */
+        greedy = ((q[1] + q[5]) / 2.0 > (q[0] + q[4]) / 2.0) ? 1 : 0;
+      else
+        greedy = (q[1] > q[0]) ? 1 : 0; /* np.argmax: first max */
       a[x] = (uint8_t)(explore ? rnd : greedy);
       double rn = R[x] + (a[x] == 0 ? p->rep_gain_C : -p->delta_R_D); /* spgg.py:321 */
       rn = fmax(rn, p->R_min);
@@ -221,12 +283,8 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q, 
   for (int i = 0; i < L; ++i)
     for (int j = 0; j < L; ++j) {
       const size_t x = (size_t)i * L + j;
-      const int s = s_old[x], sn = s_new[x], act = a[x];
-      double *q = Q + 4 * x;
-      const double q0 = q[2 * s + act];
-      const double mx = fmax(q[2 * sn], q[2 * sn + 1]);
-      const double td = rew[x] + p->gamma * mx - q0; /* algorithms.py:128 */
-      const double qtd = q0 + p->alpha * td;         /* algorithms.py:131 */
+      const int s = s_old[x], sn = s_new[x], act = a[x], e = 2 * s + act;
+      const td_draws_t dr = td_draws(algo, eps, u, b, n_sites, seed, step, thr24, i, j, x);
       double best = 0.0;
       int kstar = 0;
       for (int k = 0; k < nk; ++k) {
@@ -239,11 +297,33 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q, 
       const double lam = p->kappa * fmax(0.0, best) / (gmax + p->lambda_eps); /* spgg.py:489 */
       const int a_star = a[IDX(i - OFF[kstar][0], j - OFF[kstar][1])];
       const double nu = lam * ((a_star == act) ? 1.0 : -1.0);
-      /* NI statistic uses the table after the TD write (spgg.py:446-473,512) */
-      q[2 * s + act] = qtd;
-      const double mx2 = fmax(q[2 * sn], q[2 * sn + 1]);
-      const double td2 = rew[x] + p->gamma * mx2 - qtd;
-      q[2 * s + act] = qtd + nu; /* spgg.py:509 */
+      double *q = Q + nq * x;
+      double td2, qm[4];
+      const double *qs = q; /* the table the statistics see */
+      if (dq) {
+        /* algorithms.py:292-341: the chosen table's target is the other table's row maximum of s' */
+        double *qa = q, *qb = q + 4;
+        const double nxa = fmax(qb[2 * sn], qb[2 * sn + 1]), nxb = fmax(qa[2 * sn], qa[2 * sn + 1]);
+        if (dr.upd1) qa[e] = qa[e] + p->alpha * (rew[x] + p->gamma * nxa - qa[e]);
+        else qb[e] = qb[e] + p->alpha * (rew[x] + p->gamma * nxb - qb[e]);
+        /* TD error of the combined table after the write (spgg.py:464-468) */
+        for (int z = 0; z < 4; ++z) qm[z] = (qa[z] + qb[z]) / 2.0;
+        td2 = rew[x] + p->gamma * fmax(qm[2 * sn], qm[2 * sn + 1]) - qm[e];
+        qa[e] += nu; /* spgg.py:498-505: both tables */
+        qb[e] += nu;
+        for (int z = 0; z < 4; ++z) qm[z] = (qa[z] + qb[z]) / 2.0;
+        qs = qm;
+      } else {
+        const double q0 = q[e];
+        const double mx = next_f64(algo, q[2 * sn], q[2 * sn + 1], eps, dr.ex1, dr.rn1);
+        const double td = rew[x] + p->gamma * mx - q0; /* algorithms.py:128 */
+        const double qtd = q0 + p->alpha * td;         /* algorithms.py:131 */
+        /* NI statistic uses the table after the TD write (spgg.py:446-473,512) */
+        q[e] = qtd;
+        const double mx2 = next_f64(algo, q[2 * sn], q[2 * sn + 1], eps, dr.ex2, dr.rn2);
+        td2 = rew[x] + p->gamma * mx2 - qtd;
+        q[e] = qtd + nu; /* spgg.py:509 */
+      }
       const double pct = fabs(nu) / (fabs(p->alpha * td2) + fabs(nu) + 1e-8) * 100.0;
 
       const int wasC = (S[x] == 0);
@@ -257,9 +337,9 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q, 
       acc_st[act == 0 ? OST_SUM_REW_C : OST_SUM_REW_D] += rew[x];
       if (act == 0) acc_st[OST_SUM_RATIO] += fabs(wR * 0.5) / (fabs(rew[x]) + 1e-9) * 100.0;
       acc_st[OST_SUM_R] += R[x];
-      for (int e = 0; e < 4; ++e) {
-        acc_st[OST_SUM_Q + e] += q[e];
-        acc_st[(wasC ? OST_SUM_Q_C : OST_SUM_Q_D) + e] += q[e];
+      for (int z = 0; z < 4; ++z) {
+        acc_st[OST_SUM_Q + z] += qs[z];
+        acc_st[(wasC ? OST_SUM_Q_C : OST_SUM_Q_D) + z] += qs[z];
       }
       acc_st[OST_SUM_NI] += pct;
       if (best > 0.0) {
@@ -312,6 +392,7 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
   const float gainC = (float)p->rep_gain_C, lossD = (float)p->delta_R_D;
   const float rmin = (float)p->R_min, rmax = (float)p->R_max;
   const double wP = p->wP, wR = 1.0 - p->wP;
+  const int algo = p->algorithm, dq = (algo == OALGO_DOUBLE_QLEARNING), nq = dq ? 8 : 4;
   float tab[128];
   oracle_reward_table(p, tab);
 
@@ -351,12 +432,16 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
         explore = (u[x] < eps);
         rnd = b[x];
       } else {
-        const uint32_t w = site_word(seed, step, i, j);
+        const uint32_t w = site_word(seed, step, 0u, i, j);
         explore = ((w >> 8) < thr24);
         rnd = (int)(w & 1u);
       }
-      const float *q = Q + 4 * x + 2 * s;
-      const int greedy = (q[1] > q[0]) ? 1 : 0;
+      const float *q = Q + nq * x + 2 * s;
+      int greedy;
+      if (dq) /* k_step's q_mean of the two tables */
+        greedy = ((q[1] + q[5]) / 2.0f > (q[0] + q[4]) / 2.0f) ? 1 : 0;
+      else
+        greedy = (q[1] > q[0]) ? 1 : 0;
       a[x] = (uint8_t)(explore ? rnd : greedy);
       float rn = R[x] + (a[x] == 0 ? gainC : -lossD);
       rn = fmaxf(rn, rmin);
@@ -397,12 +482,8 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
   for (int i = 0; i < L; ++i)
     for (int j = 0; j < L; ++j) {
       const size_t x = (size_t)i * L + j;
-      const int s = s_old[x], sn = s_new[x], act = a[x];
-      float *q = Q + 4 * x;
-      const float q0 = q[2 * s + act];
-      const float mx = fmaxf(q[2 * sn], q[2 * sn + 1]);
-      const float td = fmaf(gamma, mx, rew[x]) - q0;
-      const float qtd = fmaf(alpha, td, q0);
+      const int s = s_old[x], sn = s_new[x], act = a[x], e = 2 * s + act;
+      const td_draws_t dr = td_draws(algo, eps, u, b, n_sites, seed, step, thr24, i, j, x);
       float best = 0.0f;
       int kstar = 0;
       for (int k = 0; k < nk; ++k) {
@@ -415,10 +496,33 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
       const float lam = (kappa * fmaxf(0.0f, best)) * inv_den;
       const int a_star = a[IDX(i - OFF[kstar][0], j - OFF[kstar][1])];
       const float nu = (a_star == act) ? lam : -lam;
-      q[2 * s + act] = qtd;
-      const float mx2 = fmaxf(q[2 * sn], q[2 * sn + 1]);
-      const float td2 = fmaf(gamma, mx2, rew[x]) - qtd;
-      q[2 * s + act] = qtd + nu;
+      float *q = Q + nq * x;
+      float td2, qm[4];
+      const float *qs = q; /* the table the statistics see */
+      if (dq) {
+        /* k_step's Double-Q branch: separately rounded products and sums, means by division */
+        float *t1 = q, *t2 = q + 4;
+        const float nx1 = qmaxf(t2[2 * sn], t2[2 * sn + 1]), nx2 = qmaxf(t1[2 * sn], t1[2 * sn + 1]);
+        if (dr.upd1) t1[e] = t1[e] + alpha * ((rew[x] + gamma * nx1) - t1[e]);
+        else t2[e] = t2[e] + alpha * ((rew[x] + gamma * nx2) - t2[e]);
+        for (int z = 0; z < 4; ++z) qm[z] = (t1[z] + t2[z]) / 2.0f;
+        td2 = (rew[x] + gamma * qmaxf(qm[2 * sn], qm[2 * sn + 1])) - qm[e];
+        t1[e] = t1[e] + nu;
+        t2[e] = t2[e] + nu;
+        for (int z = 0; z < 4; ++z) qm[z] = (t1[z] + t2[z]) / 2.0f;
+        qs = qm;
+      } else {
+        /* td_update_f32 */
+        const float ef = (float)eps;
+        const float q0 = q[e];
+        const float mx = next_f32(algo, q[2 * sn], q[2 * sn + 1], ef, dr.ex1, dr.rn1);
+        const float td = fmaf(gamma, mx, rew[x]) - q0;
+        const float qtd = fmaf(alpha, td, q0);
+        q[e] = qtd;
+        const float mx2 = next_f32(algo, q[2 * sn], q[2 * sn + 1], ef, dr.ex2, dr.rn2);
+        td2 = fmaf(gamma, mx2, rew[x]) - qtd;
+        q[e] = qtd + nu;
+      }
       const double pct =
           (double)fabsf(nu) / ((double)fabsf(alpha * td2) + (double)fabsf(nu) + 1e-8) * 100.0;
 
@@ -435,9 +539,9 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
       acc_st[act == 0 ? OST_SUM_REW_C : OST_SUM_REW_D] += rewd;
       if (act == 0) acc_st[OST_SUM_RATIO] += fabs(wR * 0.5) / (fabs(rewd) + 1e-9) * 100.0;
       acc_st[OST_SUM_R] += R[x];
-      for (int e = 0; e < 4; ++e) {
-        acc_st[OST_SUM_Q + e] += q[e];
-        acc_st[(wasC ? OST_SUM_Q_C : OST_SUM_Q_D) + e] += q[e];
+      for (int z = 0; z < 4; ++z) {
+        acc_st[OST_SUM_Q + z] += qs[z];
+        acc_st[(wasC ? OST_SUM_Q_C : OST_SUM_Q_D) + z] += qs[z];
       }
       acc_st[OST_SUM_NI] += pct;
       if (best > 0.0f) {

@@ -35,11 +35,14 @@ enum {
   OST_NSTAT = 40
 };
 
+/* TD rules: the codes of include/spgg.h (SPGG_ALGO_*) */
+enum { OALGO_QLEARNING = 0, OALGO_SARSA = 1, OALGO_EXPECTED_SARSA = 2, OALGO_DOUBLE_QLEARNING = 3 };
+
 typedef struct {
   int32_t L;
   int32_t M;          /* 1 or 2 (use_second_order)           */
   int32_t state_mode; /* 0 = reputation, 1 = action          */
-  int32_t reserved;
+  int32_t algorithm;  /* OALGO_*                             */
   double r, c, cost;
   double alpha, gamma;
   double kappa;       /* influence_factor                    */
@@ -49,11 +52,20 @@ typedef struct {
 } oracle_params_t;
 
 /* One iteration, fp64, reference operation order, replayed draws.
- * S: L*L bytes (0=C, 1=D); R: L*L doubles; Q: L*L*4 doubles laid out (s,a).
- * u,b: that iteration's draw arrays (algorithms.py:105,108).
- * If u == NULL the draws come from Philox4x32-10 (seed, step) with the
- * integer threshold thr24 (explore <=> (word>>8) < thr24; random action = word&1).
- * stats: OST_NSTAT doubles (may be NULL). Returns 0. */
+ * S: L*L bytes (0=C, 1=D); R: L*L doubles; Q: L*L*4 doubles laid out (s,a), or for
+ * Double Q-learning L*L*8 laid out (table,s,a), the two tables of a site side by side.
+ * u,b: that iteration's draw pairs, pair k at u + k*L*L (algorithms.py:105,108).  Q-learning
+ * and Expected SARSA draw one pair; SARSA three (action, next action of the update, next
+ * action of the NI statistic: spgg.py:410,433,452); Double Q-learning two, the table choice
+ * being u of pair 1 (update table 1 <=> u < 0.5, algorithms.py:302).
+ * If u == NULL the draws come from Philox4x32-10 with the integer threshold thr24
+ * (explore <=> (word>>8) < thr24; random action = word&1): the action from counter
+ * (j/4, i, step, 0), SARSA's next actions from (j/4, i, step, 1) and (j/4, i, step, 2),
+ * Double Q's table choice from (j/4, i, step, 1) (table 1 <=> (word>>8) < 2^23).
+ * eps / thr24 are those of iteration `step`: the select and SARSA's / Expected SARSA's
+ * policy of the next state use the same epsilon.
+ * stats: OST_NSTAT doubles (may be NULL); the Q sums are over the mean of the two tables
+ * for Double Q-learning (algorithms.py:263). Returns 0. */
 int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q,
                     double eps, const double *u, const uint8_t *b,
                     uint64_t seed, uint32_t step, uint32_t thr24, double *stats);
@@ -61,13 +73,17 @@ int oracle_step_f64(const oracle_params_t *p, uint8_t *S, double *R, double *Q,
 /* One iteration with the throughput-mode arithmetic: fp32 Q, fp32 R, rewards
  * from the integer table rew[SigmaN][C_old][coop_new] (exact-count payoff),
  * explicit fmaf, Philox draws (or replayed u,b when u != NULL; u compared in
- * double against eps). */
+ * double against eps).  Draws, Q layout and TD rules as oracle_step_f64. */
 int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q,
                     double eps, const double *u, const uint8_t *b,
                     uint64_t seed, uint32_t step, uint32_t thr24, double *stats);
 
 /* Philox4x32-10, exposed for known-answer tests. */
 void oracle_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
+
+/* the Philox word both step functions draw for site (i,j) at iteration `step` from stream
+ * `stream` (0: action, 1 and 2: SARSA's next actions, 1: Double Q's table choice) */
+uint32_t oracle_site_word(uint64_t seed, uint32_t step, uint32_t stream, int i, int j);
 
 /* explore threshold used by both implementations: ceil(eps * 2^24) clamped to [0, 2^24] */
 uint32_t oracle_thr24(double eps);

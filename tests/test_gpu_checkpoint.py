@@ -18,6 +18,11 @@ CASES = [
     ("fast_tma_m2_action", dict(C2, L=256), "fp32", {"SPGG_NO_RESIDENT": "1"}, "fast"),
     ("general_fp32", dict(C1, L=100), "fp32", {"SPGG_NO_RESIDENT": "1"}, "general"),
     ("general_fp64", dict(C2, L=48), "fp64", {}, "general"),
+    # the other TD rules run on k_step only; Double Q-learning checkpoints both tables
+    ("sarsa_fp32", dict(C1, L=100, algorithm="sarsa"), "fp32", {}, "general"),
+    ("expected_sarsa_fp64", dict(C2, L=48, algorithm="expected_sarsa"), "fp64", {}, "general"),
+    ("double_q_fp32", dict(C1, L=100, algorithm="double_qlearning"), "fp32", {}, "general"),
+    ("double_q_fp64", dict(C2, L=48, algorithm="double_qlearning"), "fp64", {}, "general"),
 ]
 
 
@@ -28,13 +33,13 @@ def test_resume_is_bit_identical(monkeypatch, name, p, precision, env, path):
         monkeypatch.setenv(k, v)
     p = full_params(p)
     L, n, k = p["L"], 100, 50
+    one = spgg_b200.Engine(p, seeds=31, precision=precision)
+    assert one.describe().startswith(path), one.describe()
     rs = np.random.RandomState(9)
-    Q0 = rs.uniform(-0.01, 0.01, (L, L, 2, 2))
+    Q0 = rs.uniform(-0.01, 0.01, (L, L, one.nq))   # Double Q-learning: both tables, [site][table][s][a]
     S0 = rs.randint(0, 2, (L, L))
     R0 = np.zeros((L, L))
 
-    one = spgg_b200.Engine(p, seeds=31, precision=precision)
-    assert one.describe().startswith(path), one.describe()
     one.set_state(S0, R0, Q0)
     one.step(k)
     one.step(n - k)

@@ -66,6 +66,8 @@ def test_fp64_replay_vs_oracle(state, second, L):
     assert np.array_equal(rows[:, ints], rows_o[:, ints])
     assert np.array_equal(rows[:, 33], rows_o[:, 33])  # gmax is an exact max
     np.testing.assert_allclose(rows[:, 4:11], rows_o[:, 4:11], rtol=1e-10, atol=1e-9)
+    # sum of R before the action: recorded by the launch that chooses the action, one row earlier
+    np.testing.assert_allclose(eng.stats()[:-1, 17], rows_o[:, 17], rtol=1e-10, atol=1e-9)
     np.testing.assert_allclose(rows[:, 18:31], rows_o[:, 18:31], rtol=1e-9, atol=1e-9)
     eng.close()
 
@@ -150,6 +152,11 @@ def test_fp32_philox_vs_oracle_bit_exact(monkeypatch, name, p):
     assert np.array_equal(rows[:, ints], rows_o[:, ints])
     assert np.array_equal(rows[:, 33].astype(np.float32), rows_o[:, 33].astype(np.float32))
     np.testing.assert_allclose(rows[:, 4:11], rows_o[:, 4:11], rtol=1e-6, atol=1e-6)
+    sum_r = eng.stats()[:-1, 17]   # sum of R before the action: recorded by the launch that chooses it
+    if eng.status().r_is_int8:
+        assert np.array_equal(sum_r, rows_o[:, 17])   # integer units, scaled once
+    else:
+        np.testing.assert_allclose(sum_r, rows_o[:, 17], rtol=1e-6, atol=1e-6 * L * L)
     np.testing.assert_allclose(rows[:, 18:31], rows_o[:, 18:31], rtol=1e-4, atol=1e-3)
     eng.close()
 
@@ -205,31 +212,62 @@ def test_fp32_replay_draws_vs_oracle():
     eng.close()
 
 
-@pytest.mark.parametrize("path", ["resident", "per_iteration"])
-def test_chunking_is_invisible(monkeypatch, path):
+CHUNK_CASES = [("resident", "qlearning", "philox")] + [
+    ("per_iteration", algo, draws) for algo in ("qlearning", "sarsa", "expected_sarsa", "double_qlearning")
+    for draws in ("philox", "replay")]
+
+
+@pytest.mark.parametrize("path,algorithm,draws", CHUNK_CASES, ids=["-".join(c) for c in CHUNK_CASES])
+def test_chunking_is_invisible(monkeypatch, path, algorithm, draws):
     """step(7)+step(13) == step(20): the counter-based stream and the skewed pipeline do not
-    depend on where the host cuts the run."""
+    depend on where the host cuts the run - for every TD rule, with Philox draws or with the
+    replayed draw pairs re-armed at every chunk (SARSA's and Double Q's further pairs feed the
+    update launched in the next call)."""
     if path == "per_iteration":
         monkeypatch.setenv("SPGG_NO_RESIDENT", "1")
     L = 160
-    p = full_params(dict(C1, L=L, use_second_order=True))
+    p = full_params(dict(C1, L=L, use_second_order=True, algorithm=algorithm))
     rs = np.random.RandomState(9)
-    Q0 = rs.uniform(-0.01, 0.01, (L, L, 2, 2))
+    nq = 8 if algorithm == "double_qlearning" else 4
+    Q0 = rs.uniform(-0.01, 0.01, (L, L, nq))
     S0 = rs.randint(0, 2, (L, L))
+    pairs = {"sarsa": 3, "double_qlearning": 2}.get(algorithm, 1)
+    u = rs.rand(20, pairs, L, L)
+    b = rs.randint(0, 2, (20, pairs, L, L)).astype(np.uint8)
     outs = []
+    mixed = False
     for chunks in ((20,), (7, 13), (1,) * 20):
         eng = _engine(p, seeds=99, precision="fp32")
+        if algorithm != "qlearning":
+            assert eng.describe().endswith("k_step) (fp32 Q, int8 R)"), eng.describe()
+        # replayed selects run on the general kernel; on the fast path a chunk's closing update (no select)
+        # then runs k_step_fast, so where the chunks end decides which kernel folds an iteration's statistics
+        mixed = draws == "replay" and eng.describe().startswith("fast")
         eng.set_state(S0, np.zeros((L, L)), Q0)
         rows = []
+        t0 = 0
         for c in chunks:
+            if draws == "replay":
+                if pairs == 1:
+                    eng.set_replay(u[t0:t0 + c, 0], b[t0:t0 + c, 0])
+                else:
+                    eng.set_replay(u[t0:t0 + c], b[t0:t0 + c])
             eng.step(c)
+            t0 += c
             rows.append(eng.stats()[1:])
         outs.append(eng.get_state() + (np.vstack(rows),))
         assert eng.status().iteration == 20
         eng.close()
     for o in outs[1:]:
         for a, b in zip(outs[0], o):
-            assert np.array_equal(a, b)
+            if mixed and a.ndim == 2 and a.shape[1] == 40:
+                # as in test_fast_path_equals_general_path: the two layouts group fp32 partial sums differently
+                exact = [c for c in range(18) if c != 10] + [31, 32, 33]
+                assert np.array_equal(a[:, exact], b[:, exact])
+                np.testing.assert_allclose(a[:, 10], b[:, 10], rtol=1e-5, atol=1e-4)
+                np.testing.assert_allclose(a[:, 18:31], b[:, 18:31], rtol=1e-5, atol=1e-4)
+            else:
+                assert np.array_equal(a, b)
 
 
 def test_batched_replicas_equal_single_runs(monkeypatch):
@@ -341,6 +379,7 @@ def test_L4096_32_iterations_vs_oracle_and_invariants():
     assert np.array_equal(rows[:, ints], rows_o[:, ints])
     assert np.array_equal(rows[:, 33].astype(np.float32), rows_o[:, 33].astype(np.float32))  # exact max
     np.testing.assert_allclose(rows[:, 4:11], rows_o[:, 4:11], rtol=1e-5)
+    assert np.array_equal(eng.stats()[:-1, 17], rows_o[:, 17])   # sum of R before the action: int8 units, scaled once
     np.testing.assert_allclose(rows[:, 18:31], rows_o[:, 18:31], rtol=2e-4, atol=1e-2)
     eng.step(40)
     rows = eng.stats()

@@ -43,18 +43,28 @@ def test_numpy_oracle_reproduces_reference_bit_for_bit(golden_dir, name):
         assert np.array_equal(out["snapshots"][10][1], z["ds_Sn_snapshot_10"])
 
 
-@pytest.mark.parametrize("name", GOLDEN)
+TD_GOLDEN = ["sarsa_rep_m1", "sarsa_act_m2", "expsarsa_rep_m2", "expsarsa_act_m1"]
+DQ_GOLDEN = ["doubleq_rep_m1", "doubleq_act_m2"]
+
+
+@pytest.mark.parametrize("name", GOLDEN + TD_GOLDEN + DQ_GOLDEN)
 def test_c_oracle_fp64_reproduces_reference_bit_for_bit(golden_dir, name):
+    """Every TD rule: S, R, Q (both Double-Q tables and their mean) and the integer series."""
     from oracle import c_oracle
     z, p = load_golden(golden_dir, name)
     p = full_params(p)
     L, n = p["L"], int(z["u"].shape[0])
-    sim = c_oracle.Sim(p, z["s0"], np.zeros((L, L)), z["q0"], "fp64")
-    rows = sim.run(n, _draws(z))
+    dq = p.get("algorithm") == "double_qlearning"
+    Q0 = np.stack([z["q1_0"], z["q2_0"]], axis=2) if dq else z["q0"]
+    sim = c_oracle.Sim(p, z["s0"], np.zeros((L, L)), Q0, "fp64")
+    rows = sim.run(n, lambda t, L_: (z["u"][t - 1], z["b"][t - 1]))
     assert rows.shape[0] == n
     assert np.array_equal(sim.S, z["s_final"])
     assert np.array_equal(sim.R, z["r_final"])
-    assert np.array_equal(sim.Q, z["q_final"])
+    if dq:
+        assert np.array_equal(sim.Q[:, :, 0], z["q1_final"])
+        assert np.array_equal(sim.Q[:, :, 1], z["q2_final"])
+    assert np.array_equal(sim.q_combined, z["q_final"])
     ST = c_oracle.ST
     assert np.array_equal(rows[:, ST["N_CD"]].astype(np.int64), z["ds_switch_C_to_D"])
     assert np.array_equal(rows[:, ST["N_DC"]].astype(np.int64), z["ds_switch_D_to_C"])
@@ -203,6 +213,109 @@ def test_c_oracle_fp32_follows_fp64_on_short_horizons():
     np.testing.assert_allclose(c.Q, a.Q, rtol=0, atol=2e-2)
 
 
+@pytest.mark.parametrize("algo", ["sarsa", "expected_sarsa", "double_qlearning"])
+def test_c_oracle_fp32_td_rules_follow_fp64_on_short_horizons(algo):
+    """As above for the other TD rules, with the draw pairs each consumes (SARSA three, Double Q
+    two): the fp32 restatement of k_step stays within the fp64 reference order on 3 steps."""
+    from oracle import c_oracle
+    L, n = 32, 3
+    p = full_params(dict(L=L, r=3.0, cost=1, alpha=0.8, epsilon_decay=0.99, influence_factor=1.0,
+                         use_second_order=False, reward_weight_payoff=0.95, rep_gain_C=1.0,
+                         algorithm=algo))
+    pairs = c_oracle.PAIRS[c_oracle.ALGOS[algo]]
+    rs = np.random.RandomState(11)
+    Q0 = rs.uniform(-0.01, 0.01, (L, L, 2, 2, 2) if algo == "double_qlearning" else (L, L, 2, 2))
+    S0 = rs.randint(0, 2, (L, L))
+    u = rs.rand(n, pairs, L, L)
+    b = rs.randint(0, 2, (n, pairs, L, L)).astype(np.uint8)
+    a = c_oracle.Sim(p, S0, np.zeros((L, L)), Q0, "fp64")
+    c = c_oracle.Sim(p, S0, np.zeros((L, L)), Q0, "fp32")
+    a.run(n, lambda t, L_: (u[t - 1], b[t - 1]))
+    c.run(n, lambda t, L_: (u[t - 1], b[t - 1]))
+    assert (a.S != c.S).mean() < 0.02
+    np.testing.assert_allclose(c.Q, a.Q, rtol=0, atol=2e-2)
+    assert np.abs(c.Q - a.Q).max() > 0                  # the two arithmetics are distinct
+    np.testing.assert_allclose(c.q_combined, a.q_combined, rtol=0, atol=2e-2)
+
+
+@pytest.mark.parametrize("algo", ["qlearning", "sarsa", "expected_sarsa", "double_qlearning"])
+@pytest.mark.parametrize("L,second,state", [(37, False, "reputation"), (37, True, "action"),
+                                            (64, True, "reputation"), (64, False, "action")])
+def test_c_oracle_fp64_equals_numpy_oracle_for_every_td_rule(algo, L, second, state):
+    """oracle_step_f64 restates oracle/spgg_numpy.py (pinned to the reference above) for every TD
+    rule: S, R, Q (both Double-Q tables) and the integer series bit for bit, odd and even sides."""
+    from oracle import c_oracle, spgg_numpy
+    n = 25
+    p = full_params(dict(L=L, r=3.6, cost=1, alpha=0.8, epsilon_decay=0.9, influence_factor=0.7,
+                         use_second_order=second, state_representation=state,
+                         reward_weight_payoff=0.95, rep_gain_C=1.0, algorithm=algo, iterations=n))
+    pairs = c_oracle.PAIRS[c_oracle.ALGOS[algo]]
+    rs = np.random.RandomState(L + 7 * pairs + second)
+    Q0 = rs.uniform(-0.01, 0.01, (L, L, 2, 2, 2) if algo == "double_qlearning" else (L, L, 2, 2))
+    S0 = rs.randint(0, 2, (L, L))
+    u = rs.rand(n, pairs, L, L)
+    b = rs.randint(0, 2, (n, pairs, L, L)).astype(np.uint8)
+    if algo == "sarsa":
+        draws = lambda t, L_: tuple(x for k in range(3) for x in (u[t - 1, k], b[t - 1, k]))  # noqa: E731
+    elif algo == "double_qlearning":
+        draws = lambda t, L_: (u[t - 1, 0], b[t - 1, 0], u[t - 1, 1])  # noqa: E731
+    else:
+        draws = lambda t, L_: (u[t - 1, 0], b[t - 1, 0])  # noqa: E731
+    q0_np = (Q0[:, :, 0], Q0[:, :, 1]) if algo == "double_qlearning" else Q0
+    ref = spgg_numpy.simulate(p, S0.astype(np.int64), np.zeros((L, L)), q0_np, draws)
+    sim = c_oracle.Sim(p, S0, np.zeros((L, L)), Q0, "fp64")
+    rows = sim.run(n, lambda t, L_: (u[t - 1], b[t - 1]))
+    assert rows.shape[0] == n == len(ref["switch_C_to_D"])
+    assert np.array_equal(sim.S, ref["Sn_final"])
+    assert np.array_equal(sim.R, ref["R_final"])
+    if algo == "double_qlearning":
+        assert np.array_equal(sim.Q[:, :, 0], ref["q1_final"])
+        assert np.array_equal(sim.Q[:, :, 1], ref["q2_final"])
+    assert np.array_equal(sim.q_combined, ref["q_final"])
+    ST = c_oracle.ST
+    assert np.array_equal(rows[:, ST["N_CD"]].astype(np.int64), ref["switch_C_to_D"])
+    assert np.array_equal(rows[:, ST["N_DC"]].astype(np.int64), ref["switch_D_to_C"])
+    assert np.array_equal(rows[:, ST["NC_OLD"]] / (L * L), ref["coop_rate_history"][:n])
+    assert np.array_equal(rows[:, ST["GMAX"]], ref["gmax"])
+    for k in range(6):
+        assert np.array_equal(rows[:, ST["GROUP0"] + k] / (L * L) * 100, ref[f"group_comp_d{k}_history"])
+    # the float statistics are plain sums here and NumPy means there
+    np.testing.assert_allclose(rows[:, ST["SUM_NI"]] / (L * L), ref["neighbor_influence_percent"],
+                               rtol=1e-9, atol=1e-12)
+    np.testing.assert_allclose(rows[:, ST["SUM_Q"]] / (L * L), ref["avg_q_s0_c_history"], rtol=1e-9,
+                               atol=1e-15)
+    assert len(np.unique(sim.S)) == 2                  # the run did not end uniform
+
+
+def test_philox_streams_of_the_td_rules():
+    """The Philox words the step functions draw for a site are those of the documented counters
+    (j/4, i, t, stream), word j%4 - the counters k_step's philox_row forms - and the fp32 step
+    acts on them: with epsilon = 1 every action is word0 & 1, and Double Q updates table 1 exactly
+    where (word1 >> 8) < 2^23."""
+    from oracle import c_oracle
+    seed = 0x123456789ABCDEF0
+    key = [seed & 0xFFFFFFFF, seed >> 32]
+    for (t, i, j) in ((1, 0, 0), (7, 5, 13), (3, 36, 31), (2, 4095, 4094)):
+        for stream in (0, 1, 2):
+            want = int(c_oracle.philox([j // 4, i, t, stream], key)[j % 4])
+            assert c_oracle.site_word(seed, t, stream, i, j) == want, (t, i, j, stream)
+    L = 37
+    p = full_params(dict(L=L, r=3.0, cost=1, epsilon=1.0, epsilon_decay=1.0, influence_factor=0.0,
+                         state_representation="action", algorithm="double_qlearning"))
+    rs = np.random.RandomState(4)
+    Q0 = rs.uniform(-0.01, 0.01, (L, L, 2, 2, 2)).astype(np.float32)
+    S0 = rs.randint(0, 2, (L, L))
+    sim = c_oracle.Sim(p, S0, np.zeros((L, L)), Q0, "fp32", seed=seed)
+    sim.step()
+    w0 = np.array([[c_oracle.site_word(seed, 1, 0, i, j) for j in range(L)] for i in range(L)], np.uint64)
+    w1 = np.array([[c_oracle.site_word(seed, 1, 1, i, j) for j in range(L)] for i in range(L)], np.uint64)
+    assert np.array_equal(sim.S, (w0 & 1).astype(np.uint8))
+    upd1 = (w1 >> 8) < (1 << 23)
+    changed1 = (sim.Q[:, :, 0] != Q0[:, :, 0]).any(axis=(2, 3))
+    changed2 = (sim.Q[:, :, 1] != Q0[:, :, 1]).any(axis=(2, 3))
+    assert np.array_equal(changed1, upd1) and np.array_equal(changed2, ~upd1)
+
+
 def test_early_exit_series_lengths():
     """Uniform lattice: the loop records the pre-action entries and breaks (spgg.py:405):
     T_c = T + 1."""
@@ -212,9 +325,6 @@ def test_early_exit_series_lengths():
     out = spgg_numpy.simulate(p, np.zeros((L, L), np.int64), np.zeros((L, L)),
                               np.zeros((L, L, 2, 2)), lambda t, L_: (None, None))
     assert len(out["coop_rate_history"]) == 1 and "epsilon_history_final" not in out
-
-
-TD_GOLDEN = ["sarsa_rep_m1", "sarsa_act_m2", "expsarsa_rep_m2", "expsarsa_act_m1"]
 
 
 def _td_draws(z):
