@@ -155,6 +155,25 @@ int spgg_state_digest(spgg_t *h, int replica, uint64_t out[3]);
  * the bin index is corrected against the edges as NumPy does.  n_bins <= 64. */
 int spgg_r_histogram(spgg_t *h, int replica, int n_bins, const double *edges, int64_t *counts);
 
+/* scipy.ndimage.label(S == which) of one replica on the device (cluster_sizes,
+ * spgg.py:631-633): which = 0 selects the cooperators, 1 the defectors; 4-connected,
+ * non-periodic unless flags has SPGG_CLUSTER_PERIODIC, which also joins row L-1 to row 0
+ * and column L-1 to column 0 (the torus the dynamics live on).  Labels run 1..n in
+ * increasing order of each cluster's smallest linear index row*L + col, which is scipy's
+ * numbering; the result does not depend on scheduling.  Sees the state spgg_get_state
+ * would return.  Whole-lattice handles only (rows == L, rows*L < 2^31; else
+ * SPGG_E_UNSUPPORTED).  The result stays on the handle for the two getters below until
+ * the next spgg_clusters call or until the state changes (spgg_step / spgg_begin_steps,
+ * spgg_set_state, spgg_init_random, spgg_set_progress, spgg_strip_rewind); the getters
+ * return SPGG_E_STATE without one.  The first call allocates device scratch that the
+ * handle keeps until spgg_destroy: 8 bytes a site (union-find parents and set sizes),
+ * 2 bits a site (root mask, rank offsets) and room for ceil(L*L/2) int64 sizes, about
+ * 12.25 bytes a site in all (206 MB at L=4096, 13.2 GB at L=32768). */
+#define SPGG_CLUSTER_PERIODIC 1
+int spgg_clusters(spgg_t *h, int replica, int which, int flags, int64_t *n_clusters);
+int spgg_cluster_sizes(spgg_t *h, int64_t *sizes, int64_t n);   /* n must equal n_clusters: sizes[k-1] = #sites of label k */
+int spgg_cluster_labels(spgg_t *h, int32_t *labels);            /* rows*L values, row-major, 0 where not selected */
+
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox
  * keyed by `seed`; for lattices too large to stage through host memory. */

@@ -28,6 +28,7 @@ STATE_REPUTATION, STATE_ACTION = 0, 1
 ALGO_QLEARNING, ALGO_SARSA, ALGO_EXPECTED_SARSA, ALGO_DOUBLE_QLEARNING = 0, 1, 2, 3
 RSTORE_AUTO, RSTORE_INT8, RSTORE_FP32 = 0, 1, 2
 E_INVALID, E_CUDA, E_STATE, E_UNSUPPORTED = -1, -2, -3, -4
+CLUSTER_PERIODIC = 1
 
 
 class Params(C.Structure):
@@ -62,6 +63,7 @@ EXPORTS = (
     "spgg_state_digest", "spgg_phase_iteration", "spgg_strip_can_speculate", "spgg_strip_iteration",
     "spgg_strip_report_ptr", "spgg_strip_verify", "spgg_strip_failed", "spgg_strip_rewind",
     "spgg_r_histogram", "spgg_ipc_export", "spgg_ipc_attach", "spgg_ring_export", "spgg_ring_attach",
+    "spgg_clusters", "spgg_cluster_sizes", "spgg_cluster_labels",
 )
 
 _lib = None
@@ -104,6 +106,9 @@ def load():
     lib.spgg_strip_failed.argtypes = [vp]
     lib.spgg_strip_rewind.argtypes = [vp, i32]
     lib.spgg_r_histogram.argtypes = [vp, i32, i32, vp, vp]
+    lib.spgg_clusters.argtypes = [vp, i32, i32, i32, C.POINTER(i64)]
+    lib.spgg_cluster_sizes.argtypes = [vp, vp, i64]
+    lib.spgg_cluster_labels.argtypes = [vp, vp]
     lib.spgg_ipc_export.argtypes = [vp, vp]
     lib.spgg_ipc_attach.argtypes = [vp, i32, vp, i32, i32]
     lib.spgg_ring_export.argtypes = [vp, vp]

@@ -134,6 +134,10 @@ struct spgg_handle {
   long long pend_t0 = 0;
   int pend_n = 0, pend_cur0 = 0, pend_rel = 0;
   cudaStream_t pend_stream = nullptr;
+  // spgg_clusters: device scratch (spgg_clusters.cuh) and whether it holds the result of the current state
+  CclScratch ccl;
+  bool ccl_valid = false;
+  int64_t ccl_n = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -334,6 +338,7 @@ static int free_all(spgg_handle *h) {
   cudaFree(h->d_stop); cudaFree(h->d_eps); cudaFree(h->d_thr); cudaFree(h->d_u); cudaFree(h->d_b);
   cudaFree(h->d_sc_S); cudaFree(h->d_sc_R); cudaFree(h->d_sc_Q); cudaFree(h->d_sc_info);
   cudaFree(h->d_gimg); cudaFree(h->d_gpart); cudaFree(h->d_gnsel);
+  ccl_free(&h->ccl);
   return 0;
 }
 
@@ -762,6 +767,7 @@ extern "C" int spgg_set_state(spgg_t *h, int rep, const uint8_t *S, const double
   if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
   int rcode = finish_pending(h);
   if (rcode) return rcode;
+  h->ccl_valid = false;
   CUDA_TRY(cudaSetDevice(h->device));
   rcode = ensure_scratch(h, true);
   if (rcode) return rcode;
@@ -888,6 +894,7 @@ extern "C" int spgg_begin_steps(spgg_t *h, int n_steps, void *stream_) {
   if (n_steps < 1) return fail(SPGG_E_INVALID, "n_steps must be >= 1");
   int rcode = finish_pending(h);
   if (rcode) return rcode;
+  h->ccl_valid = false;
   for (int r = 0; r < h->n_rep; ++r)
     if (h->stale[r])
       return fail(SPGG_E_STATE, "replica %d still holds the state of the previous run: give every replica of a "
@@ -1254,6 +1261,7 @@ extern "C" int spgg_init_random(spgg_t *h, int rep, uint64_t seed) {
   if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
   int rcode = finish_pending(h);
   if (rcode) return rcode;
+  h->ccl_valid = false;
   CUDA_TRY(cudaSetDevice(h->device));
   const uint32_t lo = (uint32_t)seed, hi = (uint32_t)(seed >> 32);
   const int grid = 148 * 8;
@@ -1283,6 +1291,7 @@ extern "C" int spgg_set_progress(spgg_t *h, int64_t iteration, const double *eps
     if (!(epsilon[r] >= 0.0 && epsilon[r] <= 1.0)) return fail(SPGG_E_INVALID, "epsilon[%d] = %g outside [0, 1]", r, epsilon[r]);
   }
   if (h->iter != 0) return fail(SPGG_E_STATE, "spgg_set_progress follows the state uploads of a resumed run");
+  h->ccl_valid = false;
   CUDA_TRY(cudaSetDevice(h->device));
   h->iter = (long long)iteration;
   h->replay_first = h->iter;
@@ -1345,6 +1354,57 @@ extern "C" int spgg_r_histogram(spgg_t *h, int rep, int n_bins, const double *ed
   cudaFree(d_edges); cudaFree(d_cnt);
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_r_histogram: %s", cudaGetErrorString(e));
   for (int i = 0; i < n_bins; ++i) counts[i] = (int64_t)host_cnt[i];
+  h->launches += 1;
+  return SPGG_OK;
+}
+
+// ---------------------------------------------------------------- clusters
+// scipy.ndimage.label of one replica's strategies (include/spgg.h); the kernels live in spgg_clusters.cu
+extern "C" int spgg_clusters(spgg_t *h, int rep, int which, int flags, int64_t *n_clusters) {
+  if (!h || !n_clusters) return fail(SPGG_E_INVALID, "spgg_clusters: null argument");
+  if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
+  if (which != 0 && which != 1) return fail(SPGG_E_INVALID, "which must be 0 (cooperators) or 1 (defectors), got %d", which);
+  if (flags & ~SPGG_CLUSTER_PERIODIC) return fail(SPGG_E_INVALID, "unknown cluster flags 0x%x", flags);
+  if (!h->g.wrap_rows) return fail(SPGG_E_UNSUPPORTED, "cluster labelling needs the whole lattice (rows == L), not a strip");
+  if ((long long)h->g.rows * h->g.L >= (1ll << 31)) return fail(SPGG_E_UNSUPPORTED, "cluster labelling needs rows*L < 2^31");
+  int rcode = finish_pending(h);
+  if (rcode) return rcode;
+  h->ccl_valid = false;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaError_t e = ccl_alloc(&h->ccl, h->g.L);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(SPGG_E_CUDA, "spgg_clusters: scratch for L=%d: %s", h->g.L, cudaGetErrorString(e));
+  }
+  const Geom &g = h->g;
+  const uint32_t *S = h->d_S[h->cur] + (size_t)rep * g.bits_stride + (size_t)GH * g.pitchW + WPAD;
+  int64_t n = 0;
+  e = launch_clusters(h->ccl, S, g.pitchW, which, flags & SPGG_CLUSTER_PERIODIC, &n);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_clusters: %s", cudaGetErrorString(e));
+  h->launches += 5;
+  h->ccl_n = n;
+  h->ccl_valid = true;
+  *n_clusters = n;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_cluster_sizes(spgg_t *h, int64_t *sizes, int64_t n) {
+  if (!h || !sizes) return fail(SPGG_E_INVALID, "spgg_cluster_sizes: null argument");
+  if (!h->ccl_valid) return fail(SPGG_E_STATE, "spgg_cluster_sizes: no spgg_clusters result for the current state");
+  if (n != h->ccl_n) return fail(SPGG_E_INVALID, "spgg_cluster_sizes: n = %lld, the labelling found %lld clusters", (long long)n, (long long)h->ccl_n);
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (n > 0) CUDA_TRY(cudaMemcpy(sizes, h->ccl.sizes, sizeof(int64_t) * (size_t)n, cudaMemcpyDeviceToHost));
+  return SPGG_OK;
+}
+
+extern "C" int spgg_cluster_labels(spgg_t *h, int32_t *labels) {
+  if (!h || !labels) return fail(SPGG_E_INVALID, "spgg_cluster_labels: null argument");
+  if (!h->ccl_valid) return fail(SPGG_E_STATE, "spgg_cluster_labels: no spgg_clusters result for the current state");
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaError_t e = launch_cluster_labels(h->ccl);
+  if (e == cudaSuccess)
+    e = cudaMemcpy(labels, h->ccl.total, sizeof(int32_t) * (size_t)h->g.rows * h->g.L, cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_cluster_labels: %s", cudaGetErrorString(e));
   h->launches += 1;
   return SPGG_OK;
 }
@@ -1485,6 +1545,7 @@ extern "C" int spgg_strip_rewind(spgg_t *h, int bad) {
   if (!h || !h->pending || !h->d_bad) return fail(SPGG_E_STATE, "spgg_strip_rewind outside a chunk");
   if (bad < 1 || bad > h->pend_n) return fail(SPGG_E_INVALID, "launch %d outside the chunk of %d", bad, h->pend_n);
   h->in_rerun = true;   // (the test hook does not spoil re-runs; cleared by the next spgg_begin_steps)
+  h->ccl_valid = false;
   if (h->d_ring) {      // ring mode: every rank empties its own ring and starts counting launches again; the
     CUDA_TRY(cudaMemset(h->d_ring, 0, sizeof(unsigned) * RING_SLOTS * RING_WORDS));  // caller puts a barrier
     h->gen = 0;                                                                        // between this and the re-run

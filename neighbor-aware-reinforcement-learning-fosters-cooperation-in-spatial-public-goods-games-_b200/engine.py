@@ -163,6 +163,34 @@ class Engine:
         L_.check(self.lib.spgg_r_histogram(self._h, replica, int(bins), edges.ctypes.data, counts.ctypes.data))
         return counts, edges
 
+    # -- clusters (include/spgg.h: spgg_clusters)
+    def _clusters(self, replica, of, periodic) -> int:
+        which = {"C": 0, "D": 1, 0: 0, 1: 1}.get(of if isinstance(of, (str, int)) and not isinstance(of, bool) else None)
+        if which is None:
+            raise ValueError(f"of must be 'C' or 'D' (or 0 / 1), got {of!r}")
+        n = C.c_int64()
+        L_.check(self.lib.spgg_clusters(self._h, int(replica), which, L_.CLUSTER_PERIODIC if periodic else 0,
+                                        C.byref(n)))
+        return int(n.value)
+
+    def cluster_sizes(self, replica: int = 0, of="C", periodic: bool = False) -> np.ndarray:
+        """Sizes (int64) of the 4-connected clusters of cooperators (``of="C"``) or defectors (``"D"``),
+        computed on the device: ``np.bincount(label(S == of)[0].ravel())[1:]`` with scipy's labelling
+        (spgg.py:631-633), in the order of each cluster's first site in raster order.  ``periodic=True``
+        also joins clusters across the edges of the torus."""
+        n = self._clusters(replica, of, periodic)
+        sizes = np.empty(n, np.int64)
+        L_.check(self.lib.spgg_cluster_sizes(self._h, sizes.ctypes.data, n))
+        return sizes
+
+    def cluster_labels(self, replica: int = 0, of="C", periodic: bool = False):
+        """``scipy.ndimage.label(S == of)`` computed on the device: (labels int32 (rows, L), n); labels
+        1..n numbered by each cluster's first site in raster order, 0 where the site is not selected."""
+        n = self._clusters(replica, of, periodic)
+        labels = np.empty((self.rows, self.L), np.int32)
+        L_.check(self.lib.spgg_cluster_labels(self._h, labels.ctypes.data))
+        return labels, n
+
     def set_replay(self, u, b):
         """``u`` (n,rows,L) float64 and ``b`` (n,rows,L) 0/1: the reference's draw
         arrays for the next n iterations (algorithms.py:105,108)."""

@@ -159,8 +159,9 @@ class SPGG:
         else:
             deferred.append(write)
 
-    def _write_final(self, data_file, ser, S, R, rep_hist_final, rep_bins_final):
-        """Dataset names, order and dtypes of spgg.py:595-633."""
+    def _write_final(self, data_file, ser, S, R, rep_hist_final, rep_bins_final, cluster_sizes):
+        """Dataset names, order and dtypes of spgg.py:595-633.  ``cluster_sizes``: the sizes of the
+        4-connected, non-periodic clusters of cooperators (spgg.py:631-633), labelled on the device."""
         for key in ("it_records_final", "epsilon_history_final", "rep_avg_history_final",
                     "coop_rate_history", "switch_C_to_D", "switch_D_to_C",
                     "neighbor_influence_percent", "payoff_component_history",
@@ -181,11 +182,7 @@ class SPGG:
         data_file.create_dataset("R_final", data=R)
         data_file.create_dataset("rep_hist_final", data=rep_hist_final)
         data_file.create_dataset("rep_bins_final", data=rep_bins_final)
-        # 4-connected, non-periodic clusters of cooperators (spgg.py:631-633), linear time
-        from scipy.ndimage import label
-        clusters, n_clusters = label(S == 0)
-        sizes = np.bincount(clusters.ravel(), minlength=n_clusters + 1)[1:]
-        data_file.create_dataset("cluster_sizes", data=sizes.astype(np.int64))
+        data_file.create_dataset("cluster_sizes", data=np.asarray(cluster_sizes, dtype=np.int64))
 
 
 class _HostWorker:
@@ -313,6 +310,8 @@ def run_models(models, filenames):
         for r, m in enumerate(models):
             S, R, _ = eng.get_state(r, want_q=False)
             hist_f, bins_f = eng.r_histogram(20, m.R_min, m.R_max, r)
+            # scipy.ndimage.label(S == 0) on the device; here, not on the writer thread: one thread per handle
+            sizes_f = eng.cluster_sizes(r)
             ri = np.vstack(rows_it[r]) if rows_it[r] else np.zeros((0, L_.NSTAT))
             sb = np.concatenate(sum_r_before[r]) if sum_r_before[r] else np.zeros(0)
             # the schedule the engine ran is the algorithm object's (it may be an instance the caller built)
@@ -322,8 +321,8 @@ def run_models(models, filenames):
                                   stop_all_coop=bool((S == 0).all()))
             # the final datasets go to the file on the host thread while the Q table (the largest array)
             # comes back from the device
-            worker.run([lambda m=m, r=r, ser=ser, S=S, R=R, hist_f=hist_f, bins_f=bins_f:
-                        m._write_final(files[r], ser, S, R, hist_f, bins_f)])
+            worker.run([lambda m=m, r=r, ser=ser, S=S, R=R, hist_f=hist_f, bins_f=bins_f, sizes_f=sizes_f:
+                        m._write_final(files[r], ser, S, R, hist_f, bins_f, sizes_f)])
             Q = eng.get_q(r)
             if eng.nq == 8:
                 m.algorithm.q_table_1 = np.ascontiguousarray(Q[:, :, 0])
