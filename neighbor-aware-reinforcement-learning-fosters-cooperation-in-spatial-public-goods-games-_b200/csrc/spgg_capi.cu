@@ -108,6 +108,9 @@ struct spgg_handle {
   unsigned long long *d_sc_info = nullptr;
   // fast path (spgg_fast.cuh): TMA descriptors of the two plane sets
   bool fast = false;
+  // an uploaded R lies outside [-16, 15] int8 units, which k_step_fast's biased bytes cannot hold: the
+  // next select runs on k_step, whose reputation update clips every R into [R_min, R_max] ⊆ [-15, 15]
+  bool r_wide = false;
   FastMaps fmaps[2];  // [cur]: loads from plane set cur, stores into cur^1
   // lattice-resident path (spgg_resident.cuh): one cluster per replica, whole chunks per launch
   bool resident = false;
@@ -740,7 +743,7 @@ static int ensure_scratch(spgg_handle *h, bool want_q) {
   if (!h->d_sc_S) {
     CUDA_TRY(cudaMalloc((void **)&h->d_sc_S, n));
     CUDA_TRY(cudaMalloc((void **)&h->d_sc_R, n * sizeof(double)));
-    CUDA_TRY(cudaMalloc((void **)&h->d_sc_info, 2 * sizeof(unsigned long long)));
+    CUDA_TRY(cudaMalloc((void **)&h->d_sc_info, 3 * sizeof(unsigned long long)));
   }
   if (want_q && !h->d_sc_Q) CUDA_TRY(cudaMalloc((void **)&h->d_sc_Q, n * h->nq() * sizeof(double)));
   return SPGG_OK;
@@ -773,7 +776,7 @@ extern "C" int spgg_set_state(spgg_t *h, int rep, const uint8_t *S, const double
   if (rcode) return rcode;
   const Geom &g = h->g;
   const RepConst &rc = h->rc_host[rep];
-  CUDA_TRY(cudaMemset(h->d_sc_info, 0, 2 * sizeof(unsigned long long)));
+  CUDA_TRY(cudaMemset(h->d_sc_info, 0, 3 * sizeof(unsigned long long)));
   const int chunk = stage_rows(h);
   for (int i0 = 0; i0 < g.rows; i0 += chunk) {
     const int nr = std::min(chunk, g.rows - i0);
@@ -791,11 +794,19 @@ extern "C" int spgg_set_state(spgg_t *h, int rep, const uint8_t *S, const double
     CUDA_TRY(cudaGetLastError());
     h->launches += 1;
   }
-  unsigned long long info[2];
+  unsigned long long info[3];
   CUDA_TRY(cudaMemcpy(info, h->d_sc_info, sizeof(info), cudaMemcpyDeviceToHost));
   if (info[0] == 1) return fail(SPGG_E_INVALID, "strategy array holds values other than 0/1");
   if (info[0] == 2)
     return fail(SPGG_E_INVALID, "R is not representable in int8 units of %g; use r_storage=FP32", rc.rq);
+  if (info[2] && h->fast) {
+    // a strip's boundary rows reach its neighbours from k_step_fast itself (peer-mapped stores, the
+    // report ring), so a strip cannot take the k_step detour of the whole lattice
+    if (!g.wrap_rows)
+      return fail(SPGG_E_INVALID, "R outside [%g, %g] (int8 units -16..15 of %g): a strip on the fast path "
+                  "cannot hold it", -16.0 * rc.rq, 15.0 * rc.rq, rc.rq);
+    h->r_wide = true;
+  }
   begin_new_run(h, rep);
   h->eps_cur[rep] = h->params[rep].epsilon;
   int stop = -1;
@@ -974,7 +985,7 @@ static int launch_step(spgg_handle *h, int do_update, int do_select, cudaStream_
   a.b3 = (upd_replay && np_ == 3) ? h->d_b + ((size_t)ue * 3 + 2) * ss : nullptr;
   a.j = (int)j; a.rel = h->pend_rel; a.cap = h->cap;
   a.do_update = do_update; a.do_select = do_select;
-  const bool use_fast = h->fast && !replay;
+  const bool use_fast = h->fast && !replay && !(do_select && h->r_wide);
   a.spec = 0; a.gcarry = nullptr; a.bad_at = nullptr; a.gvec = nullptr;
   for (int d = 0; d < 2; ++d) {   // ghost rows of the neighbours' OUTPUT planes (parity cur^1), fast path only
     const bool on = h->peer_on && use_fast && do_select;
@@ -1048,7 +1059,10 @@ static int launch_step(spgg_handle *h, int do_update, int do_select, cudaStream_
   h->launches += 1;
   h->last_rel = h->pend_rel; h->last_upd = do_update; h->last_spec = a.spec; h->last_sel = do_select;
   h->last_gen = a.ring_world > 0 ? h->gen++ : -1;
-  if (do_select) h->cur ^= 1;
+  if (do_select) {
+    h->cur ^= 1;
+    h->r_wide = false;   // every R was just clipped into [R_min, R_max]
+  }
   if (h->pend_rel >= 0 && h->pend_rel < (int)h->pend_cur_after.size()) {
     h->pend_cur_after[h->pend_rel] = (char)h->cur;
     h->pend_q_after[h->pend_rel] = (char)h->qcur;

@@ -390,8 +390,8 @@ __device__ __forceinline__ void step_fast_body(const FastMaps &tm, const KArgs &
       if constexpr (ACTION) {
         StW = CW;                                          // own previous action (spgg.py:291)
       } else {
-        // reputation state (spgg.py:292-307): v = R + 16 in each byte (|R| <= 15 is a launch
-        // precondition); sum of n values v > 16 n  <=>  sum of R > 0
+        // reputation state (spgg.py:292-307): v = R + 16 in each byte (R in [-16, 15] units: spgg_set_state sends a wider R to k_step's
+        // select, which clips it into [R_min, R_max], or rejects it on a strip); sum of n values v > 16 n  <=>  sum of R > 0
         const uint32_t *rp = st_R + wo + M * FROWW;
         auto bias = [](uint32_t x) { return (x ^ 0x10101010u) & 0x1F1F1F1Fu; };
         const uint32_t c = bias(RW), l = bias(rp[-1]), r = bias(rp[1]);

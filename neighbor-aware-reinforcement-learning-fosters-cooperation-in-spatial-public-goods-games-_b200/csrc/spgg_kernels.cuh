@@ -1264,7 +1264,8 @@ __global__ void k_init_random(Geom g, int rep, void *Q, void *R, uint32_t *S, ui
 
 // host layout (reference arrays: _Sn bytes 0/1, R float64, q_table float64 (rows,L,2,2))
 // <-> device planes, `nrows` rows starting at local row i0.  One warp per 32-site word.
-// info[0] = error flag (1: S not 0/1, 2: R not representable in int8 units), info[1] = #cooperators
+// info[0] = error flag (1: S not 0/1, 2: R not representable in int8 units), info[1] = #cooperators,
+// info[2] = 1 if an int8 R lies outside [-16, 15] units (beyond k_step_fast's biased bytes)
 template <class Md>
 __global__ void k_import_rows(Geom g, int rep, int i0, int nrows, const uint8_t *S, const double *R,
                               const double *Q, void *Qd, void *Rd, uint32_t *Sd, double rq,
@@ -1280,6 +1281,7 @@ __global__ void k_import_rows(Geom g, int rep, int i0, int nrows, const uint8_t 
   const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
   unsigned long long coop = 0;
+  bool wide = false;
   for (long long it = warp0; it < n_items; it += n_warps) {
     const int ii = (int)(it / words), w = (int)(it % words);
     const int i = i0 + ii, col = w * 32 + lane;
@@ -1295,6 +1297,7 @@ __global__ void k_import_rows(Geom g, int rep, int i0, int nrows, const uint8_t 
       if constexpr (sizeof(RT) == 1) {
         const double q = r / rq;
         if (q != floor(q) || q < -128.0 || q > 127.0) atomicExch(info, 2ull);
+        wide = wide || q < -16.0 || q > 15.0;
         rv = (RT)(int)q;
       } else {
         rv = (RT)r;
@@ -1309,6 +1312,7 @@ __global__ void k_import_rows(Geom g, int rep, int i0, int nrows, const uint8_t 
     if (lane == 0) store_bits_word(Sp, g, i, w, word);
   }
   if (lane == 0 && coop) atomicAdd(info + 1, coop);
+  if (wide) atomicExch(info + 2, 1ull);
 }
 
 template <class Md>
