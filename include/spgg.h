@@ -143,10 +143,12 @@ int spgg_get_state(spgg_t *h, int replica, uint8_t *S, double *R, double *Q);
 int spgg_set_progress(spgg_t *h, int64_t iteration, const double *epsilon);
 
 /* Position-keyed 64-bit digests of one replica's owned rows: out[0] strategies,
- * out[1] reputations, out[2] Q.  A site contributes hash(global row, column) *
+ * out[1] reputations, out[2] Q.  A site contributes (hash(global row, column) | 1) *
  * (bits of its value as a double + 1) mod 2^64, so the digests of the strips of a
  * lattice add up (mod 2^64) to the digest of the whole lattice: multi-GPU runs are
- * compared with single-GPU runs without moving a 20 GB state through the host. */
+ * compared with single-GPU runs without moving a 20 GB state through the host.  The
+ * multiplier is odd, so a change of any one value (a sign flip, +0.0 -> -0.0) changes
+ * its word.  oracle/spgg_oracle.c: oracle_state_digest computes the same on the host. */
 int spgg_state_digest(spgg_t *h, int replica, uint64_t out[3]);
 
 /* np.histogram(R, bins=n_bins, range=(edges[0], edges[n_bins])) of a replica's

@@ -1341,9 +1341,11 @@ __global__ void k_export_rows(Geom g, int rep, int i0, int nrows, uint8_t *S, do
 }
 
 // Position-keyed digests of one replica's owned rows: out[0] strategies, out[1] reputations,
-// out[2] Q.  Every site contributes hash(global row, column[, entry]) * (value bits + 1) modulo
-// 2^64, so the digests of the strips of a lattice ADD UP to the digest of the whole lattice:
+// out[2] Q.  Every site contributes (hash(global row, column[, entry]) | 1) * (value bits + 1)
+// modulo 2^64, so the digests of the strips of a lattice ADD UP to the digest of the whole lattice:
 // an N-strip run is compared with a single-handle run without moving either state to the host.
+// The multiplier is odd, hence invertible mod 2^64: any change of one value changes its term.  (An
+// even one would miss a sign flip, which moves the bits by 2^63.)  oracle_state_digest restates this.
 __device__ __forceinline__ unsigned long long digest_mix(unsigned long long x) {
   x ^= x >> 33; x *= 0xff51afd7ed558ccdull; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ull; x ^= x >> 33;
   return x;
@@ -1362,7 +1364,7 @@ __global__ void k_state_digest(Geom g, int rep, const void *Qd, const void *Rd, 
        e += (long long)gridDim.x * blockDim.x) {
     const int i = (int)(e / g.L), col = (int)(e % g.L);
     const unsigned long long key = ((unsigned long long)(unsigned)(g.row0 + i) << 32) | (unsigned)col;
-    const unsigned long long hS = digest_mix(key * 3 + 1), hR = digest_mix(key * 3 + 2);
+    const unsigned long long hS = digest_mix(key * 3 + 1) | 1ull, hR = digest_mix(key * 3 + 2) | 1ull;
     const unsigned bit = (Sp[(long long)(i + GH) * g.pitchW + WPAD + (col >> 5)] >> (col & 31)) & 1u;
     dS += hS * (unsigned long long)(bit + 1u);
     double rv = (double)Rp[(long long)(i + GH) * g.pitchB + CPAD + col];
@@ -1370,7 +1372,8 @@ __global__ void k_state_digest(Geom g, int rep, const void *Qd, const void *Rd, 
     dR += hR * ((unsigned long long)__double_as_longlong(rv) + 1ull);
     for (int z = 0; z < nq; ++z) {
       const double qv = (double)Qp[e * nq + z];
-      dQ += digest_mix(key * 3 + 3 + ((unsigned long long)(z + 1) << 58)) * ((unsigned long long)__double_as_longlong(qv) + 1ull);
+      dQ += (digest_mix(key * 3 + 3 + ((unsigned long long)(z + 1) << 58)) | 1ull) *
+            ((unsigned long long)__double_as_longlong(qv) + 1ull);
     }
   }
   for (int o = 16; o > 0; o >>= 1) {

@@ -64,6 +64,14 @@ def lib():
         _lib.oracle_thr24.argtypes = [C.c_double]
         _lib.oracle_reward_table.argtypes = [C.POINTER(OracleParams), C.c_void_p]
         _lib.oracle_num_threads.restype = C.c_int
+        i32, vp = C.c_int, C.c_void_p
+        _lib.oracle_state_digest.argtypes = [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp]
+        _lib.oracle_digest_weights.argtypes = [i32, i32, i32, i32, i32, vp]
+        _lib.oracle_init_random.argtypes = [i32, i32, i32, i32, i32, C.c_uint64, vp, vp, vp]
+        _lib.oracle_init_random.restype = None
+        _lib.oracle_init_random_digest.argtypes = [i32, i32, i32, i32, i32, C.c_uint64, vp]
+        _lib.oracle_explore_actions.argtypes = [i32, i32, i32, C.c_uint64, C.c_uint32, vp]
+        _lib.oracle_explore_actions.restype = None
     return _lib
 
 
@@ -104,6 +112,82 @@ def reward_table(p: dict) -> np.ndarray:
     op = params_from_dict(p)
     lib().oracle_reward_table(C.byref(op), tab.ctypes.data)
     return tab
+
+
+def _digest_shape(L, rows, period):
+    return (period, period) if period else (rows, L)
+
+
+def digest_weights(L: int, nq: int, period: int | None = None, row0: int = 0, rows: int | None = None):
+    """The multipliers ``state_digest`` applies, one set per value slot: (P, P, 2 + nq) uint64 for a
+    lattice of period P, else (rows, L, 2 + nq).  Computing them is the costly part of a digest;
+    pass them back to ``state_digest`` to digest many states of the same geometry."""
+    rows = L if rows is None else int(rows)
+    w = np.empty(_digest_shape(L, rows, period) + (2 + nq,), np.uint64)
+    if lib().oracle_digest_weights(int(L), int(row0), rows, int(period or 0), int(nq), w.ctypes.data):
+        raise ValueError(f"period {period} does not divide L = {L}")
+    return w
+
+
+def state_digest(S, R, Q=None, L: int | None = None, row0: int = 0, period: int | None = None,
+                 weights=None):
+    """``Engine.digest`` of a host state (include/spgg.h: spgg_state_digest): S (rows, L) 0/1, R (rows, L)
+    and Q (rows, L, 2, 2[, 2]) as ``Engine.get_state`` returns them, the rows starting at global row
+    ``row0``.  With ``period`` = P the arrays hold a P x P state and the digest is that of the L x L
+    lattice tiled with it.  Q = None digests S and R only (the Q word is 0)."""
+    S = np.ascontiguousarray(S, np.uint8)
+    R = np.ascontiguousarray(R, np.float64)
+    rows, width = S.shape
+    L = width if L is None else int(L)
+    if R.shape != S.shape or _digest_shape(L, rows, period) != S.shape:
+        raise ValueError(f"S {S.shape} and R {R.shape} do not describe the geometry (L={L}, period={period})")
+    nq = 4
+    if Q is not None:
+        Q = np.ascontiguousarray(Q, np.float64)
+        nq = Q.size // S.size
+        if nq not in (4, 8) or Q.size != nq * S.size:
+            raise ValueError(f"Q must hold 4 or 8 values per site, got shape {Q.shape}")
+    if weights is not None and weights.shape != S.shape + (2 + nq,):
+        raise ValueError(f"weights {weights.shape} do not match the state")
+    out = np.zeros(3, np.uint64)
+    rc = lib().oracle_state_digest(int(L), int(row0), rows, int(period or 0), nq,
+                                   S.ctypes.data, R.ctypes.data, None if Q is None else Q.ctypes.data,
+                                   None if weights is None else np.ascontiguousarray(weights).ctypes.data,
+                                   out.ctypes.data)
+    if rc:
+        raise ValueError(f"period {period} does not divide L = {L}")
+    return tuple(int(x) for x in out)
+
+
+def init_random(L: int, seed: int, nq: int = 4, precision: str = "fp32", row0: int = 0, rows: int | None = None):
+    """``Engine.init_random(seed)`` restated on the host: (S, R, Q) of rows [row0, row0 + rows) in the
+    layout of ``Engine.get_state``."""
+    rows = L if rows is None else int(rows)
+    S = np.empty((rows, L), np.uint8)
+    R = np.empty((rows, L), np.float64)
+    Q = np.empty((rows, L, 2, 2) if nq == 4 else (rows, L, 2, 2, 2), np.float64)
+    lib().oracle_init_random(int(L), int(row0), rows, int(nq), int(precision == "fp32"), int(seed) & (2 ** 64 - 1),
+                             S.ctypes.data, R.ctypes.data, Q.ctypes.data)
+    return S, R, Q
+
+
+def init_random_digest(L: int, seed: int, nq: int = 4, precision: str = "fp32", row0: int = 0,
+                       rows: int | None = None):
+    """``state_digest(*init_random(...))`` without holding the state: for lattices beyond host memory."""
+    rows = L if rows is None else int(rows)
+    out = np.zeros(3, np.uint64)
+    if lib().oracle_init_random_digest(int(L), int(row0), rows, int(nq), int(precision == "fp32"),
+                                       int(seed) & (2 ** 64 - 1), out.ctypes.data):
+        raise ValueError(f"nq must be 4 or 8, got {nq}")
+    return tuple(int(x) for x in out)
+
+
+def explore_actions(L: int, seed: int, step: int, i0: int, i1: int):
+    """Actions (0 = C, 1 = D) of rows [i0, i1) at iteration ``step`` when epsilon = 1: every site explores
+    and takes bit 0 of its stream-0 Philox word (``site_word``)."""
+    a = np.empty((i1 - i0, L), np.uint8)
+    lib().oracle_explore_actions(int(L), int(i0), int(i1), int(seed) & (2 ** 64 - 1), int(step), a.ctypes.data)
+    return a
 
 
 class Sim:

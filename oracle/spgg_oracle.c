@@ -22,6 +22,10 @@
  * against oracle_step_f64 on dyadic parameter sets where both are exact.  For every TD rule
  * it follows k_step (csrc/spgg_kernels.cuh: td_update_f32 and the Double-Q branch).
  *
+ * The end of the file restates two helpers of the C ABI that the large-lattice tests check
+ * against: spgg_state_digest (also for a lattice that tiles a smaller state) and
+ * spgg_init_random, plus the actions of an iteration at epsilon = 1.
+ *
  * Build with -ffp-contract=off (see oracle/Makefile): the reference is NumPy,
  * every operation is individually rounded.
  */
@@ -559,4 +563,160 @@ int oracle_step_f32(const oracle_params_t *p, uint8_t *S, float *R, float *Q, do
   memcpy(R, Rn, n_sites * sizeof(float));
   free(N); free(SN); free(a); free(s_old); free(s_new); free(Rn); free(rew);
   return 0;
+}
+
+/* ================================================================ digests */
+/* k_state_digest (csrc/spgg_kernels.cuh): site (i, j) of global row i adds to each word
+ * (hash | 1) * (bits of its value as a double + 1) mod 2^64, the hash keyed by (i, j) and the
+ * word (S, R, Q entry z).  The odd multiplier is invertible mod 2^64, so a change of one value
+ * changes the sum. */
+static inline uint64_t digest_mix(uint64_t x) {
+  x ^= x >> 33; x *= 0xff51afd7ed558ccdull; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ull; x ^= x >> 33;
+  return x;
+}
+
+static inline uint64_t dbits(double v) {
+  uint64_t u;
+  memcpy(&u, &v, sizeof(u));
+  return u;
+}
+
+/* multipliers of the value slot (a, b): with period 0 those of site (row0 + a, b), with period P
+ * the sum over the sites (a + uP, b + vP) of the L x L lattice that carry that slot's value */
+static void slot_weights(int L, int row0, int period, int nq, int a, int b, uint64_t *w) {
+  const int k = period ? L / period : 1, step = period ? period : 0;
+  for (int m = 0; m < 2 + nq; ++m) w[m] = 0;
+  for (int u = 0; u < k; ++u)
+    for (int v = 0; v < k; ++v) {
+      const uint64_t key = ((uint64_t)(uint32_t)(row0 + a + u * step) << 32) | (uint32_t)(b + v * step);
+      w[0] += digest_mix(key * 3 + 1) | 1u;
+      w[1] += digest_mix(key * 3 + 2) | 1u;
+      for (int z = 0; z < nq; ++z) w[2 + z] += digest_mix(key * 3 + 3 + ((uint64_t)(z + 1) << 58)) | 1u;
+    }
+}
+
+static int digest_geometry(int L, int rows, int period, int *nr, int *nc) {
+  if (period) {
+    if (period < 1 || L % period != 0) return -1;
+    *nr = *nc = period;
+  } else {
+    *nr = rows; *nc = L;
+  }
+  return 0;
+}
+
+int oracle_digest_weights(int L, int row0, int rows, int period, int nq, uint64_t *w) {
+  int nr, nc;
+  if (digest_geometry(L, rows, period, &nr, &nc)) return -1;
+  const int nw = 2 + nq;
+#pragma omp parallel for schedule(dynamic, 1)
+  for (int a = 0; a < nr; ++a)
+    for (int b = 0; b < nc; ++b) slot_weights(L, row0, period, nq, a, b, w + ((size_t)a * nc + b) * nw);
+  return 0;
+}
+
+int oracle_state_digest(int L, int row0, int rows, int period, int nq, const uint8_t *S,
+                        const double *R, const double *Q, const uint64_t *w, uint64_t out[3]) {
+  int nr, nc;
+  if (digest_geometry(L, rows, period, &nr, &nc)) return -1;
+  const int nw = 2 + nq;
+  uint64_t dS = 0, dR = 0, dQ = 0;
+#pragma omp parallel for schedule(dynamic, 1) reduction(+ : dS, dR, dQ)
+  for (int a = 0; a < nr; ++a)
+    for (int b = 0; b < nc; ++b) {
+      const size_t x = (size_t)a * nc + b;
+      uint64_t ws[2 + 8];
+      const uint64_t *wx = ws;
+      if (w) wx = w + x * nw;
+      else slot_weights(L, row0, period, nq, a, b, ws);
+      dS += wx[0] * (uint64_t)((S[x] != 0) + 1);
+      dR += wx[1] * (dbits(R[x]) + 1);
+      if (Q)
+        for (int z = 0; z < nq; ++z) dQ += wx[2 + z] * (dbits(Q[x * nq + z]) + 1);
+    }
+  out[0] = dS; out[1] = dR; out[2] = Q ? dQ : 0;
+  return 0;
+}
+
+/* ============================================================ k_init_random */
+/* Q entry z of table t of site (i, j): Philox counter (j, row0 + i, t, 1), word z; the device
+ * evaluates -0.01 + 0.02 * u as one fused multiply-add in double, then rounds to the Q type */
+static inline double init_q(uint32_t word, int fp32) {
+  const double uu = (double)(word >> 8) * (1.0 / 16777216.0);
+  const double q = fma(0.02, uu, -0.01);
+  return fp32 ? (double)(float)q : q;
+}
+
+/* strategy word wi of global row gi: counter (wi >> 2, gi, 0, 2), word wi & 3, masked beyond L */
+static inline uint32_t init_s_word(uint64_t seed, int L, int gi, int wi) {
+  const uint32_t ctr[4] = {(uint32_t)(wi >> 2), (uint32_t)gi, 0u, 2u};
+  const uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
+  uint32_t w[4];
+  oracle_philox4x32_10(ctr, key, w);
+  uint32_t word = w[wi & 3];
+  const int rem = L - wi * 32;
+  if (rem < 32) word &= (1u << rem) - 1u;
+  return word;
+}
+
+static inline void init_q_site(uint64_t seed, int gi, int j, int nq, int fp32, double *q) {
+  const uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
+  for (int t = 0; t < nq / 4; ++t) {
+    const uint32_t ctr[4] = {(uint32_t)j, (uint32_t)gi, (uint32_t)t, 1u};
+    uint32_t w[4];
+    oracle_philox4x32_10(ctr, key, w);
+    for (int z = 0; z < 4; ++z) q[4 * t + z] = init_q(w[z], fp32);
+  }
+}
+
+void oracle_init_random(int L, int row0, int rows, int nq, int fp32, uint64_t seed, uint8_t *S, double *R,
+                        double *Q) {
+  const int nW = (L + 31) >> 5;
+#pragma omp parallel for schedule(static)
+  for (int i = 0; i < rows; ++i) {
+    for (int wi = 0; wi < nW; ++wi) {
+      const uint32_t word = init_s_word(seed, L, row0 + i, wi);
+      for (int c = wi * 32; c < L && c < wi * 32 + 32; ++c) S[(size_t)i * L + c] = (uint8_t)((word >> (c & 31)) & 1u);
+    }
+    for (int j = 0; j < L; ++j) {
+      const size_t x = (size_t)i * L + j;
+      R[x] = 0.0;
+      init_q_site(seed, row0 + i, j, nq, fp32, Q + x * nq);
+    }
+  }
+}
+
+int oracle_init_random_digest(int L, int row0, int rows, int nq, int fp32, uint64_t seed, uint64_t out[3]) {
+  if (nq != 4 && nq != 8) return -1;
+  const int nW = (L + 31) >> 5;
+  uint64_t dS = 0, dR = 0, dQ = 0;
+#pragma omp parallel for schedule(dynamic, 1) reduction(+ : dS, dR, dQ)
+  for (int i = 0; i < rows; ++i)
+    for (int wi = 0; wi < nW; ++wi) {
+      const uint32_t word = init_s_word(seed, L, row0 + i, wi);
+      for (int j = wi * 32; j < L && j < wi * 32 + 32; ++j) {
+        uint64_t ws[2 + 8];
+        double q[8];
+        slot_weights(L, row0, 0, nq, i, j, ws);
+        init_q_site(seed, row0 + i, j, nq, fp32, q);
+        dS += ws[0] * (uint64_t)(((word >> (j & 31)) & 1u) + 1);
+        dR += ws[1] * (dbits(0.0) + 1);
+        for (int z = 0; z < nq; ++z) dQ += ws[2 + z] * (dbits(q[z]) + 1);
+      }
+    }
+  out[0] = dS; out[1] = dR; out[2] = dQ;
+  return 0;
+}
+
+/* ======================================================== epsilon = 1 actions */
+void oracle_explore_actions(int L, int i0, int i1, uint64_t seed, uint32_t step, uint8_t *a) {
+  const uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
+#pragma omp parallel for schedule(static)
+  for (int i = i0; i < i1; ++i)
+    for (int j4 = 0; j4 < L; j4 += 4) {
+      const uint32_t ctr[4] = {(uint32_t)(j4 >> 2), (uint32_t)i, step, 0u};
+      uint32_t w[4];
+      oracle_philox4x32_10(ctr, key, w);
+      for (int z = 0; z < 4 && j4 + z < L; ++z) a[(size_t)(i - i0) * L + j4 + z] = (uint8_t)(w[z] & 1u);
+    }
 }

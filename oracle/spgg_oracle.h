@@ -93,6 +93,34 @@ void oracle_reward_table(const oracle_params_t *p, float *tab128);
 
 int oracle_num_threads(void);
 
+/* spgg_state_digest restated (csrc/spgg_kernels.cuh: k_state_digest): out[0] strategies, out[1]
+ * reputations, out[2] Q, each the sum mod 2^64 over sites of (hash | 1) * (value bits + 1).
+ * S: bytes (0 = C, else D); R, Q (nq = 4 or 8 per site): the values as the device holds them,
+ * widened to double (int8 units times rq, fp32, fp64).  Q == NULL leaves out[2] = 0.
+ * period == 0: the arrays hold `rows` rows of an L-wide lattice starting at global row row0.
+ * period == P: they hold a P x P state, and the digest is that of the L x L lattice (L % P == 0,
+ * rows from row0) whose site (i, j) holds the value of (i % P, j % P).
+ * w: NULL, or the multipliers oracle_digest_weights computed for the same geometry, which makes
+ * repeated digests of a periodic lattice cost P*P instead of L*L hashes.  Returns 0, or -1 when
+ * P does not divide L. */
+int oracle_state_digest(int L, int row0, int rows, int period, int nq, const uint8_t *S,
+                        const double *R, const double *Q, const uint64_t *w, uint64_t out[3]);
+/* w: (rows * L or P * P) * (2 + nq) multipliers, per slot S, R, Q[0..nq) */
+int oracle_digest_weights(int L, int row0, int rows, int period, int nq, uint64_t *w);
+
+/* spgg_init_random restated (k_init_random): rows [row0, row0 + rows) of an L x L lattice.  Q
+ * entry z of table t at site (i, j) from Philox counter (j, i, t, 1) word z, rounded to float
+ * when fp32; strategy word w of row i from counter (w / 4, i, 0, 2) word w % 4, bits beyond
+ * column L - 1 masked; R = 0. */
+void oracle_init_random(int L, int row0, int rows, int nq, int fp32, uint64_t seed, uint8_t *S, double *R,
+                        double *Q);
+/* the digest of that state, without holding it: for lattices too large for host memory */
+int oracle_init_random_digest(int L, int row0, int rows, int nq, int fp32, uint64_t seed, uint64_t out[3]);
+
+/* actions (0 = C, 1 = D) of rows [i0, i1) at iteration `step` when epsilon = 1: every site
+ * explores, and its action is bit 0 of its stream-0 Philox word (oracle_site_word) */
+void oracle_explore_actions(int L, int i0, int i1, uint64_t seed, uint32_t step, uint8_t *a);
+
 #ifdef __cplusplus
 }
 #endif
