@@ -164,8 +164,9 @@ int spgg_r_histogram(spgg_t *h, int replica, int n_bins, const double *edges, in
  * increasing order of each cluster's smallest linear index row*L + col, which is scipy's
  * numbering; the result does not depend on scheduling.  Sees the state spgg_get_state
  * would return.  Whole-lattice handles only (rows == L, rows*L < 2^31; else
- * SPGG_E_UNSUPPORTED).  The result stays on the handle for the two getters below until
- * the next spgg_clusters call or until the state changes (spgg_step / spgg_begin_steps,
+ * SPGG_E_UNSUPPORTED; a strip labels through spgg_strip_clusters below).  The result stays
+ * on the handle for the two getters below until the next spgg_clusters /
+ * spgg_strip_clusters call or until the state changes (spgg_step / spgg_begin_steps,
  * spgg_set_state, spgg_init_random, spgg_set_progress, spgg_strip_rewind); the getters
  * return SPGG_E_STATE without one.  The first call allocates device scratch that the
  * handle keeps until spgg_destroy: 8 bytes a site (union-find parents and set sizes),
@@ -173,8 +174,40 @@ int spgg_r_histogram(spgg_t *h, int replica, int n_bins, const double *edges, in
  * 12.25 bytes a site in all (206 MB at L=4096, 13.2 GB at L=32768). */
 #define SPGG_CLUSTER_PERIODIC 1
 int spgg_clusters(spgg_t *h, int replica, int which, int flags, int64_t *n_clusters);
-int spgg_cluster_sizes(spgg_t *h, int64_t *sizes, int64_t n);   /* n must equal n_clusters: sizes[k-1] = #sites of label k */
-int spgg_cluster_labels(spgg_t *h, int32_t *labels);            /* rows*L values, row-major, 0 where not selected */
+/* After spgg_clusters: sizes[k-1] = #sites of label k, n must equal n_clusters.  After
+ * spgg_strip_clusters_resolve: the n_owned clusters whose smallest site lies in this strip,
+ * in raster order, i.e. labels first_label+1 .. first_label+n_owned. */
+int spgg_cluster_sizes(spgg_t *h, int64_t *sizes, int64_t n);
+/* rows*L values, row-major, 0 where not selected; on a strip the labels of the whole lattice
+ * (a site of a cluster whose smallest site lies in another strip gets that cluster's label). */
+int spgg_cluster_labels(spgg_t *h, int32_t *labels);
+
+/* The same labelling of a lattice split into row strips, one handle (single replica) per
+ * rank; the result is defined on the whole L x L lattice and equals spgg_clusters of one
+ * handle holding it, bit for bit.  Needs L*L < 2^31 (global site indices are int32), else
+ * SPGG_E_UNSUPPORTED.  Per call, on every rank:
+ *   1. spgg_strip_clusters labels this strip's rows (replica 0, current state, after
+ *      finishing a pending chunk) and writes one boundary record of
+ *      spgg_strip_cluster_record_bytes() bytes (device memory; depends on L only) - the
+ *      strip's number of clusters and, for each site of its first and last row, its
+ *      cluster within the strip, with that cluster's smallest site, raster rank and size;
+ *   2. the caller gathers the records of all `world` ranks, in rank order, into one device
+ *      buffer on every rank (one all-gather);
+ *   3. spgg_strip_clusters_resolve joins the clusters across the strip boundaries (and
+ *      across row L-1 | 0 with SPGG_CLUSTER_PERIODIC; the column seam is joined in step 1),
+ *      on the device and the same way on every rank.  It returns this strip's number of
+ *      owned clusters, the label before the first of them and the number of clusters of
+ *      the lattice; spgg_cluster_sizes / spgg_cluster_labels above then serve the result.
+ * The records must agree on L, which and flags and their rows must tile [0, L) in rank
+ * order (else SPGG_E_INVALID).  A pass that is not resolved yet counts as no result for
+ * the getters; the events listed at spgg_clusters discard both.  Scratch: that of
+ * spgg_clusters for the strip's rows*L sites, 8 bytes per boundary site (a site of the
+ * strip's first or last row) for building the record, whose 16 bytes per boundary site
+ * the caller provides, and, in the resolution, 16 bytes per boundary site of every strip. */
+int64_t spgg_strip_cluster_record_bytes(spgg_t *h);
+int spgg_strip_clusters(spgg_t *h, int which, int flags, void *dev_record);
+int spgg_strip_clusters_resolve(spgg_t *h, int world, int rank, const void *dev_records,
+                                int64_t *n_owned, int64_t *first_label, int64_t *n_total);
 
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox

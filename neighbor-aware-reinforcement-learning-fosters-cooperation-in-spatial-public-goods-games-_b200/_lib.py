@@ -64,6 +64,7 @@ EXPORTS = (
     "spgg_strip_report_ptr", "spgg_strip_verify", "spgg_strip_failed", "spgg_strip_rewind",
     "spgg_r_histogram", "spgg_ipc_export", "spgg_ipc_attach", "spgg_ring_export", "spgg_ring_attach",
     "spgg_clusters", "spgg_cluster_sizes", "spgg_cluster_labels",
+    "spgg_strip_cluster_record_bytes", "spgg_strip_clusters", "spgg_strip_clusters_resolve",
 )
 
 _lib = None
@@ -109,6 +110,10 @@ def load():
     lib.spgg_clusters.argtypes = [vp, i32, i32, i32, C.POINTER(i64)]
     lib.spgg_cluster_sizes.argtypes = [vp, vp, i64]
     lib.spgg_cluster_labels.argtypes = [vp, vp]
+    lib.spgg_strip_cluster_record_bytes.argtypes = [vp]
+    lib.spgg_strip_cluster_record_bytes.restype = i64
+    lib.spgg_strip_clusters.argtypes = [vp, i32, i32, vp]
+    lib.spgg_strip_clusters_resolve.argtypes = [vp, i32, i32, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]
     lib.spgg_ipc_export.argtypes = [vp, vp]
     lib.spgg_ipc_attach.argtypes = [vp, i32, vp, i32, i32]
     lib.spgg_ring_export.argtypes = [vp, vp]

@@ -141,6 +141,11 @@ struct spgg_handle {
   CclScratch ccl;
   bool ccl_valid = false;
   int64_t ccl_n = 0;
+  // spgg_strip_clusters: record / resolution scratch, and the strip-local pass awaiting its resolution
+  CclStripScratch ccl_strip;
+  bool ccl_local = false;
+  int ccl_which = 0, ccl_flags = 0;
+  int64_t ccl_local_n = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -342,6 +347,7 @@ static int free_all(spgg_handle *h) {
   cudaFree(h->d_sc_S); cudaFree(h->d_sc_R); cudaFree(h->d_sc_Q); cudaFree(h->d_sc_info);
   cudaFree(h->d_gimg); cudaFree(h->d_gpart); cudaFree(h->d_gnsel);
   ccl_free(&h->ccl);
+  ccl_strip_free(&h->ccl_strip);
   return 0;
 }
 
@@ -770,7 +776,7 @@ extern "C" int spgg_set_state(spgg_t *h, int rep, const uint8_t *S, const double
   if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
   int rcode = finish_pending(h);
   if (rcode) return rcode;
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   CUDA_TRY(cudaSetDevice(h->device));
   rcode = ensure_scratch(h, true);
   if (rcode) return rcode;
@@ -905,7 +911,7 @@ extern "C" int spgg_begin_steps(spgg_t *h, int n_steps, void *stream_) {
   if (n_steps < 1) return fail(SPGG_E_INVALID, "n_steps must be >= 1");
   int rcode = finish_pending(h);
   if (rcode) return rcode;
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   for (int r = 0; r < h->n_rep; ++r)
     if (h->stale[r])
       return fail(SPGG_E_STATE, "replica %d still holds the state of the previous run: give every replica of a "
@@ -1275,7 +1281,7 @@ extern "C" int spgg_init_random(spgg_t *h, int rep, uint64_t seed) {
   if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
   int rcode = finish_pending(h);
   if (rcode) return rcode;
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   CUDA_TRY(cudaSetDevice(h->device));
   const uint32_t lo = (uint32_t)seed, hi = (uint32_t)(seed >> 32);
   const int grid = 148 * 8;
@@ -1305,7 +1311,7 @@ extern "C" int spgg_set_progress(spgg_t *h, int64_t iteration, const double *eps
     if (!(epsilon[r] >= 0.0 && epsilon[r] <= 1.0)) return fail(SPGG_E_INVALID, "epsilon[%d] = %g outside [0, 1]", r, epsilon[r]);
   }
   if (h->iter != 0) return fail(SPGG_E_STATE, "spgg_set_progress follows the state uploads of a resumed run");
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   CUDA_TRY(cudaSetDevice(h->device));
   h->iter = (long long)iteration;
   h->replay_first = h->iter;
@@ -1383,9 +1389,9 @@ extern "C" int spgg_clusters(spgg_t *h, int rep, int which, int flags, int64_t *
   if ((long long)h->g.rows * h->g.L >= (1ll << 31)) return fail(SPGG_E_UNSUPPORTED, "cluster labelling needs rows*L < 2^31");
   int rcode = finish_pending(h);
   if (rcode) return rcode;
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   CUDA_TRY(cudaSetDevice(h->device));
-  cudaError_t e = ccl_alloc(&h->ccl, h->g.L);
+  cudaError_t e = ccl_alloc(&h->ccl, h->g.rows, h->g.L);
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     return fail(SPGG_E_CUDA, "spgg_clusters: scratch for L=%d: %s", h->g.L, cudaGetErrorString(e));
@@ -1396,6 +1402,7 @@ extern "C" int spgg_clusters(spgg_t *h, int rep, int which, int flags, int64_t *
   e = launch_clusters(h->ccl, S, g.pitchW, which, flags & SPGG_CLUSTER_PERIODIC, &n);
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_clusters: %s", cudaGetErrorString(e));
   h->launches += 5;
+  h->ccl.base = 0;
   h->ccl_n = n;
   h->ccl_valid = true;
   *n_clusters = n;
@@ -1420,6 +1427,95 @@ extern "C" int spgg_cluster_labels(spgg_t *h, int32_t *labels) {
     e = cudaMemcpy(labels, h->ccl.total, sizeof(int32_t) * (size_t)h->g.rows * h->g.L, cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_cluster_labels: %s", cudaGetErrorString(e));
   h->launches += 1;
+  return SPGG_OK;
+}
+
+// Row strips (include/spgg.h): the strip-local labelling writes a boundary record; the records of all
+// ranks, gathered by the caller, are resolved into this strip's part of the whole lattice's labelling
+static int strip_clusters_supported(spgg_t *h, const char *fn) {
+  if (h->n_rep != 1) return fail(SPGG_E_UNSUPPORTED, "%s: strip labelling serves single-replica handles", fn);
+  if ((long long)h->g.L * h->g.L >= (1ll << 31))
+    return fail(SPGG_E_UNSUPPORTED, "%s: global site indices need L*L < 2^31 (L=%d)", fn, h->g.L);
+  return SPGG_OK;
+}
+
+extern "C" int64_t spgg_strip_cluster_record_bytes(spgg_t *h) {
+  if (!h) return fail(SPGG_E_INVALID, "null handle");
+  int rcode = strip_clusters_supported(h, "spgg_strip_cluster_record_bytes");
+  return rcode ? rcode : ccl_record_bytes(h->g.L);
+}
+
+extern "C" int spgg_strip_clusters(spgg_t *h, int which, int flags, void *dev_record) {
+  if (!h || !dev_record) return fail(SPGG_E_INVALID, "spgg_strip_clusters: null argument");
+  if (which != 0 && which != 1) return fail(SPGG_E_INVALID, "which must be 0 (cooperators) or 1 (defectors), got %d", which);
+  if (flags & ~SPGG_CLUSTER_PERIODIC) return fail(SPGG_E_INVALID, "unknown cluster flags 0x%x", flags);
+  int rcode = strip_clusters_supported(h, "spgg_strip_clusters");
+  if (rcode) return rcode;
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  h->ccl_valid = h->ccl_local = false;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const Geom &g = h->g;
+  cudaError_t e = ccl_alloc(&h->ccl, g.rows, g.L);
+  if (e == cudaSuccess) e = ccl_strip_alloc(&h->ccl_strip, g.L, 0);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(SPGG_E_CUDA, "spgg_strip_clusters: scratch for %d x %d sites: %s", g.rows, g.L, cudaGetErrorString(e));
+  }
+  const uint32_t *S = h->d_S[h->cur] + (size_t)GH * g.pitchW + WPAD;
+  e = launch_strip_clusters(h->ccl, h->ccl_strip, S, g.pitchW, g.row0, which, flags & SPGG_CLUSTER_PERIODIC, dev_record,
+                            &h->ccl_local_n);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_strip_clusters: %s", cudaGetErrorString(e));
+  h->launches += 9;   // seven kernels of ours, CUB's sort and unique counted as one each
+  h->ccl_local = true;
+  h->ccl_which = which;
+  h->ccl_flags = flags;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_strip_clusters_resolve(spgg_t *h, int world, int rank, const void *dev_records, int64_t *n_owned,
+                                           int64_t *first_label, int64_t *n_total) {
+  if (!h || !dev_records || !n_owned || !first_label || !n_total)
+    return fail(SPGG_E_INVALID, "spgg_strip_clusters_resolve: null argument");
+  if (world < 1 || rank < 0 || rank >= world) return fail(SPGG_E_INVALID, "rank %d outside a world of %d", rank, world);
+  if (!h->ccl_local) return fail(SPGG_E_STATE, "spgg_strip_clusters_resolve: no spgg_strip_clusters pass of the current state");
+  const Geom &g = h->g;
+  const long long rb = ccl_record_bytes(g.L);
+  std::vector<int> hd((size_t)world * CCL_REC_HDR);
+  CUDA_TRY(cudaSetDevice(h->device));
+  CUDA_TRY(cudaMemcpy2D(hd.data(), CCL_REC_HDR * sizeof(int), dev_records, (size_t)rb, CCL_REC_HDR * sizeof(int), world,
+                        cudaMemcpyDeviceToHost));
+  int next = 0;
+  for (int k = 0; k < world; ++k) {
+    const int *r = hd.data() + (size_t)k * CCL_REC_HDR;
+    if (r[CCL_H_MAGIC] != CCL_REC_MAGIC) return fail(SPGG_E_INVALID, "record %d is not a strip cluster record", k);
+    if (r[CCL_H_L] != g.L) return fail(SPGG_E_INVALID, "record %d: L = %d, this handle's L = %d", k, r[CCL_H_L], g.L);
+    if (r[CCL_H_WHICH] != h->ccl_which || r[CCL_H_FLAGS] != h->ccl_flags)
+      return fail(SPGG_E_INVALID, "record %d: which %d / flags 0x%x, this strip labelled which %d / flags 0x%x", k,
+                  r[CCL_H_WHICH], r[CCL_H_FLAGS], h->ccl_which, h->ccl_flags);
+    if (r[CCL_H_ROW0] != next || r[CCL_H_ROWS] < 1 || r[CCL_H_ROWS] > g.L - next)
+      return fail(SPGG_E_INVALID, "record %d: rows [%d, %d) do not continue the strips above at row %d", k, r[CCL_H_ROW0],
+                  r[CCL_H_ROW0] + r[CCL_H_ROWS], next);
+    if (r[CCL_H_NPARTS] < 0 || r[CCL_H_NPARTS] > 2 * g.L || r[CCL_H_NLOCAL] < r[CCL_H_NPARTS])
+      return fail(SPGG_E_INVALID, "record %d: %d boundary roots of %d roots", k, r[CCL_H_NPARTS], r[CCL_H_NLOCAL]);
+    next += r[CCL_H_ROWS];
+  }
+  if (next != g.L) return fail(SPGG_E_INVALID, "the %d records cover rows [0, %d) of %d", world, next, g.L);
+  const int *mine = hd.data() + (size_t)rank * CCL_REC_HDR;
+  if (mine[CCL_H_ROW0] != g.row0 || mine[CCL_H_ROWS] != g.rows || mine[CCL_H_NLOCAL] != h->ccl_local_n)
+    return fail(SPGG_E_INVALID, "record %d is not this strip's (rows [%d, %d))", rank, g.row0, g.row0 + g.rows);
+  cudaError_t e = ccl_strip_alloc(&h->ccl_strip, g.L, world);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(SPGG_E_CUDA, "spgg_strip_clusters_resolve: scratch for %d records: %s", world, cudaGetErrorString(e));
+  }
+  h->ccl_local = false;   // the resolution rewrites the strip-local result
+  e = launch_strip_resolve(h->ccl, h->ccl_strip, dev_records, world, rank, h->ccl_flags & SPGG_CLUSTER_PERIODIC, n_owned,
+                           first_label, n_total);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_strip_clusters_resolve: %s", cudaGetErrorString(e));
+  h->launches += 10;
+  h->ccl_n = *n_owned;
+  h->ccl_valid = true;
   return SPGG_OK;
 }
 
@@ -1559,7 +1655,7 @@ extern "C" int spgg_strip_rewind(spgg_t *h, int bad) {
   if (!h || !h->pending || !h->d_bad) return fail(SPGG_E_STATE, "spgg_strip_rewind outside a chunk");
   if (bad < 1 || bad > h->pend_n) return fail(SPGG_E_INVALID, "launch %d outside the chunk of %d", bad, h->pend_n);
   h->in_rerun = true;   // (the test hook does not spoil re-runs; cleared by the next spgg_begin_steps)
-  h->ccl_valid = false;
+  h->ccl_valid = h->ccl_local = false;
   if (h->d_ring) {      // ring mode: every rank empties its own ring and starts counting launches again; the
     CUDA_TRY(cudaMemset(h->d_ring, 0, sizeof(unsigned) * RING_SLOTS * RING_WORDS));  // caller puts a barrier
     h->gen = 0;                                                                        // between this and the re-run

@@ -53,6 +53,14 @@ def params_struct(p: dict, seed: int = 0, precision: str = "fp32", rows=None, ro
         wP=float(p.get("reward_weight_payoff", 1.0)), seed=int(seed) & (2 ** 64 - 1))
 
 
+def cluster_which(of) -> int:
+    """``of`` of the cluster methods -> the ``which`` of the C ABI (0 cooperators, 1 defectors)."""
+    which = {"C": 0, "D": 1, 0: 0, 1: 1}.get(of if isinstance(of, (str, int)) and not isinstance(of, bool) else None)
+    if which is None:
+        raise ValueError(f"of must be 'C' or 'D' (or 0 / 1), got {of!r}")
+    return which
+
+
 class Engine:
     """``n`` independent lattices on one device.  ``param_list`` is one dict (or a
     sequence of dicts, one per replica) with the reference ctor's argument names."""
@@ -165,9 +173,7 @@ class Engine:
 
     # -- clusters (include/spgg.h: spgg_clusters)
     def _clusters(self, replica, of, periodic) -> int:
-        which = {"C": 0, "D": 1, 0: 0, 1: 1}.get(of if isinstance(of, (str, int)) and not isinstance(of, bool) else None)
-        if which is None:
-            raise ValueError(f"of must be 'C' or 'D' (or 0 / 1), got {of!r}")
+        which = cluster_which(of)
         n = C.c_int64()
         L_.check(self.lib.spgg_clusters(self._h, int(replica), which, L_.CLUSTER_PERIODIC if periodic else 0,
                                         C.byref(n)))

@@ -257,6 +257,91 @@ class StripEngine:
         self.dist.all_gather_object(parts, [int(x) for x in d], group=self.group)
         return tuple(sum(p[i] for p in parts) % 2 ** 64 for i in range(3))
 
+    # -- clusters (include/spgg.h: spgg_strip_clusters)
+    def _clusters(self, of, periodic) -> int:
+        """Label the whole lattice: strip-local pass, one all-gather of the boundary records, resolution
+        on every rank.  Returns the number of clusters this strip owns; ``_n_total``: those of the lattice."""
+        return self._resolve_records(self._gather_records(self._label_strip(of, periodic)))
+
+    def _label_strip(self, of, periodic):
+        """Strip-local labelling; returns the device buffer of all ranks' records with this rank's filled in."""
+        from .engine import cluster_which
+        lib, h = self.lib, self.h
+        which = cluster_which(of)
+        self._settle()
+        nb = int(lib.spgg_strip_cluster_record_bytes(h))
+        L_.check(min(nb, 0))
+        rec = self.torch.empty(self.world * nb, dtype=self.torch.uint8, device=self.dev)
+        mine = rec[self.rank * nb:(self.rank + 1) * nb]
+        L_.check(lib.spgg_strip_clusters(h, which, L_.CLUSTER_PERIODIC if periodic else 0, mine.data_ptr()))
+        return rec
+
+    def _gather_records(self, rec):
+        """The one collective of the labelling: every rank's record into every rank's buffer, in rank order."""
+        torch = self.torch
+        if self.world == 1:
+            return rec
+        nb = rec.numel() // self.world
+        mine = rec[self.rank * nb:(self.rank + 1) * nb]
+        if self.host_staged:
+            hrec = torch.empty(rec.numel(), dtype=torch.uint8).pin_memory()
+            hmine = torch.empty(nb, dtype=torch.uint8).pin_memory()
+            hmine.copy_(mine)
+            self.dist.all_gather(list(hrec.split(nb)), hmine, group=self.group)
+            rec.copy_(hrec)
+        else:
+            self.dist.all_gather_into_tensor(rec, mine.clone(), group=self.group)
+        torch.cuda.current_stream().synchronize()
+        return rec
+
+    def _resolve_records(self, rec) -> int:
+        n, first, total = C.c_int64(), C.c_int64(), C.c_int64()
+        L_.check(self.lib.spgg_strip_clusters_resolve(self.h, self.world, self.rank, rec.data_ptr(), C.byref(n),
+                                                      C.byref(first), C.byref(total)))
+        self._n_total = int(total.value)
+        return int(n.value)
+
+    def _owned_sizes(self, n: int) -> np.ndarray:
+        sizes = np.empty(n, np.int64)
+        L_.check(self.lib.spgg_cluster_sizes(self.h, sizes.ctypes.data, n))
+        return sizes
+
+    def _gather_sizes(self, sizes: np.ndarray) -> np.ndarray:
+        """Every rank's owned sizes, concatenated in rank order (= label order), on every rank."""
+        torch = self.torch
+        if self.world == 1:
+            return sizes
+        counts = [None] * self.world
+        self.dist.all_gather_object(counts, len(sizes), group=self.group)
+        pad = max(max(counts), 1)
+        t = torch.zeros(pad, dtype=torch.int64)
+        t[:len(sizes)] = torch.from_numpy(sizes)
+        if self.host_staged:
+            parts = [torch.empty_like(t) for _ in range(self.world)]
+            self.dist.all_gather(parts, t, group=self.group)
+            out = torch.cat([p[:c] for p, c in zip(parts, counts)])
+        else:
+            td = t.to(self.dev)
+            allp = torch.empty(self.world * pad, dtype=torch.int64, device=self.dev)
+            self.dist.all_gather_into_tensor(allp, td, group=self.group)
+            out = torch.cat([p[:c] for p, c in zip(allp.split(pad), counts)]).cpu()
+        return out.numpy()
+
+    def cluster_sizes(self, of="C", periodic: bool = False) -> np.ndarray:
+        """``Engine.cluster_sizes`` of the WHOLE lattice (all ranks call this; every rank gets the same
+        int64 array): sizes of the 4-connected clusters of cooperators (``of="C"``) or defectors (``"D"``)
+        in the order of each cluster's first site in raster order, ``periodic=True`` joining clusters
+        across the edges of the torus."""
+        return self._gather_sizes(self._owned_sizes(self._clusters(of, periodic)))
+
+    def cluster_labels(self, of="C", periodic: bool = False):
+        """This rank's rows of ``scipy.ndimage.label(S == of)`` over the whole lattice (all ranks call
+        this): (labels int32 (rows, L), n) with n the number of clusters of the lattice."""
+        self._clusters(of, periodic)
+        labels = np.empty((self.rows, self.L), np.int32)
+        L_.check(self.lib.spgg_cluster_labels(self.h, labels.ctypes.data))
+        return labels, self._n_total
+
     # -- stepping
     def _stream(self):
         return C.c_void_p(self.torch.cuda.current_stream().cuda_stream)
