@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -151,6 +152,7 @@ struct spgg_handle {
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
   size_t elem_val() const { return mode == MODE_F64 ? 8 : 4; }
   int nq() const { return params[0].algorithm == SPGG_ALGO_DOUBLE_QLEARNING ? 8 : 4; }  // Q values per site
+  ~spgg_handle();  // frees whatever device memory and peer mappings the handle holds
 };
 
 // ---------------------------------------------------------------- constants
@@ -204,21 +206,26 @@ static void build_repconst(const spgg_params_t &p, RepConst *rc) {
 }
 
 // ---------------------------------------------------------------- dispatch
-// the general and the lean kernels are instantiated in their own translation units (spgg_dispatch.h)
-static size_t step_smem(int mode, int TR) {
+// f(ModeF32I8{}), f(ModeF32F{}) or f(ModeF64{}): the host side of a kernel templated on the arithmetic mode.
+// The general and the lean kernels are instantiated in their own translation units (spgg_dispatch.h)
+template <class F>
+static auto with_mode(int mode, F &&f) {
   switch (mode) {
-    case MODE_F32_I8: return SmemLayout<ModeF32I8>(TR).total;
-    case MODE_F32_F: return SmemLayout<ModeF32F>(TR).total;
-    default: return SmemLayout<ModeF64>(TR).total;
+    case MODE_F32_I8: return f(ModeF32I8{});
+    case MODE_F32_F: return f(ModeF32F{});
+    default: return f(ModeF64{});
   }
 }
 
+static size_t step_smem(int mode, int TR) {
+  return with_mode(mode, [&](auto md) { return SmemLayout<decltype(md)>(TR).total; });
+}
+
 // launch with programmatic stream serialization (the fast kernels call griddepcontrol.wait
-// before touching anything an earlier kernel wrote); SPGG_NO_PDL=1 falls back to plain launches
+// before touching anything an earlier kernel wrote)
 template <class... KArgsT, class... Args>
 static cudaError_t launch_pdl(void (*kern)(KArgsT...), int grid, int block, size_t smem, cudaStream_t st,
                               Args... args) {
-  static const bool use_pdl = getenv("SPGG_NO_PDL") == nullptr;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3((unsigned)block);
@@ -228,7 +235,7 @@ static cudaError_t launch_pdl(void (*kern)(KArgsT...), int grid, int block, size
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 
@@ -281,23 +288,31 @@ static ResGeom resident_geom(int L, int cs, size_t smem_limit, int grid = 0) {
   rg.QR = (L + 3) / 4;
   rg.pitch = (RG + rg.QR * 4 + RG + 15) / 16 * 16;
   const int quads = rg.rows_max * rg.QR;
-  int max_thr = RES_THREADS;
-  if (const char *e = getenv("SPGG_RES_THREADS")) max_thr = std::max(64, std::min(RES_THREADS, atoi(e) / 32 * 32));  // tuning experiments
-  rg.threads = std::max(64, std::min(max_thr, (quads + 31) / 32 * 32));
+  rg.threads = std::max(64, std::min(RES_THREADS, (quads + 31) / 32 * 32));
   rg.CS = (ResSmem(rg).total <= smem_limit) ? cs : 0;
   return rg;
 }
 
-static int make_map(CUtensorMap *map, void *base, uint64_t row_bytes, uint64_t n_rows, uint64_t n_rep,
-                    uint64_t rep_stride_bytes, uint32_t box_bytes, uint32_t box_rows, uint64_t visible_bytes = 0) {
+// the driver's cuTensorMapEncodeTiled, or 0 with the error set
+static PFN_cuTensorMapEncodeTiled_v12000 tensor_map_encoder() {
   static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
   if (!encode) {
     void *fn = nullptr;
     cudaDriverEntryPointQueryResult q;
-    CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
-    if (!fn || q != cudaDriverEntryPointSuccess) return fail(SPGG_E_CUDA, "cuTensorMapEncodeTiled not available");
+    const cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q);
+    if (e != cudaSuccess || !fn || q != cudaDriverEntryPointSuccess) {
+      fail(SPGG_E_CUDA, "cuTensorMapEncodeTiled not available (%s)", cudaGetErrorString(e));
+      return nullptr;
+    }
     encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
   }
+  return encode;
+}
+
+static int make_map(CUtensorMap *map, void *base, uint64_t row_bytes, uint64_t n_rows, uint64_t n_rep,
+                    uint64_t rep_stride_bytes, uint32_t box_bytes, uint32_t box_rows, uint64_t visible_bytes = 0) {
+  const PFN_cuTensorMapEncodeTiled_v12000 encode = tensor_map_encoder();
+  if (!encode) return SPGG_E_CUDA;
   // visible_bytes < row_bytes: the tensor ends before the pitch (loads beyond it give zeros, stores are dropped)
   const cuuint64_t dims[3] = {visible_bytes ? visible_bytes : row_bytes, n_rows, n_rep};
   const cuuint64_t strides[2] = {row_bytes, rep_stride_bytes};
@@ -314,14 +329,8 @@ static int make_map(CUtensorMap *map, void *base, uint64_t row_bytes, uint64_t n
 // 128-site row segment, 128-byte swizzle so that a lane's four consecutive float4 are
 // conflict-free in shared memory
 static int make_map_q(CUtensorMap *map, void *base, uint64_t L, uint64_t n_rows, uint64_t n_rep) {
-  static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
-  if (!encode) {
-    void *fn = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
-    if (!fn || q != cudaDriverEntryPointSuccess) return fail(SPGG_E_CUDA, "cuTensorMapEncodeTiled not available");
-    encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
-  }
+  const PFN_cuTensorMapEncodeTiled_v12000 encode = tensor_map_encoder();
+  if (!encode) return SPGG_E_CUDA;
   const cuuint64_t dims[4] = {128, L / 8, n_rows, n_rep};
   const cuuint64_t strides[3] = {128, L * 16, n_rows * L * 16};
   const cuuint32_t box[4] = {128, TC / 8, (cuuint32_t)FastSmem<1>::kRowsPerWarp, 1};  // a warp's rows of a tile
@@ -337,25 +346,22 @@ static int make_map_q(CUtensorMap *map, void *base, uint64_t L, uint64_t n_rows,
 extern "C" int spgg_abi_version(void) { return SPGG_ABI_VERSION; }
 extern "C" const char *spgg_last_error(void) { return g_err.c_str(); }
 
-static int free_all(spgg_handle *h) {
-  for (void *p : h->ipc_opened) cudaIpcCloseMemHandle(p);
-  h->ipc_opened.clear();
-  cudaFree(h->d_rc); cudaFree(h->d_valtab); cudaFree(h->d_Qb[0]); cudaFree(h->d_Qb[1]); cudaFree(h->d_gcarry); cudaFree(h->d_bad); cudaFree(h->d_gvec); cudaFree(h->d_ring);
-  for (int i = 0; i < 2; ++i) { cudaFree(h->d_R[i]); cudaFree(h->d_code[i]); cudaFree(h->d_S[i]); }
-  cudaFree(h->d_gmax); cudaFree(h->d_stats); cudaFree(h->d_partials); cudaFree(h->d_tickets);
-  cudaFree(h->d_stop); cudaFree(h->d_eps); cudaFree(h->d_thr); cudaFree(h->d_u); cudaFree(h->d_b);
-  cudaFree(h->d_sc_S); cudaFree(h->d_sc_R); cudaFree(h->d_sc_Q); cudaFree(h->d_sc_info);
-  cudaFree(h->d_gimg); cudaFree(h->d_gpart); cudaFree(h->d_gnsel);
-  ccl_free(&h->ccl);
-  ccl_strip_free(&h->ccl_strip);
-  return 0;
+spgg_handle::~spgg_handle() {
+  for (void *p : ipc_opened) cudaIpcCloseMemHandle(p);
+  cudaFree(d_rc); cudaFree(d_valtab); cudaFree(d_Qb[0]); cudaFree(d_Qb[1]); cudaFree(d_gcarry); cudaFree(d_bad); cudaFree(d_gvec); cudaFree(d_ring);
+  for (int i = 0; i < 2; ++i) { cudaFree(d_R[i]); cudaFree(d_code[i]); cudaFree(d_S[i]); }
+  cudaFree(d_gmax); cudaFree(d_stats); cudaFree(d_partials); cudaFree(d_tickets);
+  cudaFree(d_stop); cudaFree(d_eps); cudaFree(d_thr); cudaFree(d_u); cudaFree(d_b);
+  cudaFree(d_sc_S); cudaFree(d_sc_R); cudaFree(d_sc_Q); cudaFree(d_sc_info);
+  cudaFree(d_gimg); cudaFree(d_gpart); cudaFree(d_gnsel);
+  ccl_free(&ccl);
+  ccl_strip_free(&ccl_strip);
 }
 
 extern "C" void spgg_destroy(spgg_t *h) {
   if (!h) return;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
-  free_all(h);
   delete h;
 }
 
@@ -386,7 +392,9 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   if (device < 0 || device >= ndev) return fail(SPGG_E_CUDA, "device %d not available (%d devices)", device, ndev);
   CUDA_TRY(cudaSetDevice(device));
 
-  spgg_handle *h = new spgg_handle();
+  // owned until it is complete: every error return below frees what was built so far
+  std::unique_ptr<spgg_handle> hp(new spgg_handle());
+  spgg_handle *h = hp.get();
   h->device = device;
   h->n_rep = n_replicas;
   h->params.assign(params, params + n_replicas);
@@ -402,7 +410,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   if (p0.precision == SPGG_PREC_FP64) h->mode = MODE_F64;
   else if (p0.r_storage == SPGG_RSTORE_FP32) h->mode = MODE_F32_F;
   else if (p0.r_storage == SPGG_RSTORE_INT8) {
-    if (!all_i8) { delete h; return fail(SPGG_E_INVALID, "reputation parameters are not representable in int8 units"); }
+    if (!all_i8) return fail(SPGG_E_INVALID, "reputation parameters are not representable in int8 units");
     h->mode = MODE_F32_I8;
   } else h->mode = all_i8 ? MODE_F32_I8 : MODE_F32_F;
 
@@ -412,13 +420,11 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   g.pitchW = WPAD + ((p0.L + 31) / 32 + 3) / 4 * 4 + WPAD;
   // fast path (spgg_fast.cuh): int8 throughput mode on 128-aligned lattices, |R| <= 15 units
   {
-    const RepConst &r0 = h->rc_host[0];
     bool ok = (h->mode == MODE_F32_I8) && (g.L % 32 == 0) && (g.L >= TC) && (g.rows % FTR == 0) &&
               p0.algorithm == SPGG_ALGO_QLEARNING && getenv("SPGG_NO_FAST") == nullptr;
     for (int r = 0; r < n_replicas && ok; ++r)
       ok = h->rc_host[r].rmin_i >= -15 && h->rc_host[r].rmax_i <= 15 && h->rc_host[r].gain_i >= 0 &&
            h->rc_host[r].loss_i >= 0;
-    (void)r0;
     h->fast = ok;
   }
   // resident path (spgg_resident.cuh): whole lattice, int8 throughput mode, Q-learning, on-chip fit
@@ -434,8 +440,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
     // clusters of 8 CTAs (15 co-resident on a B200) serve batches best; a lattice that is alone (or
     // nearly) on the GPU, or too large for 8 blocks, is spread over a non-portable cluster of 16
     ResGeom rg = resident_geom(g.L, 8, lim);
-    if (eligible && g.L >= 32 && (rg.CS == 0 || n_replicas <= 4 || getenv("SPGG_RES_CS16") != nullptr) &&
-        getenv("SPGG_RES_CS8") == nullptr) {
+    if (eligible && g.L >= 32 && (rg.CS == 0 || n_replicas <= 4) && getenv("SPGG_RES_CS8") == nullptr) {
       const ResGeom rg16 = resident_geom(g.L, 16, lim);
       if (rg16.CS == 16 &&
           cudaFuncSetAttribute(rf, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
@@ -486,10 +491,6 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   }
   g.TR = h->fast ? FTR : (g.rows >= 512 ? 16 : (g.rows >= 64 ? 8 : 4));
   h->threads = h->fast ? FTHREADS : 32 * std::min(8, g.TR);
-  if (!h->fast && getenv("SPGG_GEN_TR") && getenv("SPGG_GEN_THREADS")) {   // tuning experiments: tile rows / block size of the general path
-    g.TR = std::max(4, std::min(16, atoi(getenv("SPGG_GEN_TR"))));
-    h->threads = std::max(32, std::min(256, atoi(getenv("SPGG_GEN_THREADS")) / 32 * 32));
-  }
   g.n_tx = (g.L + TC - 1) / TC;
   g.n_ty = (g.rows + g.TR - 1) / g.TR;
   g.n_rep = n_replicas;
@@ -534,7 +535,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   }
   CUDA_TRY(cudaFuncSetAttribute(pick_gmax_lean(h->mode, h->M), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)h->smem_gmax));
-  if (occ < 1) { delete h; return fail(SPGG_E_CUDA, "kernel does not fit on an SM (smem %zu)", h->smem_step); }
+  if (occ < 1) return fail(SPGG_E_CUDA, "kernel does not fit on an SM (smem %zu)", h->smem_step);
   const long long n_tiles = (long long)g.n_tx * g.n_ty;
   long long per_rep = std::max<long long>(1, ((long long)prop.multiProcessorCount * occ) / n_replicas);
   g.ctas_per_rep = (int)std::min<long long>(n_tiles, per_rep);
@@ -554,10 +555,8 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
 #define ALLOC(ptr, bytes)                                                                   \
   do {                                                                                      \
     cudaError_t e_ = cudaMalloc((void **)&(ptr), (bytes));                                  \
-    if (e_ != cudaSuccess) {                                                                \
-      free_all(h); delete h;                                                                \
+    if (e_ != cudaSuccess)                                                                  \
       return fail(SPGG_E_CUDA, "cudaMalloc(%zu bytes) failed: %s", (size_t)(bytes), cudaGetErrorString(e_)); \
-    }                                                                                       \
     cudaMemset((ptr), 0, (bytes));                                                          \
   } while (0)
   ALLOC(h->d_rc, sizeof(RepConst) * n_replicas);
@@ -586,16 +585,14 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
       if (!e) e = make_map(&fm.st_R, h->d_R[i ^ 1], (uint64_t)g.pitchB, nrows, n_replicas, (uint64_t)g.plane_stride, TC, FTR, (uint64_t)(CPAD + g.L));
       if (!e) e = make_map(&fm.st_S, h->d_S[i ^ 1], (uint64_t)g.pitchW * 4, nrows, n_replicas, (uint64_t)g.bits_stride * 4, TC / 8, FTR);
       if (!e) e = make_map_q(&h->qmaps[i], h->d_Qb[(i == 1 && h->spec) ? 1 : 0], (uint64_t)g.L, (uint64_t)g.rows, (uint64_t)n_replicas);
-      if (e) { free_all(h); delete h; return e; }
+      if (e) return e;
     }
   }
   CUDA_TRY(cudaMemcpy(h->d_rc, h->rc_host.data(), sizeof(RepConst) * n_replicas, cudaMemcpyHostToDevice));
   if (h->mode == MODE_F64) {
     const size_t vb = sizeof(double) * 2 * ((size_t)n_replicas << VALTAB_BITS);
-    if (cudaMalloc((void **)&h->d_valtab, vb) != cudaSuccess) {
-      free_all(h); delete h;
+    if (cudaMalloc((void **)&h->d_valtab, vb) != cudaSuccess)
       return fail(SPGG_E_CUDA, "cudaMalloc(%zu bytes) failed (reward table)", vb);
-    }
     CUDA_TRY(launch_build_valtab(h->d_rc, h->d_valtab, n_replicas));
   }
   std::vector<int> neg(n_replicas, -1);
@@ -608,7 +605,7 @@ extern "C" int spgg_create(const spgg_params_t *params, int n_replicas, int devi
   for (int r = 0; r < n_replicas; ++r) h->eps_cur[r] = params[r].epsilon;
   h->stop_at.assign(n_replicas, -1);
   h->stale.assign(n_replicas, 0);
-  *out = h;
+  *out = hp.release();
   return SPGG_OK;
 }
 
@@ -645,7 +642,6 @@ static int rerun_failed_speculation(spgg_handle *h) {
     int bad = 0x7fffffff;
     CUDA_TRY(cudaMemcpy(&bad, h->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
     if (bad == 0x7fffffff) return SPGG_OK;
-    if (getenv("SPGG_SPEC_DEBUG")) fprintf(stderr, "[spgg] speculation failed at launch %d of %d (t0 %lld), %lld speculative launches so far\n", bad, h->pend_n, h->pend_t0, h->spec_launches);
     if (bad < 1 || bad > h->pend_n) return fail(SPGG_E_STATE, "speculation bookkeeping out of range (%d of %d)", bad, h->pend_n);
     int rcode0 = rewind_to_failed_launch(h, bad);
     if (rcode0) return rcode0;
@@ -791,12 +787,10 @@ extern "C" int spgg_set_state(spgg_t *h, int rep, const uint8_t *S, const double
     CUDA_TRY(cudaMemcpyAsync(h->d_sc_R, R + off, n * sizeof(double), cudaMemcpyHostToDevice, 0));
     CUDA_TRY(cudaMemcpyAsync(h->d_sc_Q, Q + off * h->nq(), n * h->nq() * sizeof(double), cudaMemcpyHostToDevice, 0));
     const int grid = (int)std::min<long long>(148 * 16, ((long long)nr * ((g.L + 31) / 32) * 32 + 255) / 256);
-#define IMPORT(Md) k_import_rows<Md><<<std::max(1, grid), 256>>>(g, rep, i0, nr, h->d_sc_S, h->d_sc_R, h->d_sc_Q, \
-                       h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], rc.rq, h->d_sc_info, h->nq())
-    if (h->mode == MODE_F32_I8) IMPORT(ModeF32I8);
-    else if (h->mode == MODE_F32_F) IMPORT(ModeF32F);
-    else IMPORT(ModeF64);
-#undef IMPORT
+    with_mode(h->mode, [&](auto md) {
+      k_import_rows<decltype(md)><<<std::max(1, grid), 256>>>(g, rep, i0, nr, h->d_sc_S, h->d_sc_R, h->d_sc_Q,
+          h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], rc.rq, h->d_sc_info, h->nq());
+    });
     CUDA_TRY(cudaGetLastError());
     h->launches += 1;
   }
@@ -838,12 +832,10 @@ extern "C" int spgg_get_state(spgg_t *h, int rep, uint8_t *S, double *R, double 
     const int nr = std::min(chunk, g.rows - i0);
     const size_t n = (size_t)nr * g.L, off = (size_t)i0 * g.L;
     const int grid = (int)std::min<long long>(148 * 16, ((long long)n + 255) / 256);
-#define EXPORT(Md) k_export_rows<Md><<<std::max(1, grid), 256>>>(g, rep, i0, nr, S ? h->d_sc_S : nullptr, \
-                       R ? h->d_sc_R : nullptr, Q ? h->d_sc_Q : nullptr, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], rc.rq, h->nq())
-    if (h->mode == MODE_F32_I8) EXPORT(ModeF32I8);
-    else if (h->mode == MODE_F32_F) EXPORT(ModeF32F);
-    else EXPORT(ModeF64);
-#undef EXPORT
+    with_mode(h->mode, [&](auto md) {
+      k_export_rows<decltype(md)><<<std::max(1, grid), 256>>>(g, rep, i0, nr, S ? h->d_sc_S : nullptr,
+          R ? h->d_sc_R : nullptr, Q ? h->d_sc_Q : nullptr, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], rc.rq, h->nq());
+    });
     CUDA_TRY(cudaGetLastError());
     h->launches += 1;
     if (S) CUDA_TRY(cudaMemcpyAsync(S + off, h->d_sc_S, n, cudaMemcpyDeviceToHost, 0));
@@ -1285,9 +1277,9 @@ extern "C" int spgg_init_random(spgg_t *h, int rep, uint64_t seed) {
   CUDA_TRY(cudaSetDevice(h->device));
   const uint32_t lo = (uint32_t)seed, hi = (uint32_t)(seed >> 32);
   const int grid = 148 * 8;
-  if (h->mode == MODE_F32_I8) k_init_random<ModeF32I8><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], lo, hi, h->nq());
-  else if (h->mode == MODE_F32_F) k_init_random<ModeF32F><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], lo, hi, h->nq());
-  else k_init_random<ModeF64><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], lo, hi, h->nq());
+  with_mode(h->mode, [&](auto md) {
+    k_init_random<decltype(md)><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], lo, hi, h->nq());
+  });
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaDeviceSynchronize());
   h->launches += 1;
@@ -1335,11 +1327,9 @@ extern "C" int spgg_state_digest(spgg_t *h, int rep, uint64_t out[3]) {
   CUDA_TRY(cudaMemset(d_out, 0, 3 * sizeof(unsigned long long)));
   const int grid = 148 * 8;
   const double rq = h->rc_host[rep].rq;
-#define DIGEST(Md) k_state_digest<Md><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], h->nq(), rq, d_out)
-  if (h->mode == MODE_F32_I8) DIGEST(ModeF32I8);
-  else if (h->mode == MODE_F32_F) DIGEST(ModeF32F);
-  else DIGEST(ModeF64);
-#undef DIGEST
+  with_mode(h->mode, [&](auto md) {
+    k_state_digest<decltype(md)><<<grid, 256>>>(h->g, rep, h->Qcur(), h->d_R[h->cur], h->d_S[h->cur], h->nq(), rq, d_out);
+  });
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess) e = cudaMemcpy(out, d_out, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
   cudaFree(d_out);
@@ -1363,11 +1353,9 @@ extern "C" int spgg_r_histogram(spgg_t *h, int rep, int n_bins, const double *ed
   cudaMemset(d_cnt, 0, sizeof(unsigned long long) * 64);
   const double rq = h->rc_host[rep].rq;
   const int grid = 148 * 8;
-#define HIST(Md) k_r_histogram<Md><<<grid, 256>>>(h->g, rep, h->d_R[h->cur], rq, n_bins, d_edges, d_cnt)
-  if (h->mode == MODE_F32_I8) HIST(ModeF32I8);
-  else if (h->mode == MODE_F32_F) HIST(ModeF32F);
-  else HIST(ModeF64);
-#undef HIST
+  with_mode(h->mode, [&](auto md) {
+    k_r_histogram<decltype(md)><<<grid, 256>>>(h->g, rep, h->d_R[h->cur], rq, n_bins, d_edges, d_cnt);
+  });
   unsigned long long host_cnt[64];
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess) e = cudaMemcpy(host_cnt, d_cnt, sizeof(unsigned long long) * 64, cudaMemcpyDeviceToHost);
@@ -1671,27 +1659,15 @@ extern "C" int64_t spgg_halo_bytes(spgg_t *h) {
   return per_rep * h->n_rep;
 }
 
-template <class Md>
-static void launch_pack(spgg_handle *h, void *up, void *down, cudaStream_t st) {
-  const long long rep_bytes = spgg_halo_bytes(h) / h->n_rep;
-  dim3 grid(std::max(1, std::min(64, (GH * h->g.pitchB + 255) / 256)), h->n_rep);
-  k_halo_pack<Md><<<grid, 256, 0, st>>>(h->g, h->d_code[h->cur], h->d_R[h->cur], h->d_S[h->cur],
-                                        (unsigned char *)up, (unsigned char *)down, rep_bytes);
-}
-template <class Md>
-static void launch_unpack(spgg_handle *h, const void *up, const void *down, cudaStream_t st) {
-  const long long rep_bytes = spgg_halo_bytes(h) / h->n_rep;
-  dim3 grid(std::max(1, std::min(64, (GH * h->g.pitchB + 255) / 256)), h->n_rep);
-  k_halo_unpack<Md><<<grid, 256, 0, st>>>(h->g, h->d_code[h->cur], h->d_R[h->cur], h->d_S[h->cur],
-                                          (const unsigned char *)up, (const unsigned char *)down, rep_bytes);
-}
-
 extern "C" int spgg_halo_pack(spgg_t *h, void *to_up, void *to_down, void *stream_) {
   if (!h || !to_up || !to_down) return fail(SPGG_E_INVALID, "spgg_halo_pack: null argument");
   cudaStream_t st = (cudaStream_t)stream_;
-  if (h->mode == MODE_F32_I8) launch_pack<ModeF32I8>(h, to_up, to_down, st);
-  else if (h->mode == MODE_F32_F) launch_pack<ModeF32F>(h, to_up, to_down, st);
-  else launch_pack<ModeF64>(h, to_up, to_down, st);
+  const long long rep_bytes = spgg_halo_bytes(h) / h->n_rep;
+  const dim3 grid(std::max(1, std::min(64, (GH * h->g.pitchB + 255) / 256)), h->n_rep);
+  with_mode(h->mode, [&](auto md) {
+    k_halo_pack<decltype(md)><<<grid, 256, 0, st>>>(h->g, h->d_code[h->cur], h->d_R[h->cur], h->d_S[h->cur],
+        (unsigned char *)to_up, (unsigned char *)to_down, rep_bytes);
+  });
   CUDA_TRY(cudaGetLastError());
   h->launches += 1;
   return SPGG_OK;
@@ -1700,9 +1676,12 @@ extern "C" int spgg_halo_pack(spgg_t *h, void *to_up, void *to_down, void *strea
 extern "C" int spgg_halo_unpack(spgg_t *h, const void *from_up, const void *from_down, void *stream_) {
   if (!h || !from_up || !from_down) return fail(SPGG_E_INVALID, "spgg_halo_unpack: null argument");
   cudaStream_t st = (cudaStream_t)stream_;
-  if (h->mode == MODE_F32_I8) launch_unpack<ModeF32I8>(h, from_up, from_down, st);
-  else if (h->mode == MODE_F32_F) launch_unpack<ModeF32F>(h, from_up, from_down, st);
-  else launch_unpack<ModeF64>(h, from_up, from_down, st);
+  const long long rep_bytes = spgg_halo_bytes(h) / h->n_rep;
+  const dim3 grid(std::max(1, std::min(64, (GH * h->g.pitchB + 255) / 256)), h->n_rep);
+  with_mode(h->mode, [&](auto md) {
+    k_halo_unpack<decltype(md)><<<grid, 256, 0, st>>>(h->g, h->d_code[h->cur], h->d_R[h->cur], h->d_S[h->cur],
+        (const unsigned char *)from_up, (const unsigned char *)from_down, rep_bytes);
+  });
   CUDA_TRY(cudaGetLastError());
   h->launches += 1;
   return SPGG_OK;

@@ -20,10 +20,7 @@ step_fn_t pick_step(int mode, int M, int action, int replay);
 step_fn_t pick_lean(int mode, int M, int action, int replay);
 gmax_fn_t pick_gmax_lean(int mode, int M);
 cudaError_t launch_build_valtab(const RepConst *rc_all, double *tab, int n_rep);
-#ifndef SPGG_LEAN_TR_MAX
-#define SPGG_LEAN_TR_MAX 16
-#endif
-constexpr int LEAN_TR_MAX = SPGG_LEAN_TR_MAX;   // k_step_lean addresses the shared-memory layout of 16-row tiles
+constexpr int LEAN_TR_MAX = 16;   // k_step_lean addresses the shared-memory layout of 16-row tiles
 // spgg_clusters.cu: ccl_alloc / ccl_free / launch_clusters / launch_cluster_labels (spgg_clusters.cuh)
 
 }  // namespace spgg

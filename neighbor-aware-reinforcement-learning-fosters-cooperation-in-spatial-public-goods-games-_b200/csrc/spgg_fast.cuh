@@ -22,17 +22,11 @@
 
 namespace spgg {
 
-#ifndef SPGG_FTR
-#define SPGG_FTR 16
-#endif
-#ifndef SPGG_FTHREADS
-#define SPGG_FTHREADS 256
-#endif
-constexpr int FTR = SPGG_FTR;      // tile rows
+constexpr int FTR = 16;            // tile rows
 constexpr int FROWB = 160;         // staged row bytes of code / R: 16 ghost + 128 + 16 ghost
 constexpr int FROWW = FROWB / 4;   // the same in 32-bit words
 constexpr int FSROWB = 48;         // staged row bytes of strategy bits: 16 + 16 + 16
-constexpr int FTHREADS = SPGG_FTHREADS;
+constexpr int FTHREADS = 256;
 
 template <int M>
 struct FastSmem {
@@ -157,9 +151,6 @@ struct FastMaps {
   CUtensorMap q_ld, q_st;
 };
 
-#ifndef SPGG_FAST_MINBLOCKS
-#define SPGG_FAST_MINBLOCKS 2
-#endif
 // UPD / SEL are compile-time so the four sites a thread handles per row form one straight-line
 // block the scheduler can interleave.
 // PART: the lattice side is a multiple of 32 but not of 128 - the last tile column is partial.  Its tiles
@@ -777,7 +768,7 @@ __device__ __forceinline__ void step_fast_body(const FastMaps &tm, const KArgs &
 }
 
 template <int M, bool ACTION, bool UPD, bool SEL, bool PART = false>
-__global__ void __launch_bounds__(FTHREADS, SPGG_FAST_MINBLOCKS)
+__global__ void __launch_bounds__(FTHREADS, 2)
 k_step_fast(const __grid_constant__ FastMaps tm, KArgs a) {
   pdl_launch_dependents();
   pdl_wait();  // the planes, the stop flags and gmax come from the kernels before this one

@@ -797,11 +797,8 @@ __device__ __forceinline__ float td_update_f32(const RepConst &rc, float vx, flo
 // The general kernel is latency-bound (one site per thread and row, dependent shared-memory stencils):
 // what it needs is resident warps, not registers.  Measured at L=4000 (fp32, int8 R), us per iteration:
 // 1 CTA/SM (190 registers) 1604, 2 CTAs/SM 891, 3 CTAs/SM (80 registers, a few hundred bytes of spills) 718.
-#ifndef SPGG_GEN_MINBLOCKS
-#define SPGG_GEN_MINBLOCKS 3
-#endif
 template <class Md, int M, bool ACTION, bool REPLAY>
-__global__ void __launch_bounds__(MAX_THREADS, SPGG_GEN_MINBLOCKS) k_step(KArgs a) {
+__global__ void __launch_bounds__(MAX_THREADS, 3) k_step(KArgs a) {
   typedef typename Md::Q QT;
   typedef typename Md::R RT;
   typedef typename Md::Code Code;

@@ -125,12 +125,14 @@ __global__ void __launch_bounds__(MAX_THREADS) k_gmax_lean(GArgs a) {
   }
 }
 
-#ifndef SPGG_LEAN_MINBLOCKS
-#define SPGG_LEAN_MINBLOCKS 2
-#endif
+// sites of a row whose Q (and draws) k_step_lean loads before it processes the first of them
+// (measured at L=4096 in fp64: batches of 4 sites 648 us per iteration, pairs 630)
+constexpr int LEAN_BATCH = 2;
 
+// 2 CTAs per SM: with 3 (80 registers, 336 B of spills) the fp64 iteration at L=4096 took 835 us instead of 611
+// (profiles/r02_fp64_lean.md)
 template <class Md, int M, bool ACTION, bool REPLAY>
-__global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(KArgs a) {
+__global__ void __launch_bounds__(MAX_THREADS, 2) k_step_lean(KArgs a) {
   typedef typename Md::Q QT;
   typedef typename Md::R RT;
   typedef typename Md::Code Code;
@@ -244,20 +246,16 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
       const int sr = rr + HR;
       uint32_t w4[4] = {0, 0, 0, 0};
       if (sel && !REPLAY) philox_row(c0, g.row0 + i, (uint32_t)(a.j + 1), 0u, rc, lane, w4);
-      // ---- everything that comes from global memory for a batch of sites, before the first is processed
-// (measured at L=4096 in fp64: batches of 4 sites 648 us per iteration, pairs 630)
-#ifndef SPGG_LEAN_BATCH
-#define SPGG_LEAN_BATCH 2
-#endif
+      // ---- everything that comes from global memory for a batch of LEAN_BATCH sites, before the first is processed
 #pragma unroll
-      for (int kb = 0; kb < 4; kb += SPGG_LEAN_BATCH) {
+      for (int kb = 0; kb < 4; kb += LEAN_BATCH) {
       QT q[4][4];
       [[maybe_unused]] double ru[4] = {0, 0, 0, 0};    // replayed draws
       [[maybe_unused]] uint8_t rb[4] = {0, 0, 0, 0};
       [[maybe_unused]] double rat[4] = {0, 0, 0, 0};   // fp64: ratio statistic of the site's code (second table column)
       const long long site_row = (long long)i * g.L + c0 + lane;
 #pragma unroll
-      for (int k4 = kb; k4 < kb + SPGG_LEAN_BATCH; ++k4) {
+      for (int k4 = kb; k4 < kb + LEAN_BATCH; ++k4) {
         const bool valid = FULL || (c0 + 32 * k4 + lane < g.L);
         const long long site = site_row + 32 * k4;
         if (valid) {
@@ -279,7 +277,7 @@ __global__ void __launch_bounds__(MAX_THREADS, SPGG_LEAN_MINBLOCKS) k_step_lean(
         }
       }
 #pragma unroll
-      for (int k4 = kb; k4 < kb + SPGG_LEAN_BATCH; ++k4) {
+      for (int k4 = kb; k4 < kb + LEAN_BATCH; ++k4) {
         const int cc = k4 * 32 + lane;
         const int col = c0 + cc;
         const bool valid = FULL || (col < g.L);
