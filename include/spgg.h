@@ -209,6 +209,41 @@ int spgg_strip_clusters(spgg_t *h, int which, int flags, void *dev_record);
 int spgg_strip_clusters_resolve(spgg_t *h, int world, int rank, const void *dev_records,
                                 int64_t *n_owned, int64_t *first_label, int64_t *n_total);
 
+/* Strategy pair counts of one replica on the device: for numpy axis ax and every offset d in
+ * 1..max_d, over the torus (indices mod L), n_CC = #sites x that cooperate with x + d*e_ax
+ * cooperating too, and n_diff = #sites x whose partner holds the other strategy.
+ * out: 2*(max_d+1)*2 int64, out[((ax*(max_d+1)) + d)*2 + k]; ax 0: (i,j)-(i+d,j), ax 1: (i,j)-(i,j+d);
+ * k 0: both cooperate, k 1: the two differ; d = 0: {n_C, 0}.  1 <= max_d <= L/2.
+ * The rest follows: n_DD = N - n_CC - n_diff, n_CD = n_DC = n_diff/2, and n_diff(ax, 1) / N is
+ * the interface density along ax: the fraction of the N nearest-neighbour bonds along that axis
+ * that join a cooperator and a defector.  Exact integers, so the result does not depend on scheduling.  Sees
+ * the state spgg_get_state would return; changes neither the state, the iteration counter, the
+ * statistics rows nor a cluster-labelling result.  Whole-lattice handles only (a strip gets
+ * SPGG_E_UNSUPPORTED and counts through spgg_strip_pair_counts below).  Cost: two launches,
+ * O(L^2 * max_d / 32) word operations per axis; keeps 32*(max_d+1) bytes of device scratch. */
+int spgg_pair_counts(spgg_t *h, int replica, int max_d, int64_t *out);
+
+/* The same counts of a lattice split into row strips, one single-replica handle per rank (a
+ * whole-lattice handle is a world of one).  The counts of strip k are those of the pairs whose
+ * site x lies in its rows; summed over the ranks they equal spgg_pair_counts of one handle holding
+ * the lattice.  The partners of axis 0 reach max_d rows past a strip, so per call, on every rank:
+ *   1. spgg_strip_pair_record writes this strip's record (device memory of
+ *      spgg_strip_pair_record_bytes(max_d, max_rows) bytes): a header (L, row0, rows, max_d) and
+ *      the strip's first min(max_d, rows) rows, packed, padded to max_rows rows.  max_rows must be
+ *      the same on every rank, at least min(max_d, rows) of every strip and at most max_d
+ *      (min(max_d, largest strip height) fits);
+ *   2. the caller gathers the records of all `world` ranks, in rank order, into one device
+ *      buffer on every rank (one all-gather);
+ *   3. spgg_strip_pair_counts assembles the max_d rows that follow the strip from the records
+ *      and writes this strip's counts into out (layout of spgg_pair_counts).
+ * Records that disagree on L, max_d or max_rows, or whose rows do not tile [0, L) in rank order,
+ * get SPGG_E_INVALID; handles of several replicas SPGG_E_UNSUPPORTED.  Steps 1 and 3 must see the
+ * same state.  Scratch: 4*max_d*ceil(L/32) bytes for the assembled rows. */
+int64_t spgg_strip_pair_record_bytes(spgg_t *h, int max_d, int max_rows);
+int spgg_strip_pair_record(spgg_t *h, int max_d, int max_rows, void *dev_record);
+int spgg_strip_pair_counts(spgg_t *h, int world, int rank, const void *dev_records, int max_d,
+                           int max_rows, int64_t *out);
+
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox
  * keyed by `seed`; for lattices too large to stage through host memory. */

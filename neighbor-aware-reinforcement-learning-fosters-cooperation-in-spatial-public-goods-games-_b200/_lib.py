@@ -65,6 +65,7 @@ EXPORTS = (
     "spgg_r_histogram", "spgg_ipc_export", "spgg_ipc_attach", "spgg_ring_export", "spgg_ring_attach",
     "spgg_clusters", "spgg_cluster_sizes", "spgg_cluster_labels",
     "spgg_strip_cluster_record_bytes", "spgg_strip_clusters", "spgg_strip_clusters_resolve",
+    "spgg_pair_counts", "spgg_strip_pair_record_bytes", "spgg_strip_pair_record", "spgg_strip_pair_counts",
 )
 
 _lib = None
@@ -114,6 +115,11 @@ def load():
     lib.spgg_strip_cluster_record_bytes.restype = i64
     lib.spgg_strip_clusters.argtypes = [vp, i32, i32, vp]
     lib.spgg_strip_clusters_resolve.argtypes = [vp, i32, i32, vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]
+    lib.spgg_pair_counts.argtypes = [vp, i32, i32, vp]
+    lib.spgg_strip_pair_record_bytes.argtypes = [vp, i32, i32]
+    lib.spgg_strip_pair_record_bytes.restype = i64
+    lib.spgg_strip_pair_record.argtypes = [vp, i32, i32, vp]
+    lib.spgg_strip_pair_counts.argtypes = [vp, i32, i32, vp, i32, i32, vp]
     lib.spgg_ipc_export.argtypes = [vp, vp]
     lib.spgg_ipc_attach.argtypes = [vp, i32, vp, i32, i32]
     lib.spgg_ring_export.argtypes = [vp, vp]

@@ -147,6 +147,10 @@ struct spgg_handle {
   bool ccl_local = false;
   int ccl_which = 0, ccl_flags = 0;
   int64_t ccl_local_n = 0;
+  // spgg_pair_counts / spgg_strip_pair_counts (spgg_pairs.cuh): the device counts and a strip's tail rows
+  unsigned long long *d_pair_cnt = nullptr;
+  uint32_t *d_pair_tail = nullptr;
+  size_t pair_cnt_n = 0, pair_tail_n = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -356,6 +360,7 @@ spgg_handle::~spgg_handle() {
   cudaFree(d_gimg); cudaFree(d_gpart); cudaFree(d_gnsel);
   ccl_free(&ccl);
   ccl_strip_free(&ccl_strip);
+  cudaFree(d_pair_cnt); cudaFree(d_pair_tail);
 }
 
 extern "C" void spgg_destroy(spgg_t *h) {
@@ -1504,6 +1509,144 @@ extern "C" int spgg_strip_clusters_resolve(spgg_t *h, int world, int rank, const
   h->launches += 10;
   h->ccl_n = *n_owned;
   h->ccl_valid = true;
+  return SPGG_OK;
+}
+
+// ---------------------------------------------------------------- pair counts
+// n_CC and n_diff of one replica's strategies at every offset 0..max_d along both axes (include/spgg.h); the
+// kernels live in spgg_pairs.cu.  Nothing here touches the state or a cluster-labelling result.
+static int pair_max_d(spgg_t *h, int max_d, const char *fn) {
+  if (max_d < 1 || max_d > h->g.L / 2) return fail(SPGG_E_INVALID, "%s: max_d = %d outside [1, L/2 = %d]", fn, max_d, h->g.L / 2);
+  return SPGG_OK;
+}
+
+// device counts for max_d, and room for tail_words words of tail rows
+static int pair_scratch(spgg_handle *h, int max_d, size_t tail_words) {
+  const size_t n = 4 * (size_t)(max_d + 1);
+  if (h->pair_cnt_n < n) {
+    cudaFree(h->d_pair_cnt);
+    h->d_pair_cnt = nullptr;
+    h->pair_cnt_n = 0;
+    CUDA_TRY(cudaMalloc((void **)&h->d_pair_cnt, n * sizeof(unsigned long long)));
+    h->pair_cnt_n = n;
+  }
+  if (h->pair_tail_n < tail_words) {
+    cudaFree(h->d_pair_tail);
+    h->d_pair_tail = nullptr;
+    h->pair_tail_n = 0;
+    CUDA_TRY(cudaMalloc((void **)&h->d_pair_tail, tail_words * sizeof(uint32_t)));
+    h->pair_tail_n = tail_words;
+  }
+  return SPGG_OK;
+}
+
+static const uint32_t *pair_plane(const spgg_handle *h, int rep) {
+  const Geom &g = h->g;
+  return h->d_S[h->cur] + (size_t)rep * g.bits_stride + (size_t)GH * g.pitchW + WPAD;
+}
+
+extern "C" int spgg_pair_counts(spgg_t *h, int rep, int max_d, int64_t *out) {
+  if (!h || !out) return fail(SPGG_E_INVALID, "spgg_pair_counts: null argument");
+  if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
+  if (!h->g.wrap_rows)
+    return fail(SPGG_E_UNSUPPORTED, "spgg_pair_counts needs the whole lattice (rows == L), not a strip: see spgg_strip_pair_counts");
+  int rcode = pair_max_d(h, max_d, "spgg_pair_counts");
+  if (rcode) return rcode;
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  rcode = pair_scratch(h, max_d, 0);
+  if (rcode) return rcode;
+  const Geom &g = h->g;
+  const uint32_t *S = pair_plane(h, rep);
+  cudaError_t e = launch_pair_counts(S, g.pitchW, g.rows, g.L, S, g.pitchW, max_d, h->d_pair_cnt, out);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_pair_counts: %s", cudaGetErrorString(e));
+  h->launches += 2;
+  return SPGG_OK;
+}
+
+// Row strips (include/spgg.h): a record of the strip's first min(max_d, rows) rows, padded to max_rows rows;
+// from the records of all ranks each strip assembles the max_d rows below it and counts its own sites' pairs
+static int strip_pairs_supported(spgg_t *h, int max_d, int max_rows, const char *fn) {
+  if (h->n_rep != 1) return fail(SPGG_E_UNSUPPORTED, "%s: strip pair counts serve single-replica handles", fn);
+  int rcode = pair_max_d(h, max_d, fn);
+  if (rcode) return rcode;
+  if (max_rows < std::min(max_d, h->g.rows) || max_rows > max_d)
+    return fail(SPGG_E_INVALID, "%s: max_rows = %d outside [min(max_d, rows) = %d, max_d = %d]", fn, max_rows,
+                std::min(max_d, h->g.rows), max_d);
+  return SPGG_OK;
+}
+
+extern "C" int64_t spgg_strip_pair_record_bytes(spgg_t *h, int max_d, int max_rows) {
+  if (!h) return fail(SPGG_E_INVALID, "null handle");
+  int rcode = strip_pairs_supported(h, max_d, max_rows, "spgg_strip_pair_record_bytes");
+  return rcode ? rcode : pair_record_bytes(h->g.L, max_rows);
+}
+
+extern "C" int spgg_strip_pair_record(spgg_t *h, int max_d, int max_rows, void *dev_record) {
+  if (!h || !dev_record) return fail(SPGG_E_INVALID, "spgg_strip_pair_record: null argument");
+  int rcode = strip_pairs_supported(h, max_d, max_rows, "spgg_strip_pair_record");
+  if (rcode) return rcode;
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const Geom &g = h->g;
+  cudaError_t e = launch_pair_record(pair_plane(h, 0), g.pitchW, g.row0, g.rows, g.L, max_d, max_rows, dev_record);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_strip_pair_record: %s", cudaGetErrorString(e));
+  h->launches += 1;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_strip_pair_counts(spgg_t *h, int world, int rank, const void *dev_records, int max_d, int max_rows,
+                                      int64_t *out) {
+  if (!h || !dev_records || !out) return fail(SPGG_E_INVALID, "spgg_strip_pair_counts: null argument");
+  if (world < 1 || rank < 0 || rank >= world) return fail(SPGG_E_INVALID, "rank %d outside a world of %d", rank, world);
+  int rcode = strip_pairs_supported(h, max_d, max_rows, "spgg_strip_pair_counts");
+  if (rcode) return rcode;
+  const Geom &g = h->g;
+  const long long rb = pair_record_bytes(g.L, max_rows);
+  std::vector<int> hd((size_t)world * PAIR_REC_HDR);
+  CUDA_TRY(cudaSetDevice(h->device));
+  for (int k = 0; k < world; ++k)
+    CUDA_TRY(cudaMemcpy(hd.data() + (size_t)k * PAIR_REC_HDR, (const char *)dev_records + k * rb, PAIR_REC_HDR * sizeof(int),
+                        cudaMemcpyDeviceToHost));
+  int next = 0;
+  for (int k = 0; k < world; ++k) {
+    const int *r = hd.data() + (size_t)k * PAIR_REC_HDR;
+    if (r[PAIR_H_MAGIC] != PAIR_REC_MAGIC) return fail(SPGG_E_INVALID, "record %d is not a strip pair record", k);
+    if (r[PAIR_H_L] != g.L) return fail(SPGG_E_INVALID, "record %d: L = %d, this handle's L = %d", k, r[PAIR_H_L], g.L);
+    if (r[PAIR_H_MAXD] != max_d || r[PAIR_H_MAXROWS] != max_rows)
+      return fail(SPGG_E_INVALID, "record %d: max_d %d / max_rows %d, this call's max_d %d / max_rows %d", k, r[PAIR_H_MAXD],
+                  r[PAIR_H_MAXROWS], max_d, max_rows);
+    if (r[PAIR_H_ROW0] != next || r[PAIR_H_ROWS] < 1 || r[PAIR_H_ROWS] > g.L - next)
+      return fail(SPGG_E_INVALID, "record %d: rows [%d, %d) do not continue the strips above at row %d", k, r[PAIR_H_ROW0],
+                  r[PAIR_H_ROW0] + r[PAIR_H_ROWS], next);
+    if (r[PAIR_H_NROWS] != std::min(max_d, r[PAIR_H_ROWS]) || r[PAIR_H_NROWS] > max_rows)   // the tail copy reads NROWS rows
+      return fail(SPGG_E_INVALID, "record %d holds %d rows, not min(max_d, rows) = %d within max_rows = %d", k,
+                  r[PAIR_H_NROWS], std::min(max_d, r[PAIR_H_ROWS]), max_rows);
+    next += r[PAIR_H_ROWS];
+  }
+  if (next != g.L) return fail(SPGG_E_INVALID, "the %d records cover rows [0, %d) of %d", world, next, g.L);
+  const int *mine = hd.data() + (size_t)rank * PAIR_REC_HDR;
+  if (mine[PAIR_H_ROW0] != g.row0 || mine[PAIR_H_ROWS] != g.rows)
+    return fail(SPGG_E_INVALID, "record %d is not this strip's (rows [%d, %d))", rank, g.row0, g.row0 + g.rows);
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  const int nW = (g.L + 31) / 32;
+  rcode = pair_scratch(h, max_d, (size_t)max_d * nW);
+  if (rcode) return rcode;
+  // the max_d rows below this strip: the first rows of the strips that follow it, in order, around the torus
+  // (every record holds min(max_d, rows) rows, so the walk ends within one turn)
+  for (int t = 0, k = (rank + 1) % world; t < max_d; k = (k + 1) % world) {
+    const int n = std::min(hd[(size_t)k * PAIR_REC_HDR + PAIR_H_NROWS], max_d - t);
+    CUDA_TRY(cudaMemcpy(h->d_pair_tail + (size_t)t * nW, (const char *)dev_records + k * rb + PAIR_REC_HDR * sizeof(int),
+                        (size_t)n * nW * sizeof(uint32_t), cudaMemcpyDeviceToDevice));
+    t += n;
+  }
+  cudaError_t e = launch_pair_counts(pair_plane(h, 0), g.pitchW, g.rows, g.L, h->d_pair_tail, nW, max_d, h->d_pair_cnt, out);
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_strip_pair_counts: %s", cudaGetErrorString(e));
+  h->launches += 2;
   return SPGG_OK;
 }
 

@@ -11,14 +11,6 @@
 
 namespace spgg {
 
-// the selected sites of word w of a row: S bit 1 = defect; bits beyond column L-1 are never selected
-__device__ __forceinline__ uint32_t ccl_word(const uint32_t *S, int pitchW, int L, int nW, int row, int w, int which) {
-  uint32_t v = S[(long long)row * pitchW + w];
-  v = which ? v : ~v;
-  if (w == nW - 1 && (L & 31)) v &= (1u << (L & 31)) - 1u;
-  return v;
-}
-
 // Union-find with parent[x] <= x: every root is the smallest index of its set.  A link is an atomicMin on
 // a root; if the root was linked meanwhile the loop goes on with the value it found (Playne & Hawick).
 __device__ __forceinline__ int ccl_find(const int *P, int x) {

@@ -29,6 +29,15 @@ constexpr int CCL_THREADS = CCL_TR * CCL_TWW;  // k_ccl_local: one thread per (r
 constexpr int CCL_WPB = 512;             // mask words per block of k_ccl_count / k_ccl_compact
 constexpr int CCL_SCAN_THREADS = 1024;
 
+// the selected sites of word w of a row: S bit 1 = defect; bits beyond column L-1 are never selected
+// (also read by the pair counts, spgg_pairs.cu)
+__device__ __forceinline__ uint32_t ccl_word(const uint32_t *S, int pitchW, int L, int nW, int row, int w, int which) {
+  uint32_t v = S[(long long)row * pitchW + w];
+  v = which ? v : ~v;
+  if (w == nW - 1 && (L & 31)) v &= (1u << (L & 31)) - 1u;
+  return v;
+}
+
 // Device scratch of the labelling, owned by the handle (allocated by the first spgg_clusters /
 // spgg_strip_clusters call) and sized for the handle's rows x L sites: 8 bytes a site (parent, total),
 // 2 bits a site (root mask, per-word rank offsets) and the sizes of at most ceil(rows*L/2) clusters

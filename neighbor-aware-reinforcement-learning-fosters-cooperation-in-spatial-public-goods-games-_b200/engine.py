@@ -61,6 +61,22 @@ def cluster_which(of) -> int:
     return which
 
 
+def pair_correlation(counts, n_sites: int) -> np.ndarray:
+    """Two-point correlation of the strategies from ``pair_counts`` (shape (2, max_d+1, 2)) of a lattice of
+    ``n_sites`` sites: C(ax, d) = (n_CC/N - f^2) / (f - f^2) with f = n_C/N, float64 of shape (2, max_d+1);
+    C(ax, 0) = 1, and NaN everywhere when f is 0 or 1 (no fluctuation to correlate).  The counts themselves
+    carry the other bond statistics: ``counts[:, 1, 1] / N`` is the interface density along each axis (the
+    fraction of nearest-neighbour bonds joining a cooperator and a defector)."""
+    c = np.asarray(counts, dtype=np.float64)
+    if c.ndim != 3 or c.shape[0] != 2 or c.shape[2] != 2 or c.shape[1] < 1:
+        raise ValueError(f"counts must have shape (2, max_d+1, 2), got {c.shape}")
+    N = float(n_sites)
+    f = c[0, 0, 0] / N
+    if f <= 0.0 or f >= 1.0:
+        return np.full(c.shape[:2], np.nan)
+    return (c[:, :, 0] / N - f * f) / (f - f * f)
+
+
 class Engine:
     """``n`` independent lattices on one device.  ``param_list`` is one dict (or a
     sequence of dicts, one per replica) with the reference ctor's argument names."""
@@ -196,6 +212,16 @@ class Engine:
         labels = np.empty((self.rows, self.L), np.int32)
         L_.check(self.lib.spgg_cluster_labels(self._h, labels.ctypes.data))
         return labels, n
+
+    # -- strategy pair counts (include/spgg.h: spgg_pair_counts)
+    def pair_counts(self, max_d: int, replica: int = 0) -> np.ndarray:
+        """Exact strategy pair counts over the torus, computed on the device: int64 of shape (2, max_d+1, 2)
+        with ``[ax, d, 0]`` the sites x that cooperate together with x + d along numpy axis ``ax`` and
+        ``[ax, d, 1]`` those whose partner holds the other strategy (``[ax, 0]`` = (n_C, 0));
+        1 <= max_d <= L/2.  ``pair_correlation`` turns them into C(d)."""
+        out = np.zeros((2, max(int(max_d), 0) + 1, 2), np.int64)
+        L_.check(self.lib.spgg_pair_counts(self._h, int(replica), int(max_d), out.ctypes.data))
+        return out
 
     def set_replay(self, u, b):
         """``u`` (n,rows,L) float64 and ``b`` (n,rows,L) 0/1: the reference's draw

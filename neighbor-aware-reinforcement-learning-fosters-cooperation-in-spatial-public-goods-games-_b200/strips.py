@@ -342,6 +342,32 @@ class StripEngine:
         L_.check(self.lib.spgg_cluster_labels(self.h, labels.ctypes.data))
         return labels, self._n_total
 
+    # -- strategy pair counts (include/spgg.h: spgg_strip_pair_counts)
+    def pair_counts(self, max_d: int) -> np.ndarray:
+        """``Engine.pair_counts`` of the WHOLE lattice (all ranks call this; every rank gets the same int64
+        array of shape (2, max_d+1, 2)): each strip counts the pairs whose first site it owns, from its own
+        rows and the first rows of the strips below it (one all-gather of fixed-size records); the counts
+        are summed over the ranks."""
+        lib, h, torch = self.lib, self.h, self.torch
+        max_d = int(max_d)
+        self._settle()
+        # the padding every rank agrees on: no strip holds more rows than the largest
+        max_rows = min(max_d, max(strip_rows(self.L, self.world, r)[1] for r in range(self.world)))
+        nb = int(lib.spgg_strip_pair_record_bytes(h, max_d, max_rows))
+        L_.check(min(nb, 0))
+        rec = torch.empty(self.world * nb, dtype=torch.uint8, device=self.dev)
+        L_.check(lib.spgg_strip_pair_record(h, max_d, max_rows, rec[self.rank * nb:(self.rank + 1) * nb].data_ptr()))
+        rec = self._gather_records(rec)
+        out = np.zeros((2, max_d + 1, 2), np.int64)
+        L_.check(lib.spgg_strip_pair_counts(h, self.world, self.rank, rec.data_ptr(), max_d, max_rows, out.ctypes.data))
+        if self.world == 1:
+            return out
+        t = torch.from_numpy(out)
+        if not self.host_staged:
+            t = t.to(self.dev)
+        self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM, group=self.group)
+        return t.cpu().numpy()
+
     # -- stepping
     def _stream(self):
         return C.c_void_p(self.torch.cuda.current_stream().cuda_stream)
