@@ -244,6 +244,35 @@ int spgg_strip_pair_record(spgg_t *h, int max_d, int max_rows, void *dev_record)
 int spgg_strip_pair_counts(spgg_t *h, int world, int rank, const void *dev_records, int max_d,
                            int max_rows, int64_t *out);
 
+/* Block fields of one replica on the device: the lattice cut into B x B blocks of b x b sites,
+ * B = ceil(L/b), anchored at site (0, 0), no wrap; block (I, J) covers global rows
+ * [I*b, min((I+1)*b, L)) and columns [J*b, min((J+1)*b, L)), so the last block row and column
+ * are ragged when b does not divide L.  1 <= b <= L and B*B <= 2^24 (L = 32768 needs b >= 8).
+ *   counts[(i*B + J)*2 + k]: int64, k 0 the sites of the block, k 1 its cooperators (S == 0);
+ *   sums[((i*B + J)*2 + k)*m + ch]: float64, k 0 over all sites of the block, k 1 over its
+ *     cooperators (defectors: the difference); channels ch: with SPGG_BLOCK_R first R as
+ *     spgg_get_state returns it (int8 units x quantum), with SPGG_BLOCK_Q then the nq Q entries
+ *     in spgg_get_state's order; m = (flags & R) + (flags & Q ? nq : 0).  sums may be null when
+ *     flags == 0 (counts only: reads the bit plane alone).
+ * i runs over the block rows I0 .. I1 that hold rows of the handle, I = I0 + i: a whole lattice
+ * has I0 = 0, I1 = B-1; a strip (rows < L) has I0 = floor(row0/b), I1 = floor((row0+rows-1)/b),
+ * and each block holds the contribution of the strip's own rows only, so blocks that straddle
+ * a strip boundary are partial and the results of the strips add up to the lattice's.
+ * Exactness: counts and int8-storage R sums are exact (the quantum is 2^-k).  fp32 and fp64
+ * values are summed in fp64 in an order fixed by (L, row0, rows, b), without floating-point
+ * atomics: the same state gives bit-identical sums, whichever kernel path or chunking reached
+ * it; a sum of n values x_i differs from the exact one by at most (n-1) 2^-53 sum |x_i|.
+ * Sees the state spgg_get_state would return (a pending chunk is finished first); changes
+ * neither the state, the iteration counter, the statistics rows, a cluster-labelling result
+ * nor the pair-count scratch.  SPGG_E_INVALID: bad replica, b, B, unknown flag bits, null
+ * counts, null sums with flags != 0.  Cost: one streaming pass over the bit plane and, if
+ * asked, over R and Q; keeps device scratch of 8 bytes per block, plus 16*m bytes per block
+ * with flags != 0 and 16*m bytes per piece when b > 32 (pieces per block: ceil(b/32) *
+ * ceil(b/256)), grown to the largest call and freed with the handle. */
+#define SPGG_BLOCK_R 1
+#define SPGG_BLOCK_Q 2
+int spgg_block_fields(spgg_t *h, int replica, int b, int flags, int64_t *counts, double *sums);
+
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox
  * keyed by `seed`; for lattices too large to stage through host memory. */

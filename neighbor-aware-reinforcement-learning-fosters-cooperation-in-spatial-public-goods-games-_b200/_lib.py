@@ -29,6 +29,7 @@ ALGO_QLEARNING, ALGO_SARSA, ALGO_EXPECTED_SARSA, ALGO_DOUBLE_QLEARNING = 0, 1, 2
 RSTORE_AUTO, RSTORE_INT8, RSTORE_FP32 = 0, 1, 2
 E_INVALID, E_CUDA, E_STATE, E_UNSUPPORTED = -1, -2, -3, -4
 CLUSTER_PERIODIC = 1
+BLOCK_R, BLOCK_Q = 1, 2
 
 
 class Params(C.Structure):
@@ -66,6 +67,7 @@ EXPORTS = (
     "spgg_clusters", "spgg_cluster_sizes", "spgg_cluster_labels",
     "spgg_strip_cluster_record_bytes", "spgg_strip_clusters", "spgg_strip_clusters_resolve",
     "spgg_pair_counts", "spgg_strip_pair_record_bytes", "spgg_strip_pair_record", "spgg_strip_pair_counts",
+    "spgg_block_fields",
 )
 
 _lib = None
@@ -120,6 +122,7 @@ def load():
     lib.spgg_strip_pair_record_bytes.restype = i64
     lib.spgg_strip_pair_record.argtypes = [vp, i32, i32, vp]
     lib.spgg_strip_pair_counts.argtypes = [vp, i32, i32, vp, i32, i32, vp]
+    lib.spgg_block_fields.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.spgg_ipc_export.argtypes = [vp, vp]
     lib.spgg_ipc_attach.argtypes = [vp, i32, vp, i32, i32]
     lib.spgg_ring_export.argtypes = [vp, vp]

@@ -151,6 +151,9 @@ struct spgg_handle {
   unsigned long long *d_pair_cnt = nullptr;
   uint32_t *d_pair_tail = nullptr;
   size_t pair_cnt_n = 0, pair_tail_n = 0;
+  // spgg_block_fields (spgg_blocks.cuh): counts, sums and pieces of the largest call so far
+  void *d_blk = nullptr;
+  size_t blk_bytes = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -361,6 +364,7 @@ spgg_handle::~spgg_handle() {
   ccl_free(&ccl);
   ccl_strip_free(&ccl_strip);
   cudaFree(d_pair_cnt); cudaFree(d_pair_tail);
+  cudaFree(d_blk);
 }
 
 extern "C" void spgg_destroy(spgg_t *h) {
@@ -1647,6 +1651,44 @@ extern "C" int spgg_strip_pair_counts(spgg_t *h, int world, int rank, const void
   cudaError_t e = launch_pair_counts(pair_plane(h, 0), g.pitchW, g.rows, g.L, h->d_pair_tail, nW, max_d, h->d_pair_cnt, out);
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_strip_pair_counts: %s", cudaGetErrorString(e));
   h->launches += 2;
+  return SPGG_OK;
+}
+
+// ---------------------------------------------------------------- block fields
+// Counts and fp64 sums of R and Q over b x b blocks of one replica (include/spgg.h); the kernels live in
+// spgg_blocks.cu.  Reads the planes spgg_state_digest reads; touches neither the state nor any other result.
+extern "C" int spgg_block_fields(spgg_t *h, int rep, int b, int flags, int64_t *counts, double *sums) {
+  if (!h || !counts || (flags && !sums)) return fail(SPGG_E_INVALID, "spgg_block_fields: null argument");
+  if (rep < 0 || rep >= h->n_rep) return fail(SPGG_E_INVALID, "replica %d out of range", rep);
+  if (flags & ~(SPGG_BLOCK_R | SPGG_BLOCK_Q)) return fail(SPGG_E_INVALID, "spgg_block_fields: unknown flags 0x%x", flags);
+  const Geom &g = h->g;
+  if (b < 1 || b > g.L) return fail(SPGG_E_INVALID, "spgg_block_fields: b = %d outside [1, L = %d]", b, g.L);
+  const long long B = (g.L + b - 1) / b;
+  if (B * B > BLK_MAX_BLOCKS)
+    return fail(SPGG_E_INVALID, "spgg_block_fields: %lld x %lld blocks exceed 2^24 (b = %d, L = %d)", B, B, b, g.L);
+  int rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const bool want_r = flags & SPGG_BLOCK_R, want_q = flags & SPGG_BLOCK_Q;
+  const BlockGeom q = block_geom(g.L, g.row0, g.rows, b);
+  const size_t need = block_scratch_bytes(q, (want_r ? 1 : 0) + (want_q ? h->nq() : 0));
+  if (h->blk_bytes < need) {
+    cudaFree(h->d_blk);
+    h->d_blk = nullptr;
+    h->blk_bytes = 0;
+    CUDA_TRY(cudaMalloc(&h->d_blk, need));
+    h->blk_bytes = need;
+  }
+  const uint32_t *S = h->d_S[h->cur] + (size_t)rep * g.bits_stride + (size_t)GH * g.pitchW + WPAD;
+  const void *R = (const char *)h->d_R[h->cur] + ((size_t)rep * g.plane_stride + (size_t)GH * g.pitchB + CPAD) * h->elem_R();
+  const void *Q = (const char *)h->Qcur() + (size_t)rep * g.site_stride * h->nq() * h->elem_Q();
+  const double rq = h->rc_host[rep].rq;
+  const cudaError_t e = with_mode(h->mode, [&](auto md) {
+    return launch_block_fields<decltype(md)>(q, g.pitchW, g.pitchB, S, R, Q, rq, h->nq(), want_r, want_q, h->d_blk,
+                                             counts, sums);
+  });
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_block_fields: %s", cudaGetErrorString(e));
+  h->launches += flags ? 2 + (q.nrc * q.ncs > 1) : 1;
   return SPGG_OK;
 }
 

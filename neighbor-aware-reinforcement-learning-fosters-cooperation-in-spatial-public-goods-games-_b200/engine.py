@@ -77,6 +77,61 @@ def pair_correlation(counts, n_sites: int) -> np.ndarray:
     return (c[:, :, 0] / N - f * f) / (f - f * f)
 
 
+_BLOCK_FIELDS = {"R": L_.BLOCK_R, "Q": L_.BLOCK_Q}
+
+
+def block_flags(fields) -> int:
+    """``fields`` of the block-field methods (a name or a sequence of "R" and "Q") -> the flags of the C ABI."""
+    names = (fields,) if isinstance(fields, str) else tuple(fields)
+    flags = 0
+    for f in names:
+        if not isinstance(f, str) or f not in _BLOCK_FIELDS:
+            raise ValueError(f"fields must name 'R' and/or 'Q', got {fields!r}")
+        flags |= _BLOCK_FIELDS[f]
+    return flags
+
+
+def block_rows(L: int, b: int, row0: int = 0, rows: int | None = None) -> tuple[int, int]:
+    """(I0, nI): the block rows of side ``b`` that hold rows [row0, row0 + rows) of an L x L lattice."""
+    rows = L if rows is None else rows
+    I0 = row0 // b
+    return I0, (row0 + rows - 1) // b - I0 + 1
+
+
+def block_result(counts, sums, flags: int, q_shape) -> dict:
+    """The flat arrays of ``spgg_block_fields`` (counts (nI, B, 2) int64, sums (nI, B, 2, m) float64) -> the dict
+    of ``Engine.block_fields``."""
+    out = {"n": counts[:, :, 0], "n_C": counts[:, :, 1]}
+    ch = 0
+    if flags & L_.BLOCK_R:
+        out["R"] = sums[:, :, :, 0]
+        ch = 1
+    if flags & L_.BLOCK_Q:
+        out["Q"] = sums[:, :, :, ch:].reshape(sums.shape[:3] + tuple(q_shape))
+    return out
+
+
+def block_means(fields: dict) -> dict:
+    """Means per block from ``block_fields``: ``coop`` = n_C / n, and for each of "R" and "Q" that is present
+    the mean over all sites (``R``), over the cooperators (``R_C``) and over the defectors (``R_D``) of the
+    block, shapes (B, B) for R and (B, B) + the Q shape of ``get_state`` for Q.  NaN where a class is empty."""
+    n = np.asarray(fields["n"], np.float64)
+    nC = np.asarray(fields["n_C"], np.float64)
+    nD = n - nC
+    out = {"coop": nC / n}
+    with np.errstate(invalid="ignore", divide="ignore"):
+        for key in ("R", "Q"):
+            if key not in fields:
+                continue
+            s = np.asarray(fields[key], np.float64)
+            tail = (1,) * (s.ndim - 3)
+            sA, sC = s[:, :, 0], s[:, :, 1]
+            for suffix, tot, cnt in (("", sA, n), ("_C", sC, nC), ("_D", sA - sC, nD)):
+                c = cnt.reshape(cnt.shape + tail)
+                out[key + suffix] = np.where(c > 0, tot / np.where(c > 0, c, 1.0), np.nan)
+    return out
+
+
 class Engine:
     """``n`` independent lattices on one device.  ``param_list`` is one dict (or a
     sequence of dicts, one per replica) with the reference ctor's argument names."""
@@ -95,6 +150,7 @@ class Engine:
         self.n_replicas = n
         self.L = int(arr[0].L)
         self.rows = int(arr[0].rows)
+        self.row0 = int(arr[0].row0)
         self.precision = precision
         # Q values per site: 4, or the two tables of Double Q-learning ([site][table][s][a])
         self.nq = 8 if int(arr[0].algorithm) == L_.ALGO_DOUBLE_QLEARNING else 4
@@ -222,6 +278,28 @@ class Engine:
         out = np.zeros((2, max(int(max_d), 0) + 1, 2), np.int64)
         L_.check(self.lib.spgg_pair_counts(self._h, int(replica), int(max_d), out.ctypes.data))
         return out
+
+    # -- block fields (include/spgg.h: spgg_block_fields)
+    def block_fields(self, b: int, replica: int = 0, fields=("R", "Q")) -> dict:
+        """Counts and sums over the b x b blocks of the lattice (B = ceil(L/b) per side, anchored at site
+        (0, 0), the last block row and column ragged when b does not divide L), computed on the device:
+        ``"n"`` and ``"n_C"`` int64 (B, B), the sites and the cooperators of each block; for each field asked
+        for, ``"R"`` float64 (B, B, 2) and ``"Q"`` float64 (B, B, 2) + the Q shape of ``get_state``, the sums
+        over all sites ([..., 0, ...]) and over the cooperators ([..., 1, ...]).  ``fields=()`` reads only the
+        strategy bits.  Counts and int8-stored R are exact; fp32 / fp64 values are summed in fp64 in a fixed
+        order.  On a strip handle the leading axis runs over the block rows holding its rows, with the strip's
+        own contribution.  ``block_means`` turns the result into means."""
+        flags = block_flags(fields)
+        b, L = int(b), self.L
+        counts, sums = np.zeros(2, np.int64), np.zeros(1)
+        B = -(-L // b) if 1 <= b <= L else 0
+        if B and B * B <= 1 << 24:   # else the library rejects b before writing
+            I0, nI = block_rows(L, b, self.row0, self.rows)
+            m = (1 if flags & L_.BLOCK_R else 0) + (self.nq if flags & L_.BLOCK_Q else 0)
+            counts, sums = np.zeros((nI, B, 2), np.int64), np.zeros((nI, B, 2, m))
+        L_.check(self.lib.spgg_block_fields(self._h, int(replica), b, flags, counts.ctypes.data,
+                                            sums.ctypes.data if flags else None))
+        return block_result(counts, sums, flags, (2, 2) if self.nq == 4 else (2, 2, 2))
 
     def set_replay(self, u, b):
         """``u`` (n,rows,L) float64 and ``b`` (n,rows,L) 0/1: the reference's draw

@@ -55,6 +55,24 @@ def strip_rows(L: int, world: int, rank: int, align: int = 16) -> tuple[int, int
     return row0, rows
 
 
+def assemble_block_fields(L: int, b: int, world: int, parts) -> tuple[np.ndarray, np.ndarray]:
+    """The whole lattice's block fields from the strips' (``StripEngine.block_fields``): ``parts[k]`` is rank
+    k's (counts, sums), counts int64 (nI, B, 2) and sums float64 (nI, B, 2, m) over the block rows holding
+    its rows (``engine.block_rows``), possibly padded past nI.  The strips are added in rank order into
+    (B, B, 2) and (B, B, 2, m): integer channels exactly, float channels in an order fixed by the partition."""
+    from .engine import block_rows
+    B = -(-L // b)
+    m = parts[0][1].shape[-1]
+    counts = np.zeros((B, B, 2), np.int64)
+    sums = np.zeros((B, B, 2, m))
+    for k in range(world):
+        row0, rows = strip_rows(L, world, k)
+        I0, nI = block_rows(L, b, row0, rows)
+        counts[I0:I0 + nI] += parts[k][0][:nI]
+        sums[I0:I0 + nI] += parts[k][1][:nI]
+    return counts, sums
+
+
 def neighbours(world: int, rank: int) -> tuple[int, int]:
     """(up, down): ranks owning the rows just above (row0-1) and just below; periodic."""
     return (rank - 1) % world, (rank + 1) % world
@@ -367,6 +385,47 @@ class StripEngine:
             t = t.to(self.dev)
         self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM, group=self.group)
         return t.cpu().numpy()
+
+    # -- block fields (include/spgg.h: spgg_block_fields)
+    def block_fields(self, b: int, fields=("R", "Q")) -> dict:
+        """``Engine.block_fields`` of the WHOLE lattice (all ranks call this; every rank gets the same dict of
+        (B, B) arrays): each strip sums its own rows over the block rows they touch, the partials are
+        all-gathered (padded to the largest block-row count) and added in rank order
+        (``assemble_block_fields``)."""
+        from .engine import block_flags, block_result, block_rows
+        torch = self.torch
+        flags = block_flags(fields)
+        b = int(b)
+        self._settle()
+        part = self.eng.block_fields(b, fields=fields)
+        nq = self.eng.nq
+        m = (1 if flags & L_.BLOCK_R else 0) + (nq if flags & L_.BLOCK_Q else 0)
+        nI = part["n"].shape[0]
+        counts = np.stack([part["n"], part["n_C"]], axis=-1)
+        sums = np.zeros(counts.shape[:2] + (2, m))
+        if flags & L_.BLOCK_R:
+            sums[..., 0] = part["R"]
+        if flags & L_.BLOCK_Q:
+            sums[..., m - nq:] = part["Q"].reshape(sums.shape[:3] + (nq,))
+        if self.world > 1:
+            pad = max(block_rows(self.L, b, *strip_rows(self.L, self.world, r))[1] for r in range(self.world))
+            B, w = counts.shape[1], counts.shape[1] * 2 * (1 + m)
+            # counts and the bytes of the sums travel as one int64 tensor per rank
+            t = torch.zeros((pad, w), dtype=torch.int64)
+            t[:nI] = torch.from_numpy(np.concatenate([counts.reshape(nI, -1), sums.reshape(nI, -1).view(np.int64)], 1))
+            if self.host_staged:
+                got = [torch.empty_like(t) for _ in range(self.world)]
+                self.dist.all_gather(got, t, group=self.group)
+            else:
+                allp = torch.empty((self.world * pad, w), dtype=torch.int64, device=self.dev)
+                self.dist.all_gather_into_tensor(allp, t.to(self.dev), group=self.group)
+                got = list(allp.cpu().split(pad))
+            parts = []
+            for g in got:
+                a = g.numpy()
+                parts.append((a[:, :B * 2].reshape(pad, B, 2), a[:, B * 2:].copy().view(np.float64).reshape(pad, B, 2, m)))
+            counts, sums = assemble_block_fields(self.L, b, self.world, parts)
+        return block_result(counts, sums, flags, (2, 2) if nq == 4 else (2, 2, 2))
 
     # -- stepping
     def _stream(self):
