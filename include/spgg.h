@@ -273,6 +273,40 @@ int spgg_strip_pair_counts(spgg_t *h, int world, int rank, const void *dev_recor
 #define SPGG_BLOCK_Q 2
 int spgg_block_fields(spgg_t *h, int replica, int b, int flags, int64_t *counts, double *sums);
 
+/* Value distributions of replicas rep0 .. rep0 + n_rep - 1 on the device, in one launch per kernel
+ * for all of them.  Channels ch: with SPGG_HIST_R first R as spgg_get_state returns it (int8 units
+ * x quantum), with SPGG_HIST_Q then the nq Q entries in spgg_get_state's order (nq 4, or 8 for
+ * Double Q-learning: [table][state][action]); m = (flags & R) + (flags & Q ? nq : 0).  Classes k:
+ * 0 all sites, 1 the cooperators (S == 0); defectors are the difference.  r = replica - rep0.
+ * spgg_value_ranges: minmax[(((r*m + ch)*2 + k)*2) + {0: min, 1: max}], the exact extremes as
+ *   numbers (an empty class gives +inf / -inf; the sign of a zero extreme is unspecified).
+ *   NumPy's default range of a channel is (min, max) of k 0, widened by 0.5 each way when equal.
+ * spgg_histograms: np.histogram(x, bins=n_bins, range=(e[0], e[n_bins])) of every (r, ch, k), with
+ *   e = edges + (r*m + ch)*(n_bins + 1) the np.linspace edges of that range: uniform bins,
+ *   half-open but the last closed, values outside [e[0], e[n_bins]] not counted, the fp64 float
+ *   index (x - e[0]) * n_bins / (e[n_bins] - e[0]) corrected by one against the edges as
+ *   NumPy's uniform path does (no FMA contraction).  The counts are exact:
+ *     counts[((r*m + ch)*2 + k)*n_bins + bin], int64;  1 <= n_bins <= 1024;
+ *   counts and edges may be null when m == 0.
+ *   policy (may be null): policy[(r*2 + k)*2 + s], the sites of class k whose greedy action in
+ *   state s is C: Qbar[s, 0] >= Qbar[s, 1] (np.argmax's first maximum; C is action 0), Qbar = Q,
+ *   or (QA + QB) / 2 for Double Q-learning, in fp64 as NumPy evaluates it on spgg_get_state's
+ *   arrays.  Asking for policy reads Q even without SPGG_HIST_Q.
+ * Both see the state spgg_get_state would return (a pending chunk is finished first) and change
+ * neither the state, the iteration counter, the statistics rows, a cluster-labelling result nor
+ * the pair-count and block scratch.  A strip handle counts its own rows only, so the results of
+ * the strips add up to the lattice's (extremes by min / max).  SPGG_E_INVALID: a replica range
+ * outside [0, n_replicas), unknown flag bits, n_bins outside [1, 1024], null pointers, an edge
+ * row that is not finite, not non-decreasing, or has e[0] >= e[n_bins].  Cost: one streaming pass
+ * over the bit plane and the R and Q planes asked for, per call; device scratch of about
+ * 8*n_rep*(2*m*n_bins + m*(n_bins + 5) + 517) bytes, grown to the largest call and freed with
+ * the handle. */
+#define SPGG_HIST_R 1
+#define SPGG_HIST_Q 2
+int spgg_value_ranges(spgg_t *h, int rep0, int n_rep, int flags, double *minmax);
+int spgg_histograms(spgg_t *h, int rep0, int n_rep, int flags, int n_bins, const double *edges,
+                    int64_t *counts, int64_t *policy);
+
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox
  * keyed by `seed`; for lattices too large to stage through host memory. */

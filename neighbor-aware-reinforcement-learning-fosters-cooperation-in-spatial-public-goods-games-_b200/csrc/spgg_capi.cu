@@ -154,6 +154,9 @@ struct spgg_handle {
   // spgg_block_fields (spgg_blocks.cuh): counts, sums and pieces of the largest call so far
   void *d_blk = nullptr;
   size_t blk_bytes = 0;
+  // spgg_value_ranges / spgg_histograms (spgg_hist.cuh): counts, extremes, edges of the largest call so far
+  void *d_hist = nullptr;
+  size_t hist_bytes = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -365,6 +368,7 @@ spgg_handle::~spgg_handle() {
   ccl_strip_free(&ccl_strip);
   cudaFree(d_pair_cnt); cudaFree(d_pair_tail);
   cudaFree(d_blk);
+  cudaFree(d_hist);
 }
 
 extern "C" void spgg_destroy(spgg_t *h) {
@@ -1689,6 +1693,88 @@ extern "C" int spgg_block_fields(spgg_t *h, int rep, int b, int flags, int64_t *
   });
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_block_fields: %s", cudaGetErrorString(e));
   h->launches += flags ? 2 + (q.nrc * q.ncs > 1) : 1;
+  return SPGG_OK;
+}
+
+// ---------------------------------------------------------------- value distributions
+// Extremes, np.histogram counts and greedy-policy counts of replicas rep0 .. rep0 + n_rep - 1 (include/spgg.h); the
+// kernels live in spgg_hist.cu.  Reads the planes spgg_block_fields reads; touches neither the state nor any other
+// result.
+static int hist_args(spgg_t *h, const char *fn, int rep0, int n_rep, int flags) {
+  if (rep0 < 0 || n_rep < 1 || rep0 > h->n_rep - n_rep)
+    return fail(SPGG_E_INVALID, "%s: replicas [%d, %d + %d) outside [0, %d)", fn, rep0, rep0, n_rep, h->n_rep);
+  if (flags & ~(SPGG_HIST_R | SPGG_HIST_Q)) return fail(SPGG_E_INVALID, "%s: unknown flags 0x%x", fn, flags);
+  return SPGG_OK;
+}
+
+// the planes of replica rep0 and the int8 quanta of the replicas; grows the scratch to `need` bytes
+static int hist_prepare(spgg_t *h, int rep0, int n_rep, size_t need, HistPlanes *p, std::vector<double> *rq) {
+  int rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (h->hist_bytes < need) {
+    cudaFree(h->d_hist);
+    h->d_hist = nullptr;
+    h->hist_bytes = 0;
+    CUDA_TRY(cudaMalloc(&h->d_hist, need));
+    h->hist_bytes = need;
+  }
+  const Geom &g = h->g;
+  p->L = g.L; p->rows = g.rows; p->pitchW = g.pitchW; p->pitchB = g.pitchB; p->nq = h->nq(); p->n_rep = n_rep;
+  p->S = h->d_S[h->cur] + (size_t)rep0 * g.bits_stride + (size_t)GH * g.pitchW + WPAD;
+  p->R = (const char *)h->d_R[h->cur] + ((size_t)rep0 * g.plane_stride + (size_t)GH * g.pitchB + CPAD) * h->elem_R();
+  p->Q = (const char *)h->Qcur() + (size_t)rep0 * g.site_stride * h->nq() * h->elem_Q();
+  p->bits_stride = g.bits_stride; p->plane_stride = g.plane_stride; p->q_stride = g.site_stride * h->nq();
+  rq->resize(n_rep);
+  for (int r = 0; r < n_rep; ++r) (*rq)[r] = h->rc_host[rep0 + r].rq;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_value_ranges(spgg_t *h, int rep0, int n_rep, int flags, double *minmax) {
+  if (!h || !minmax) return fail(SPGG_E_INVALID, "spgg_value_ranges: null argument");
+  int rcode = hist_args(h, "spgg_value_ranges", rep0, n_rep, flags);
+  if (rcode) return rcode;
+  const bool want_r = flags & SPGG_HIST_R, want_q = flags & SPGG_HIST_Q;
+  const int m = (want_r ? 1 : 0) + (want_q ? h->nq() : 0);
+  HistPlanes p;
+  std::vector<double> rq;
+  rcode = hist_prepare(h, rep0, n_rep, hist_scratch_bytes(n_rep, m, 1), &p, &rq);
+  if (rcode) return rcode;
+  const cudaError_t e = with_mode(h->mode, [&](auto md) {
+    return launch_value_ranges<decltype(md)>(p, want_r, want_q, rq.data(), h->d_hist, minmax);
+  });
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_value_ranges: %s", cudaGetErrorString(e));
+  h->launches += m > 0;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_histograms(spgg_t *h, int rep0, int n_rep, int flags, int n_bins, const double *edges,
+                               int64_t *counts, int64_t *policy) {
+  if (!h) return fail(SPGG_E_INVALID, "spgg_histograms: null argument");
+  int rcode = hist_args(h, "spgg_histograms", rep0, n_rep, flags);
+  if (rcode) return rcode;
+  if (n_bins < 1 || n_bins > HIST_MAX_BINS)
+    return fail(SPGG_E_INVALID, "spgg_histograms: n_bins = %d outside [1, %d]", n_bins, HIST_MAX_BINS);
+  const bool want_r = flags & SPGG_HIST_R, want_q = flags & SPGG_HIST_Q;
+  const int m = (want_r ? 1 : 0) + (want_q ? h->nq() : 0);
+  if (m > 0 && (!edges || !counts)) return fail(SPGG_E_INVALID, "spgg_histograms: null argument");
+  for (long long row = 0; row < (long long)n_rep * m; ++row) {
+    const double *e = edges + row * (n_bins + 1);
+    bool ok = std::isfinite(e[0]) && e[0] < e[n_bins];
+    for (int i = 1; ok && i <= n_bins; ++i) ok = std::isfinite(e[i]) && e[i] >= e[i - 1];
+    if (!ok)
+      return fail(SPGG_E_INVALID, "spgg_histograms: edge row %lld is not finite and increasing from edges[0] to "
+                  "edges[n_bins]", row);
+  }
+  HistPlanes p;
+  std::vector<double> rq;
+  rcode = hist_prepare(h, rep0, n_rep, hist_scratch_bytes(n_rep, m, n_bins), &p, &rq);
+  if (rcode) return rcode;
+  const cudaError_t e = with_mode(h->mode, [&](auto md) {
+    return launch_histograms<decltype(md)>(p, want_r, want_q, n_bins, edges, rq.data(), h->d_hist, counts, policy);
+  });
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_histograms: %s", cudaGetErrorString(e));
+  h->launches += (m > 0 || policy) + (want_r && h->mode == MODE_F32_I8);
   return SPGG_OK;
 }
 

@@ -132,6 +132,98 @@ def block_means(fields: dict) -> dict:
     return out
 
 
+HIST_MAX_BINS = 1024
+
+
+def hist_edges(lo, hi, bins: int) -> np.ndarray:
+    """The edges of ``np.histogram(x, bins=bins, range=(lo, hi))``: (lo, hi) checked as NumPy checks a range,
+    widened by 0.5 each way when lo == hi, then ``np.linspace``."""
+    lo, hi = float(lo), float(hi)
+    if not (np.isfinite(lo) and np.isfinite(hi)):
+        raise ValueError(f"histogram range ({lo}, {hi}) is not finite")
+    if lo > hi:
+        raise ValueError(f"histogram range ({lo}, {hi}): max must be larger than min")
+    if lo == hi:
+        lo, hi = lo - 0.5, hi + 0.5
+    return np.linspace(lo, hi, bins + 1, endpoint=True, dtype=np.float64)
+
+
+def hist_replicas(replica, n_replicas: int) -> tuple[int, int]:
+    """``replica`` of the histogram methods (an int, or a ``range`` of consecutive replicas) -> (rep0, n)."""
+    if isinstance(replica, range):
+        if replica.step != 1 or len(replica) == 0:
+            raise ValueError(f"replica must be a non-empty range of consecutive replicas, got {replica!r}")
+        rep0, n = replica.start, len(replica)
+    elif isinstance(replica, (int, np.integer)) and not isinstance(replica, bool):
+        rep0, n = int(replica), 1
+    else:
+        raise ValueError(f"replica must be an int or a range, got {replica!r}")
+    if rep0 < 0 or rep0 + n > n_replicas:
+        raise ValueError(f"replicas {rep0} .. {rep0 + n - 1} outside [0, {n_replicas})")
+    return rep0, n
+
+
+def hist_channels(flags: int, nq: int) -> list[str]:
+    """The channels of ``spgg_histograms`` for ``flags``, by field: "R" once, then "Q" nq times."""
+    return (["R"] if flags & L_.HIST_R else []) + (["Q"] * nq if flags & L_.HIST_Q else [])
+
+
+def hist_edge_rows(bins: int, chans: Sequence[str], minmax, ranges) -> np.ndarray:
+    """Edges (n, m, bins + 1) of the channels ``chans``: from ``ranges[field]`` where given, else NumPy's default
+    range per replica and channel from ``minmax`` (n, m, 2), the (min, max) over all sites of
+    ``spgg_value_ranges`` (not read for a field with a range)."""
+    ranges = {} if ranges is None else ranges
+    n = minmax.shape[0]
+    edges = np.empty((n, len(chans), bins + 1))
+    for ch, f in enumerate(chans):
+        for r in range(n):
+            lo, hi = ranges[f] if f in ranges else minmax[r, ch]
+            edges[r, ch] = hist_edges(lo, hi, bins)
+    return edges
+
+
+def hist_result(counts, policy, edges, chans, q_shape, batched: bool, replica) -> dict:
+    """The flat arrays of ``spgg_histograms`` (counts (n, m, 2, bins), policy (n, 2, 2) or None, edges
+    (n, m, bins + 1)) -> the dict of ``Engine.histograms``."""
+    n, bins = counts.shape[0], counts.shape[-1]
+    out = {"replica": replica}
+    ch = 0
+    if "R" in chans:
+        out["R"], out["R_edges"] = counts[:, 0], edges[:, 0]
+        ch = 1
+    if "Q" in chans:
+        out["Q"] = np.moveaxis(counts[:, ch:], 2, 1).reshape((n, 2) + tuple(q_shape) + (bins,))
+        out["Q_edges"] = edges[:, ch:].reshape((n,) + tuple(q_shape) + (bins + 1,))
+    if policy is not None:
+        out["policy"] = policy
+    if not batched:
+        out = {k: (v[0] if isinstance(v, np.ndarray) else v) for k, v in out.items()}
+    return out
+
+
+def class_histograms(h: dict) -> dict:
+    """The result of ``histograms`` with the defectors added: for "R", "Q" and "policy" where present the class
+    axis holds [all, cooperators, defectors] (defectors = all - cooperators), and "R_density" / "Q_density" are
+    ``np.histogram(..., density=True)`` of each class (NaN where a class has no count in range)."""
+    batched = isinstance(h["replica"], range)
+    ax = 1 if batched else 0
+    out = dict(h)
+    for key in ("R", "Q", "policy"):
+        if key not in h:
+            continue
+        c = np.asarray(h[key])
+        a, cc = np.take(c, 0, axis=ax), np.take(c, 1, axis=ax)
+        out[key] = np.stack([a, cc, a - cc], axis=ax)
+        if key == "policy":
+            continue
+        widths = np.diff(h[key + "_edges"], axis=-1)
+        widths = np.expand_dims(widths, ax)
+        tot = out[key].sum(axis=-1, keepdims=True)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            out[key + "_density"] = np.where(tot > 0, out[key] / np.where(tot > 0, tot, 1) / widths, np.nan)
+    return out
+
+
 class Engine:
     """``n`` independent lattices on one device.  ``param_list`` is one dict (or a
     sequence of dicts, one per replica) with the reference ctor's argument names."""
@@ -300,6 +392,69 @@ class Engine:
         L_.check(self.lib.spgg_block_fields(self._h, int(replica), b, flags, counts.ctypes.data,
                                             sums.ctypes.data if flags else None))
         return block_result(counts, sums, flags, (2, 2) if self.nq == 4 else (2, 2, 2))
+
+    # -- value distributions (include/spgg.h: spgg_value_ranges / spgg_histograms)
+    def _value_ranges(self, rep0: int, n: int, flags: int) -> np.ndarray:
+        m = len(hist_channels(flags, self.nq))
+        mm = np.zeros((n, m, 2, 2))
+        L_.check(self.lib.spgg_value_ranges(self._h, rep0, n, flags, mm.ctypes.data))
+        return mm
+
+    def value_ranges(self, replica=0, fields=("R", "Q")) -> dict:
+        """Exact (min, max) of every field over all sites and over the cooperators, computed on the device:
+        ``"R"`` float64 (2, 2) [class, min/max] and ``"Q"`` float64 (2,) + the Q shape of ``get_state`` + (2,),
+        class 0 all sites and 1 the cooperators (+inf / -inf for an empty class).  ``replica`` is an int or a
+        ``range`` of consecutive replicas, which adds a leading replica axis."""
+        flags = block_flags(fields)   # SPGG_HIST_R / SPGG_HIST_Q are the bits of SPGG_BLOCK_R / SPGG_BLOCK_Q
+        rep0, n = hist_replicas(replica, self.n_replicas)
+        mm = self._value_ranges(rep0, n, flags)
+        out, ch = {}, 0
+        if flags & L_.HIST_R:
+            out["R"] = mm[:, 0]
+            ch = 1
+        if flags & L_.HIST_Q:
+            qs = (2, 2) if self.nq == 4 else (2, 2, 2)
+            out["Q"] = np.moveaxis(mm[:, ch:], 2, 1).reshape((n, 2) + qs + (2,))
+        return out if isinstance(replica, range) else {k: v[0] for k, v in out.items()}
+
+    def _histograms(self, rep0: int, n: int, flags: int, bins: int, edges, policy: bool):
+        """``spgg_histograms`` of replicas rep0 .. rep0+n-1 with edges (n, m, bins + 1) -> (counts (n, m, 2,
+        bins) int64, policy (n, 2, 2) int64 or None)."""
+        m = len(hist_channels(flags, self.nq))
+        edges = np.ascontiguousarray(edges, np.float64)
+        counts = np.zeros((n, m, 2, bins), np.int64)
+        pol = np.zeros((n, 2, 2), np.int64) if policy else None
+        L_.check(self.lib.spgg_histograms(self._h, rep0, n, flags, bins, edges.ctypes.data if m else None,
+                                          counts.ctypes.data if m else None,
+                                          pol.ctypes.data if policy else None))
+        return counts, pol
+
+    def histograms(self, bins: int, replica=0, fields=("R", "Q"), ranges=None, policy: bool = True) -> dict:
+        """``np.histogram(x, bins=bins, range=...)`` of R and of every Q entry, over all sites and over the
+        cooperators, and the greedy-policy counts, computed on the device with exact integer counts.
+        ``replica``: an int, or a ``range`` of consecutive replicas (a leading replica axis on every array).
+        ``ranges``: {"R": (lo, hi), "Q": (lo, hi)}; a field without one gets NumPy's default range, (min, max)
+        over all sites of its replica and channel (``value_ranges``).  Returns ``"R"`` int64 (2, bins)
+        [all, C] and ``"R_edges"`` (bins + 1,); ``"Q"`` int64 (2,) + the Q shape of ``get_state`` + (bins,)
+        and ``"Q_edges"`` (Q shape + (bins + 1,)); with ``policy``, ``"policy"`` int64 (2, 2) [class, state],
+        the sites whose greedy action in state s is C (argmax of Q, or of (QA + QB) / 2 for Double
+        Q-learning); and ``"replica"``.  ``class_histograms`` adds the defectors and the densities."""
+        bins = int(bins)
+        if not 1 <= bins <= HIST_MAX_BINS:
+            raise ValueError(f"bins must be in [1, {HIST_MAX_BINS}], got {bins}")
+        flags = block_flags(fields)
+        rep0, n = hist_replicas(replica, self.n_replicas)
+        chans = hist_channels(flags, self.nq)
+        ranges = {} if ranges is None else dict(ranges)
+        for f in ranges:
+            if f not in ("R", "Q"):
+                raise ValueError(f"ranges may name 'R' and 'Q', got {f!r}")
+        need = any(f not in ranges for f in chans)
+        mm = self._value_ranges(rep0, n, flags)[:, :, :1] if need else np.zeros((n, len(chans), 1, 2))
+        edges = hist_edge_rows(bins, chans, mm[:, :, 0], ranges)
+        counts, pol = self._histograms(rep0, n, flags, bins, edges, policy)
+        return hist_result(counts, pol, edges, chans, (2, 2) if self.nq == 4 else (2, 2, 2),
+                           isinstance(replica, range), replica)
 
     def set_replay(self, u, b):
         """``u`` (n,rows,L) float64 and ``b`` (n,rows,L) 0/1: the reference's draw

@@ -427,6 +427,46 @@ class StripEngine:
             counts, sums = assemble_block_fields(self.L, b, self.world, parts)
         return block_result(counts, sums, flags, (2, 2) if nq == 4 else (2, 2, 2))
 
+    # -- value distributions (include/spgg.h: spgg_value_ranges / spgg_histograms)
+    def _all_reduce(self, a: np.ndarray, op) -> np.ndarray:
+        if self.world == 1:
+            return a
+        t = self.torch.from_numpy(np.ascontiguousarray(a))
+        if not self.host_staged:
+            t = t.to(self.dev)
+        self.dist.all_reduce(t, op=op, group=self.group)
+        return t.cpu().numpy()
+
+    def histograms(self, bins: int, fields=("R", "Q"), ranges=None, policy: bool = True) -> dict:
+        """``Engine.histograms`` of the WHOLE lattice (all ranks call this; every rank gets the same dict): the
+        default ranges are the min / max of the strips' ``value_ranges``, reduced over the ranks, so every rank
+        builds the same edges; each strip counts its own rows and the int64 counts are summed over the ranks
+        (exact, so the order of the ranks does not matter)."""
+        from .engine import HIST_MAX_BINS, block_flags, hist_channels, hist_edge_rows, hist_result
+        bins = int(bins)
+        if not 1 <= bins <= HIST_MAX_BINS:
+            raise ValueError(f"bins must be in [1, {HIST_MAX_BINS}], got {bins}")
+        flags = block_flags(fields)
+        eng = self.eng
+        chans = hist_channels(flags, eng.nq)
+        ranges = {} if ranges is None else dict(ranges)
+        for f in ranges:
+            if f not in ("R", "Q"):
+                raise ValueError(f"ranges may name 'R' and 'Q', got {f!r}")
+        self._settle()
+        mm = np.zeros((1, len(chans), 2))
+        if any(f not in ranges for f in chans):
+            local = eng._value_ranges(0, 1, flags)[:, :, 0]   # (1, m, 2) over the strip's sites
+            mm[..., 0] = self._all_reduce(local[..., 0].copy(), self.dist.ReduceOp.MIN)
+            mm[..., 1] = self._all_reduce(local[..., 1].copy(), self.dist.ReduceOp.MAX)
+        edges = hist_edge_rows(bins, chans, mm, ranges)
+        counts, pol = eng._histograms(0, 1, flags, bins, edges, policy)
+        if chans:
+            counts = self._all_reduce(counts, self.dist.ReduceOp.SUM)
+        if policy:
+            pol = self._all_reduce(pol, self.dist.ReduceOp.SUM)
+        return hist_result(counts, pol, edges, chans, (2, 2) if eng.nq == 4 else (2, 2, 2), False, 0)
+
     # -- stepping
     def _stream(self):
         return C.c_void_p(self.torch.cuda.current_stream().cuda_stream)
