@@ -307,6 +307,57 @@ int spgg_value_ranges(spgg_t *h, int rep0, int n_rep, int flags, double *minmax)
 int spgg_histograms(spgg_t *h, int rep0, int n_rep, int flags, int n_bins, const double *edges,
                     int64_t *counts, int64_t *policy);
 
+/* State overlaps on the device: a snapshot of replicas kept on the handle, and exact measures of
+ * what changed since.
+ * spgg_snapshot copies the current state of replicas rep0 .. rep0 + n_rep - 1 (the state
+ *   spgg_get_state would return; a pending chunk is finished first) into slot `slot` in
+ *   [0, SPGG_MAX_SNAPSHOTS): always the strategy bit plane, R with SPGG_SNAP_R, Q with
+ *   SPGG_SNAP_Q.  The copy is made on the device (device-to-device copies; the call returns when
+ *   it is done) in the handle's own plane layout.  The slot records the iteration counter, rep0,
+ *   n_rep, flags and each replica's int8 R quantum.  Snapshotting into an occupied slot replaces
+ *   it (its memory is reused when the size matches).  A slot is a copy: it survives spgg_step,
+ *   spgg_set_state, spgg_init_random, spgg_set_progress and spgg_strip_rewind, and is freed by
+ *   spgg_snapshot_free (a no-op on an empty slot) or spgg_destroy.  Memory per slot: n_rep x
+ *   (bit plane + R plane with SPGG_SNAP_R + the nq Q entries with SPGG_SNAP_Q) of the handle's
+ *   layout, ghost rows and columns included: about 17.1 B per site with fp32 Q and int8 R (18.4 GB
+ *   at L = 32768), about 40 B per site in fp64.  If the allocation fails the call returns
+ *   SPGG_E_CUDA, the slot is empty and the handle stays usable.
+ * spgg_snapshot_info: the slot's iteration, rep0, n_rep and flags (each output may be null).
+ * spgg_overlap compares the current state of replica rep0 + r with replica r of the slot, r <
+ *   n_rep; n_rep must equal the slot's, rep0 may differ from it (snapshot replica a, then overlap
+ *   replica b of the same handle).  flags must be a subset of the slot's.  Values are compared as
+ *   spgg_get_state returns them, each side with its own int8 quantum.  Channels ch: with
+ *   SPGG_SNAP_R first R, with SPGG_SNAP_Q then the nq Q entries in spgg_get_state's order, as in
+ *   spgg_histograms; m = (flags & R) + (flags & Q ? nq : 0).
+ *     counts[(r*2 + a)*2 + b], int64: the sites with strategy a in the snapshot and b now (0 = C,
+ *       1 = D); always written;
+ *     changed[r*m + ch], int64: np.count_nonzero(now != then) (numeric: +0.0 against -0.0 is
+ *       unchanged);
+ *     diffs[(r*m + ch)*3 + k], float64, d = now - then in fp64: k 0 max |d| (exact), k 1 sum |d|,
+ *       k 2 sum d^2 (no FMA contraction).
+ *   Both sums are taken in an order fixed by (L, rows) alone, without floating-point atomics: the
+ *   same pair of states gives bit-identical sums whichever kernel path, chunking or batch produced
+ *   them; a sum of n terms is within (n-1) 2^-53 sum |term| of the exact one, and exact for
+ *   int8-stored R of equal quanta.  changed and diffs may be null when m == 0.
+ * Neither call changes the state, the iteration counter, the statistics rows, a cluster-labelling
+ * result nor the pair-count, block or histogram scratch.  A strip handle snapshots and compares
+ * its own rows only, so the results of the strips add up to the lattice's (max |d| by max).
+ * SPGG_E_INVALID: a slot outside [0, SPGG_MAX_SNAPSHOTS), a replica range outside [0,
+ * n_replicas), n_rep other than the slot's, unknown flag bits or flags the slot does not hold, null
+ * counts, null changed or diffs with m > 0; outputs are untouched on every error.  SPGG_E_STATE:
+ * spgg_overlap or spgg_snapshot_info on an empty slot.  Cost: the snapshot reads and writes the
+ * planes once; the overlap is one streaming pass over both copies and a small fold launch, with
+ * device scratch of 8*n_rep*(6 + 4m + 2m*T) bytes (T <= 4096 row tiles) grown to the largest call
+ * and freed with the handle. */
+#define SPGG_MAX_SNAPSHOTS 8
+#define SPGG_SNAP_R 1        /* same bits as SPGG_BLOCK_R / SPGG_HIST_R */
+#define SPGG_SNAP_Q 2
+int spgg_snapshot(spgg_t *h, int slot, int rep0, int n_rep, int flags);
+int spgg_snapshot_info(spgg_t *h, int slot, int64_t *iteration, int *rep0, int *n_rep, int *flags);
+int spgg_snapshot_free(spgg_t *h, int slot);
+int spgg_overlap(spgg_t *h, int slot, int rep0, int n_rep, int flags,
+                 int64_t *counts, int64_t *changed, double *diffs);
+
 /* Same distributions as the reference ctor (Q ~ U(-0.01,0.01) spgg.py:121, R = 0
  * spgg.py:129, S ~ Bernoulli(1/2) spgg.py:162) generated on the device from Philox
  * keyed by `seed`; for lattices too large to stage through host memory. */

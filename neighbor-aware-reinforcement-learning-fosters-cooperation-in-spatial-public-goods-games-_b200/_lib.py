@@ -31,6 +31,8 @@ E_INVALID, E_CUDA, E_STATE, E_UNSUPPORTED = -1, -2, -3, -4
 CLUSTER_PERIODIC = 1
 BLOCK_R, BLOCK_Q = 1, 2
 HIST_R, HIST_Q = 1, 2
+MAX_SNAPSHOTS = 8
+SNAP_R, SNAP_Q = 1, 2
 
 
 class Params(C.Structure):
@@ -69,6 +71,7 @@ EXPORTS = (
     "spgg_strip_cluster_record_bytes", "spgg_strip_clusters", "spgg_strip_clusters_resolve",
     "spgg_pair_counts", "spgg_strip_pair_record_bytes", "spgg_strip_pair_record", "spgg_strip_pair_counts",
     "spgg_block_fields", "spgg_value_ranges", "spgg_histograms",
+    "spgg_snapshot", "spgg_snapshot_info", "spgg_snapshot_free", "spgg_overlap",
 )
 
 _lib = None
@@ -126,6 +129,10 @@ def load():
     lib.spgg_block_fields.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.spgg_value_ranges.argtypes = [vp, i32, i32, i32, vp]
     lib.spgg_histograms.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp]
+    lib.spgg_snapshot.argtypes = [vp, i32, i32, i32, i32]
+    lib.spgg_snapshot_info.argtypes = [vp, i32, vp, vp, vp, vp]
+    lib.spgg_snapshot_free.argtypes = [vp, i32]
+    lib.spgg_overlap.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp]
     lib.spgg_ipc_export.argtypes = [vp, vp]
     lib.spgg_ipc_attach.argtypes = [vp, i32, vp, i32, i32]
     lib.spgg_ring_export.argtypes = [vp, vp]

@@ -157,6 +157,19 @@ struct spgg_handle {
   // spgg_value_ranges / spgg_histograms (spgg_hist.cuh): counts, extremes, edges of the largest call so far
   void *d_hist = nullptr;
   size_t hist_bytes = 0;
+  // spgg_snapshot: copies of replica states in the handle's plane layout (snap_layout), kept until freed
+  struct Snapshot {
+    void *mem = nullptr;
+    size_t bytes = 0;
+    bool full = false;
+    long long iter = 0;
+    int rep0 = 0, n_rep = 0, flags = 0;
+    std::vector<double> rq;   // int8 quantum of each replica at snapshot time
+  };
+  Snapshot snaps[SPGG_MAX_SNAPSHOTS];
+  // spgg_overlap (spgg_overlap.cuh): counts, maxima, sums and tile partials of the largest call so far
+  void *d_ov = nullptr;
+  size_t ov_bytes = 0;
   size_t elem_code() const { return mode == MODE_F64 ? 4 : 1; }
   size_t elem_R() const { return mode == MODE_F64 ? 8 : (mode == MODE_F32_F ? 4 : 1); }
   size_t elem_Q() const { return mode == MODE_F64 ? 8 : 4; }
@@ -369,6 +382,8 @@ spgg_handle::~spgg_handle() {
   cudaFree(d_pair_cnt); cudaFree(d_pair_tail);
   cudaFree(d_blk);
   cudaFree(d_hist);
+  for (Snapshot &sn : snaps) cudaFree(sn.mem);
+  cudaFree(d_ov);
 }
 
 extern "C" void spgg_destroy(spgg_t *h) {
@@ -1775,6 +1790,155 @@ extern "C" int spgg_histograms(spgg_t *h, int rep0, int n_rep, int flags, int n_
   });
   if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_histograms: %s", cudaGetErrorString(e));
   h->launches += (m > 0 || policy) + (want_r && h->mode == MODE_F32_I8);
+  return SPGG_OK;
+}
+
+// ---------------------------------------------------------------- state overlaps
+// Snapshots of replica states kept on the handle, and what changed since (include/spgg.h); the kernels live in
+// spgg_overlap.cu.  Reads the planes spgg_histograms reads; touches neither the state nor any other result.
+static int snap_args(spgg_t *h, const char *fn, int slot, int rep0, int n_rep, int flags) {
+  if (slot < 0 || slot >= SPGG_MAX_SNAPSHOTS)
+    return fail(SPGG_E_INVALID, "%s: slot %d outside [0, %d)", fn, slot, SPGG_MAX_SNAPSHOTS);
+  if (rep0 < 0 || n_rep < 1 || rep0 > h->n_rep - n_rep)
+    return fail(SPGG_E_INVALID, "%s: replicas [%d, %d + %d) outside [0, %d)", fn, rep0, rep0, n_rep, h->n_rep);
+  if (flags & ~(SPGG_SNAP_R | SPGG_SNAP_Q)) return fail(SPGG_E_INVALID, "%s: unknown flags 0x%x", fn, flags);
+  return SPGG_OK;
+}
+
+// Byte offsets of a slot's planes for n_rep replicas: the bit plane at 0, R at off[1] (SPGG_SNAP_R), Q at off[2]
+// (SPGG_SNAP_Q), each a whole replica range of the live buffer; returns the slot's size
+static size_t snap_layout(const spgg_handle *h, int n_rep, int flags, size_t off[3]) {
+  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
+  const Geom &g = h->g;
+  off[0] = 0;
+  off[1] = up((size_t)n_rep * g.bits_stride * 4);
+  off[2] = off[1] + ((flags & SPGG_SNAP_R) ? up((size_t)n_rep * g.plane_stride * h->elem_R()) : 0);
+  return off[2] + ((flags & SPGG_SNAP_Q) ? up((size_t)n_rep * g.site_stride * h->nq() * h->elem_Q()) : 0);
+}
+
+extern "C" int spgg_snapshot(spgg_t *h, int slot, int rep0, int n_rep, int flags) {
+  if (!h) return fail(SPGG_E_INVALID, "spgg_snapshot: null argument");
+  int rcode = snap_args(h, "spgg_snapshot", slot, rep0, n_rep, flags);
+  if (rcode) return rcode;
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  spgg_handle::Snapshot &s = h->snaps[slot];
+  size_t off[3];
+  const size_t need = snap_layout(h, n_rep, flags, off);
+  s.full = false;
+  if (s.bytes != need) {
+    cudaFree(s.mem);
+    s.mem = nullptr;
+    s.bytes = 0;
+    const cudaError_t e = cudaMalloc(&s.mem, need);
+    if (e != cudaSuccess) {
+      (void)cudaGetLastError();
+      s.mem = nullptr;
+      return fail(SPGG_E_CUDA, "spgg_snapshot: %zu bytes for slot %d: %s", need, slot, cudaGetErrorString(e));
+    }
+    s.bytes = need;
+  }
+  const Geom &g = h->g;
+  char *mem = (char *)s.mem;
+  CUDA_TRY(cudaMemcpyAsync(mem, h->d_S[h->cur] + (size_t)rep0 * g.bits_stride, (size_t)n_rep * g.bits_stride * 4,
+                           cudaMemcpyDeviceToDevice, 0));
+  if (flags & SPGG_SNAP_R) {
+    const size_t pb = (size_t)g.plane_stride * h->elem_R();
+    CUDA_TRY(cudaMemcpyAsync(mem + off[1], (const char *)h->d_R[h->cur] + (size_t)rep0 * pb, (size_t)n_rep * pb,
+                             cudaMemcpyDeviceToDevice, 0));
+  }
+  if (flags & SPGG_SNAP_Q) {
+    const size_t qb = (size_t)g.site_stride * h->nq() * h->elem_Q();
+    CUDA_TRY(cudaMemcpyAsync(mem + off[2], (const char *)h->Qcur() + (size_t)rep0 * qb, (size_t)n_rep * qb,
+                             cudaMemcpyDeviceToDevice, 0));
+  }
+  // a step on another (non-blocking) stream must not overwrite the planes while they are being copied
+  CUDA_TRY(cudaStreamSynchronize(0));
+  s.iter = h->iter;
+  s.rep0 = rep0;
+  s.n_rep = n_rep;
+  s.flags = flags;
+  s.rq.resize(n_rep);
+  for (int r = 0; r < n_rep; ++r) s.rq[r] = h->rc_host[rep0 + r].rq;
+  s.full = true;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_snapshot_info(spgg_t *h, int slot, int64_t *iteration, int *rep0, int *n_rep, int *flags) {
+  if (!h) return fail(SPGG_E_INVALID, "spgg_snapshot_info: null argument");
+  if (slot < 0 || slot >= SPGG_MAX_SNAPSHOTS)
+    return fail(SPGG_E_INVALID, "spgg_snapshot_info: slot %d outside [0, %d)", slot, SPGG_MAX_SNAPSHOTS);
+  const spgg_handle::Snapshot &s = h->snaps[slot];
+  if (!s.full) return fail(SPGG_E_STATE, "spgg_snapshot_info: slot %d holds no snapshot", slot);
+  if (iteration) *iteration = s.iter;
+  if (rep0) *rep0 = s.rep0;
+  if (n_rep) *n_rep = s.n_rep;
+  if (flags) *flags = s.flags;
+  return SPGG_OK;
+}
+
+extern "C" int spgg_snapshot_free(spgg_t *h, int slot) {
+  if (!h) return fail(SPGG_E_INVALID, "spgg_snapshot_free: null argument");
+  if (slot < 0 || slot >= SPGG_MAX_SNAPSHOTS)
+    return fail(SPGG_E_INVALID, "spgg_snapshot_free: slot %d outside [0, %d)", slot, SPGG_MAX_SNAPSHOTS);
+  spgg_handle::Snapshot &s = h->snaps[slot];
+  if (!s.mem) return SPGG_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaFree(s.mem);
+  s = spgg_handle::Snapshot();
+  return SPGG_OK;
+}
+
+extern "C" int spgg_overlap(spgg_t *h, int slot, int rep0, int n_rep, int flags, int64_t *counts, int64_t *changed,
+                            double *diffs) {
+  if (!h || !counts) return fail(SPGG_E_INVALID, "spgg_overlap: null argument");
+  int rcode = snap_args(h, "spgg_overlap", slot, rep0, n_rep, flags);
+  if (rcode) return rcode;
+  const bool want_r = flags & SPGG_SNAP_R, want_q = flags & SPGG_SNAP_Q;
+  const int m = (want_r ? 1 : 0) + (want_q ? h->nq() : 0);
+  if (m > 0 && (!changed || !diffs)) return fail(SPGG_E_INVALID, "spgg_overlap: null argument");
+  const spgg_handle::Snapshot &s = h->snaps[slot];
+  if (!s.full) return fail(SPGG_E_STATE, "spgg_overlap: slot %d holds no snapshot", slot);
+  if (n_rep != s.n_rep)
+    return fail(SPGG_E_INVALID, "spgg_overlap: n_rep = %d, slot %d holds %d replicas", n_rep, slot, s.n_rep);
+  if (flags & ~s.flags)
+    return fail(SPGG_E_INVALID, "spgg_overlap: flags 0x%x, slot %d holds 0x%x", flags, slot, s.flags);
+  rcode = finish_pending(h);
+  if (rcode) return rcode;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const Geom &g = h->g;
+  const size_t need = overlap_scratch_bytes(g.L, g.rows, n_rep, m);
+  if (h->ov_bytes < need) {
+    cudaFree(h->d_ov);
+    h->d_ov = nullptr;
+    h->ov_bytes = 0;
+    CUDA_TRY(cudaMalloc(&h->d_ov, need));
+    h->ov_bytes = need;
+  }
+  size_t off[3];
+  snap_layout(h, n_rep, s.flags, off);
+  const char *mem = (const char *)s.mem;
+  const size_t r0 = ((size_t)GH * g.pitchB + CPAD) * h->elem_R();
+  OvPlanes p;
+  p.L = g.L; p.rows = g.rows; p.pitchW = g.pitchW; p.pitchB = g.pitchB; p.nq = h->nq(); p.n_rep = n_rep;
+  p.S[0] = h->d_S[h->cur] + (size_t)rep0 * g.bits_stride + (size_t)GH * g.pitchW + WPAD;
+  p.S[1] = (const uint32_t *)mem + (size_t)GH * g.pitchW + WPAD;
+  p.R[0] = (const char *)h->d_R[h->cur] + (size_t)rep0 * g.plane_stride * h->elem_R() + r0;
+  p.R[1] = mem + off[1] + r0;
+  p.Q[0] = (const char *)h->Qcur() + (size_t)rep0 * g.site_stride * h->nq() * h->elem_Q();
+  p.Q[1] = mem + off[2];
+  p.bits_stride = g.bits_stride; p.plane_stride = g.plane_stride; p.q_stride = g.site_stride * h->nq();
+  std::vector<double> rq(2 * (size_t)n_rep);
+  for (int r = 0; r < n_rep; ++r) {
+    rq[r] = h->rc_host[rep0 + r].rq;
+    rq[n_rep + r] = s.rq[r];
+  }
+  const cudaError_t e = with_mode(h->mode, [&](auto md) {
+    return launch_overlap<decltype(md)>(p, want_r, want_q, rq.data(), h->d_ov, counts, changed, diffs);
+  });
+  if (e != cudaSuccess) return fail(SPGG_E_CUDA, "spgg_overlap: %s", cudaGetErrorString(e));
+  h->launches += 1 + (m > 0);
   return SPGG_OK;
 }
 

@@ -2,14 +2,16 @@
 // parallel (__graft_entry__.build): spgg_capi.cu (C ABI, host logic, fast / resident / helper kernels),
 // spgg_inst_general.cu (every instantiation of k_step), spgg_inst_lean.cu (k_step_lean / k_gmax_lean /
 // k_build_valtab), spgg_clusters.cu (cluster labelling, k_ccl_*), spgg_pairs.cu (pair counts, k_pair*), spgg_blocks.cu
-// (block fields, k_block_*) and spgg_hist.cu (value distributions, k_hist*).  A kernel is compiled in the unit that
-// instantiates it; the others launch it through the function pointer or the launcher declared here.
+// (block fields, k_block_*), spgg_hist.cu (value distributions, k_hist*) and spgg_overlap.cu (state overlaps,
+// k_overlap*).  A kernel is compiled in the unit that instantiates it; the others launch it through the function
+// pointer or the launcher declared here.
 #pragma once
 #include "spgg_kernels.cuh"
 #include "spgg_clusters.cuh"
 #include "spgg_pairs.cuh"
 #include "spgg_blocks.cuh"
 #include "spgg_hist.cuh"
+#include "spgg_overlap.cuh"
 
 namespace spgg {
 
@@ -29,5 +31,6 @@ constexpr int LEAN_TR_MAX = 16;   // k_step_lean addresses the shared-memory lay
 // spgg_pairs.cu: launch_pair_counts / launch_pair_record (spgg_pairs.cuh)
 // spgg_blocks.cu: block_scratch_bytes / launch_block_fields (spgg_blocks.cuh)
 // spgg_hist.cu: hist_scratch_bytes / launch_value_ranges / launch_histograms (spgg_hist.cuh)
+// spgg_overlap.cu: overlap_scratch_bytes / launch_overlap (spgg_overlap.cuh)
 
 }  // namespace spgg

@@ -224,6 +224,59 @@ def class_histograms(h: dict) -> dict:
     return out
 
 
+def snapshot_slot(slot) -> int:
+    """``slot`` of the snapshot methods -> the slot index of the C ABI, in [0, ``SPGG_MAX_SNAPSHOTS``)."""
+    if not isinstance(slot, (int, np.integer)) or isinstance(slot, bool) or not 0 <= slot < L_.MAX_SNAPSHOTS:
+        raise ValueError(f"slot must be an int in [0, {L_.MAX_SNAPSHOTS}), got {slot!r}")
+    return int(slot)
+
+
+def overlap_result(counts, changed, diffs, flags: int, q_shape, batched: bool, t0: int, t: int) -> dict:
+    """The flat arrays of ``spgg_overlap`` (counts (n, 2, 2) int64, changed (n, m) int64, diffs (n, m, 3)) -> the
+    dict of ``Engine.overlap``."""
+    n = counts.shape[0]
+    out = {"S": counts}
+    ch = 0
+    if flags & L_.SNAP_R:
+        out["R_changed"], out["R_diff"] = changed[:, 0], diffs[:, 0]
+        ch = 1
+    if flags & L_.SNAP_Q:
+        out["Q_changed"] = changed[:, ch:].reshape((n,) + tuple(q_shape))
+        out["Q_diff"] = diffs[:, ch:].reshape((n,) + tuple(q_shape) + (3,))
+    if not batched:
+        out = {k: v[0] for k, v in out.items()}
+    out["t0"], out["t"] = int(t0), int(t)
+    return out
+
+
+def overlap_measures(o: dict, n_sites: int) -> dict:
+    """Summary measures of an ``overlap`` result over a lattice of ``n_sites`` sites (a leading replica axis
+    carries through): ``hamming`` = (n_CD + n_DC) / N, the fraction of sites whose strategy differs;
+    ``autocorrelation`` = (n_CC/N - f0 f) / sqrt(f0 (1 - f0) f (1 - f)) with f0, f the cooperator fractions then
+    and now (NaN when either state is uniform); ``persistence_C`` = n_CC / n_C(t0) and ``persistence_D`` =
+    n_DD / n_D(t0) (NaN when that class was empty at t0); and for each field present ``R_rms`` / ``Q_rms`` =
+    sqrt(sum d^2 / N) and ``R_mean_abs`` / ``Q_mean_abs`` = sum |d| / N (per Q entry)."""
+    S = np.asarray(o["S"], np.float64)
+    if S.shape[-2:] != (2, 2):
+        raise ValueError(f"o['S'] must end in (2, 2), got {S.shape}")
+    N = float(n_sites)
+    nCC, nCD, nDC, nDD = S[..., 0, 0], S[..., 0, 1], S[..., 1, 0], S[..., 1, 1]
+    f0, f = (nCC + nCD) / N, (nCC + nDC) / N
+    nC0, nD0 = nCC + nCD, nDC + nDD
+    den = np.sqrt(f0 * (1.0 - f0) * f * (1.0 - f))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out = {"hamming": (nCD + nDC) / N,
+               "autocorrelation": np.where(den > 0, (nCC / N - f0 * f) / np.where(den > 0, den, 1.0), np.nan),
+               "persistence_C": np.where(nC0 > 0, nCC / np.where(nC0 > 0, nC0, 1.0), np.nan),
+               "persistence_D": np.where(nD0 > 0, nDD / np.where(nD0 > 0, nD0, 1.0), np.nan)}
+    for key in ("R", "Q"):
+        if key + "_diff" in o:
+            d = np.asarray(o[key + "_diff"], np.float64)
+            out[key + "_rms"] = np.sqrt(d[..., 2] / N)
+            out[key + "_mean_abs"] = d[..., 1] / N
+    return {k: np.asarray(v)[()] for k, v in out.items()}
+
+
 class Engine:
     """``n`` independent lattices on one device.  ``param_list`` is one dict (or a
     sequence of dicts, one per replica) with the reference ctor's argument names."""
@@ -455,6 +508,58 @@ class Engine:
         counts, pol = self._histograms(rep0, n, flags, bins, edges, policy)
         return hist_result(counts, pol, edges, chans, (2, 2) if self.nq == 4 else (2, 2, 2),
                            isinstance(replica, range), replica)
+
+    # -- state overlaps (include/spgg.h: spgg_snapshot / spgg_overlap)
+    def snapshot(self, slot: int = 0, replica=0, fields=("R", "Q")) -> int:
+        """Keep a copy of the current state of ``replica`` (an int, or a ``range`` of consecutive replicas) in
+        ``slot`` on the device: the strategies always, R and Q as ``fields`` asks.  Replaces what the slot held;
+        the copy survives stepping and state uploads until ``drop_snapshot`` or ``close``.  Returns the
+        iteration counter stored with it."""
+        flags = block_flags(fields)   # SPGG_SNAP_R / SPGG_SNAP_Q are the bits of SPGG_BLOCK_R / SPGG_BLOCK_Q
+        slot = snapshot_slot(slot)
+        rep0, n = hist_replicas(replica, self.n_replicas)
+        L_.check(self.lib.spgg_snapshot(self._h, slot, rep0, n, flags))
+        return self.snapshot_info(slot)["iteration"]
+
+    def snapshot_info(self, slot: int = 0) -> dict:
+        """``{"iteration", "replica", "fields"}`` of the snapshot in ``slot`` (``replica`` an int, or a range
+        for several replicas)."""
+        slot = snapshot_slot(slot)
+        it, rep0, n, flags = C.c_int64(), C.c_int(), C.c_int(), C.c_int()
+        L_.check(self.lib.spgg_snapshot_info(self._h, slot, C.byref(it), C.byref(rep0), C.byref(n), C.byref(flags)))
+        rep = rep0.value if n.value == 1 else range(rep0.value, rep0.value + n.value)
+        fields = tuple(f for f, bit in (("R", L_.SNAP_R), ("Q", L_.SNAP_Q)) if flags.value & bit)
+        return {"iteration": int(it.value), "replica": rep, "fields": fields}
+
+    def drop_snapshot(self, slot: int = 0):
+        """Free the snapshot in ``slot`` (nothing happens if it is empty)."""
+        L_.check(self.lib.spgg_snapshot_free(self._h, snapshot_slot(slot)))
+
+    def _overlap(self, slot: int, rep0: int, n: int, flags: int):
+        """``spgg_overlap`` -> (counts (n, 2, 2) int64, changed (n, m) int64, diffs (n, m, 3) float64)."""
+        m = len(hist_channels(flags, self.nq))
+        counts, changed, diffs = np.zeros((n, 2, 2), np.int64), np.zeros((n, m), np.int64), np.zeros((n, m, 3))
+        L_.check(self.lib.spgg_overlap(self._h, slot, rep0, n, flags, counts.ctypes.data,
+                                       changed.ctypes.data if m else None, diffs.ctypes.data if m else None))
+        return counts, changed, diffs
+
+    def overlap(self, slot: int = 0, replica=0, fields=("R", "Q")) -> dict:
+        """What changed between the snapshot in ``slot`` and the current state, computed on the device.  Replica
+        ``replica`` + i is compared with replica i of the snapshot, so a slot taken of replica a compared at
+        replica b measures how far two replicas are apart.  Returns ``"S"`` int64 (2, 2) [then, now] (0 = C,
+        1 = D); for R ``"R_changed"`` (the number of sites whose value differs) and ``"R_diff"`` (3,) [max |d|,
+        sum |d|, sum d^2], d = now - then; for Q ``"Q_changed"`` and ``"Q_diff"`` with the Q shape of
+        ``get_state`` (+ (3,)); ``"t0"`` the snapshot's iteration and ``"t"`` the current one.  Counts and maxima
+        are exact; the sums are fp64 in an order fixed by the lattice shape.  A ``range`` of replicas adds a
+        leading replica axis.  ``overlap_measures`` turns the result into Hamming distance, autocorrelation,
+        persistence and RMS change."""
+        flags = block_flags(fields)
+        slot = snapshot_slot(slot)
+        rep0, n = hist_replicas(replica, self.n_replicas)
+        counts, changed, diffs = self._overlap(slot, rep0, n, flags)
+        t0 = self.snapshot_info(slot)["iteration"]
+        return overlap_result(counts, changed, diffs, flags, (2, 2) if self.nq == 4 else (2, 2, 2),
+                              isinstance(replica, range), t0, self.status(rep0).iteration)
 
     def set_replay(self, u, b):
         """``u`` (n,rows,L) float64 and ``b`` (n,rows,L) 0/1: the reference's draw

@@ -73,6 +73,22 @@ def assemble_block_fields(L: int, b: int, world: int, parts) -> tuple[np.ndarray
     return counts, sums
 
 
+def assemble_overlap(parts) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """The whole lattice's overlap from the strips' (``StripEngine.overlap``): ``parts[k]`` is rank k's (counts
+    (1, 2, 2) int64, changed (1, m) int64, diffs (1, m, 3) float64) over its own rows.  Counts are summed, max |d|
+    maxed, and the fp64 sums added in rank order, so every rank that assembles the same parts gets the same
+    bits."""
+    counts = np.zeros_like(parts[0][0])
+    changed = np.zeros_like(parts[0][1])
+    diffs = np.zeros_like(parts[0][2])
+    for c, ch, d in parts:
+        counts += c
+        changed += ch
+        diffs[..., 0] = np.maximum(diffs[..., 0], d[..., 0])
+        diffs[..., 1:] += d[..., 1:]
+    return counts, changed, diffs
+
+
 def neighbours(world: int, rank: int) -> tuple[int, int]:
     """(up, down): ranks owning the rows just above (row0-1) and just below; periodic."""
     return (rank - 1) % world, (rank + 1) % world
@@ -466,6 +482,45 @@ class StripEngine:
         if policy:
             pol = self._all_reduce(pol, self.dist.ReduceOp.SUM)
         return hist_result(counts, pol, edges, chans, (2, 2) if eng.nq == 4 else (2, 2, 2), False, 0)
+
+    # -- state overlaps (include/spgg.h: spgg_snapshot / spgg_overlap)
+    def snapshot(self, slot: int = 0, fields=("R", "Q")) -> int:
+        """``Engine.snapshot`` of every strip (all ranks call this): each keeps a copy of its own rows."""
+        from .engine import block_flags, snapshot_slot
+        block_flags(fields)
+        snapshot_slot(slot)
+        self._settle()
+        return self.eng.snapshot(slot, 0, fields)
+
+    def overlap(self, slot: int = 0, fields=("R", "Q")) -> dict:
+        """``Engine.overlap`` of the WHOLE lattice (all ranks call this; every rank gets the same dict): each
+        strip compares its own rows, the strips' results are all-gathered and ``assemble_overlap`` adds the counts,
+        maxes the maxima and adds the fp64 sums in rank order."""
+        from .engine import block_flags, overlap_result, snapshot_slot
+        torch = self.torch
+        flags = block_flags(fields)
+        slot = snapshot_slot(slot)
+        self._settle()
+        eng = self.eng
+        counts, changed, diffs = eng._overlap(slot, 0, 1, flags)
+        if self.world > 1:
+            m = changed.shape[1]
+            # counts and the bytes of the diffs travel as one int64 tensor per rank
+            t = torch.from_numpy(np.concatenate([counts.reshape(-1), changed.reshape(-1), diffs.reshape(-1).view(np.int64)]))
+            if self.host_staged:
+                got = [torch.empty_like(t) for _ in range(self.world)]
+                self.dist.all_gather(got, t, group=self.group)
+            else:
+                allp = torch.empty((self.world * t.numel(),), dtype=torch.int64, device=self.dev)
+                self.dist.all_gather_into_tensor(allp, t.to(self.dev), group=self.group)
+                got = list(allp.cpu().split(t.numel()))
+            parts = []
+            for g in got:
+                a = g.numpy()
+                parts.append((a[:4].reshape(1, 2, 2), a[4:4 + m].reshape(1, m), a[4 + m:].copy().view(np.float64).reshape(1, m, 3)))
+            counts, changed, diffs = assemble_overlap(parts)
+        return overlap_result(counts, changed, diffs, flags, (2, 2) if eng.nq == 4 else (2, 2, 2), False,
+                              eng.snapshot_info(slot)["iteration"], eng.status().iteration)
 
     # -- stepping
     def _stream(self):
